@@ -276,10 +276,45 @@ class Env:
         return out.tolist()
 
 
-def codec_roundtrip(env, spec, steps, warmup, use_graph, sample_clocks=False, scheme=2):
+DUMP_BYTES_MAX = 64 << 20
+DUMP_GROUPS_MAX = 1 << 20          # per-group records (20 B each) beyond this are a seeded sample
+
+
+def dump_outputs(dump_dir, env, first_held, payload, scales, comp, out):
+    """Writes what the round trip hands its caller after the last timed step, as .npy files that two builds can be
+    compared by: the scale and compressed size of every group (of a seeded sample of DUMP_GROUPS_MAX groups beyond
+    that, group_index names them), and for 16 groups picked with a fixed seed their payload (the first comp_bytes of
+    the slot, the rest zero) and their decoded values.  float32 / float64, at most DUMP_BYTES_MAX in all."""
+    import numpy as np
+
+    torch = env.torch
+    n = comp.numel()
+    held = n - first_held                                    # groups whose decode `out` still holds, from row 0
+    pick = np.sort(np.random.default_rng(0).choice(held, min(16, held), replace=False))
+    rows = torch.from_numpy(pick).to(out.device)
+    groups = pick + first_held
+    comp_h = comp.cpu().numpy()
+    pay = payload.index_select(0, rows + first_held).cpu().numpy()
+    pay = np.where(np.arange(pay.shape[1])[None, :] < comp_h[groups][:, None], pay, 0)
+    every = np.arange(n) if n <= DUMP_GROUPS_MAX else np.sort(np.random.default_rng(1).choice(n, DUMP_GROUPS_MAX, replace=False))
+    arrays = {"group_index": every.astype(np.float64),
+              "scales": scales[torch.from_numpy(every).to(scales.device)].cpu().numpy().astype(np.float32),
+              "comp_bytes": comp_h[every].astype(np.float64),
+              "sample_groups": groups.astype(np.float64), "payload_sample": pay.astype(np.float32),
+              "decoded_sample": out.index_select(0, rows).float().cpu().numpy()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES_MAX, f"--dump-outputs: {total} bytes exceed {DUMP_BYTES_MAX}"
+    os.makedirs(dump_dir, exist_ok=True)
+    suffix = f"_rank{env.rank}" if env.world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(dump_dir, f"{name}{suffix}.npy"), a)
+
+
+def codec_roundtrip(env, spec, steps, warmup, use_graph, sample_clocks=False, scheme=2, dump_dir=None):
     """K timed steps of: compress every group of this rank's shard -> (N > 1: all-gather of the page-table
     metadata on a side stream, overlapped) -> decompress every group.  Device-resident inputs.
-    -> dict with the whole-job value, the per-phase times (CUDA events on the launching stream) and the roofline."""
+    -> dict with the whole-job value, the per-phase times (CUDA events on the launching stream) and the roofline.
+    dump_dir: where to write the last timed step's outputs (dump_outputs)."""
     import ctypes as C
 
     torch, dist, L, dev, world = env.torch, env.dist, env.L, env.dev, env.world
@@ -409,6 +444,10 @@ def codec_roundtrip(env, spec, steps, warmup, use_graph, sample_clocks=False, sc
     chk = min(n_groups, 8)
     ref = codec.decompress(codec.compress(x[:chk * G], G, scheme=scheme))
     assert torch.equal(ref.view(torch.int16), out[:chk].view(torch.int16)) or out_groups != n_groups, "bench output differs"
+    if dump_dir:
+        # with one launch chunk of output buffer, `out` holds the last chunk's decode
+        first_held = 0 if out_groups == n_groups else (n_groups - 1) // cg * cg
+        dump_outputs(dump_dir, env, first_held, payload, scales, comp, out)
 
     peak, peak_src = hbm_peak()
     alg_comp = 2 * G * n_groups + comp_total + 12 * n_groups       # 2n read + c write + 12 B header per group
@@ -777,7 +816,7 @@ def run_cuda(args, rank, world, local_rank):
     use_graph = not args.no_graph
     spec = workload_spec(args.workload, world, rank, args.scale)
     log(rank, f"headline {args.workload} x{world} ...")
-    head = codec_roundtrip(env, spec, args.steps, args.warmup, use_graph, sample_clocks=True)
+    head = codec_roundtrip(env, spec, args.steps, args.warmup, use_graph, sample_clocks=True, dump_dir=args.dump_outputs)
     x = head.pop("_x")
     e2e = None
     if not args.no_e2e:
@@ -882,7 +921,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="CUDA path only (--impl cuda): write the headline round trip's "
+                    "outputs of its last timed step to DIR/<name>.npy (scales and sizes of every group, payload and "
+                    "decoded values of 16 seeded groups; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the CUDA path's outputs")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -5,12 +5,21 @@ TEST INFRASTRUCTURE ONLY.  Run in the authoring container, where /root/reference
 exists and `make -C oracle ref` has produced oracle/_ref/libspeckv_ref.so:
 
     python oracle/make_golden.py
+    python oracle/make_golden.py traces [ref|port]   # only tests/golden/reference_traces.json
 
-Every fixture is the output of the reference's unmodified sources
-(FPGACacheEngine::compress/decompress, translate_address, AddressTranslationUnit,
-LSTMPredictor::predict_top_k, SpeculativePrefetcher::prefetch, the host C API with
-/dev/null as the device).  tests/test_oracle_golden.py pins the C restatement to
-them on CPU; tests/test_codec_gpu.py pins the CUDA path to them on a B200.
+Every fixture in golden.json, codec_cases.npz and translate_cases.npz is the output of
+the reference's unmodified sources (FPGACacheEngine::compress/decompress,
+translate_address, AddressTranslationUnit, LSTMPredictor::predict_top_k,
+SpeculativePrefetcher::prefetch, the host C API with /dev/null as the device).
+tests/test_oracle_golden.py pins the C restatement to them on CPU;
+tests/test_codec_gpu.py pins the CUDA path to them on a B200.
+
+reference_traces.json is the exception that names its source in its "source" field.
+`traces ref` records it from the reference.  `traces port` records it from the C
+restatement, for a checkout without the reference's sources: the tests then pin the
+restatement to its own recorded answers, and compare it with the reference itself
+wherever oracle/_ref is built.  A `traces port` run refuses to replace a recording
+made from the reference.
 """
 import ctypes as C
 import json
@@ -256,7 +265,51 @@ def main():
     with open(os.path.join(OUT, "golden.json"), "w") as f:
         json.dump(meta, f, indent=1, sort_keys=True)
     print("wrote", OUT, {k: len(v) if hasattr(v, "__len__") else v for k, v in meta.items() if k != "generator"})
+    record_traces("ref")
+
+
+TRACE_SOURCES = {
+    "ref": "oracle/_ref (reference C++ model, unmodified): FPGACacheEngine::compress/decompress, CXLMemoryManager",
+    "port": "oracle/speckv_oracle.c (the C restatement), recorded where the reference was not built; the restatement "
+            "matched the reference on these same cases while oracle/_ref was built alongside it",
+}
+
+
+def record_traces(impl: str):
+    """tests/golden/reference_traces.json: what the reference answers on the random codec cases and residency-policy
+    traces of oracle.random_codec_cases / random_policy_trace (digests for the codec, full traces for the policy)."""
+    from oracle.oracle import random_codec_cases, random_policy_trace, run_policy_trace
+    E = {"ref": Ref, "port": Port}[impl]
+    path = os.path.join(OUT, "reference_traces.json")
+    if impl == "port" and os.path.exists(path):
+        with open(path) as f:
+            if json.load(f).get("source") == TRACE_SOURCES["ref"]:
+                raise SystemExit(f"{path} holds the reference's own answers; the restatement does not replace them")
+    inputs, payloads = random_codec_cases()
+    comp, dec = [], []
+    for x in inputs:
+        s, p = E.compress(x)
+        y = E.decompress(s, p, x.size)
+        comp.append([int(f32_bits([s])[0]), int(p.size), "%016x" % Port.fnv1a64(p), "%016x" % Port.fnv1a64(f32_bits(y))])
+    for s, p in payloads:
+        y = E.decompress(s, p, 200000)
+        dec.append([int(y.size), "%016x" % Port.fnv1a64(f32_bits(y))])
+    policy = []
+    for seed in range(4):
+        ops, n = random_policy_trace(seed)
+        r = run_policy_trace(ops, n, impl=impl)
+        policy.append(dict(r, seed=seed, n_pages=n, n_ops=len(ops)))
+    out = {"generator": "oracle/make_golden.py", "source": TRACE_SOURCES[impl],
+           "codec_random": {"compress": comp, "decompress": dec}, "policy": policy}
+    # one line per top-level entry: the traces are data, not meant to be read line by line
+    with open(path, "w") as f:
+        f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(out[k], sort_keys=True, separators=(',', ':'))}"
+                                  for k in sorted(out)) + "\n}\n")
+    print("wrote", path, "from", impl)
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:2] == ["traces"]:
+        record_traces(sys.argv[2] if len(sys.argv) > 2 else "ref")
+    else:
+        main()

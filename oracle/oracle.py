@@ -493,6 +493,58 @@ def run_policy_trace(ops, n_pages: int, caps=(1 << 40, 1 << 40, 1 << 40), impl: 
     return {"results": results, "tiers": tiers, "lru": lru, "stats": stats}
 
 
+def random_policy_trace(seed: int):
+    """-> (ops, n_pages): a random residency-policy trace for run_policy_trace that never fills L1 (the reference's
+    eviction path deadlocks).  The traces of tests/golden/reference_traces.json."""
+    import random
+    rng = random.Random(seed)
+    n = rng.choice([8, 64, 300])
+    ops = [("place", g, rng.choice([0, 1, 2, 2])) for g in range(n) if rng.random() < 0.9]
+    for _ in range(3000):
+        r, g = rng.random(), rng.randrange(n)
+        if r < 0.6:
+            ops.append(("touch", g))
+        elif r < 0.7:
+            ops.append(("hot", g))
+        elif r < 0.8:
+            ops.append(("promote", g))
+        elif r < 0.9:
+            ops.append(("demote", g))
+        elif r < 0.93:
+            ops.append(("release", g))
+        else:
+            ops.append(("place", g, rng.choice([0, 1, 2])))
+    return ops, n
+
+
+def random_codec_cases(seed: int = 11):
+    """-> (inputs, payloads): fp32 groups of mixed magnitude for compress, and arbitrary (not produced by compress)
+    (scale, payload) pairs for decompress.  The codec cases of tests/golden/reference_traces.json."""
+    rng = np.random.default_rng(seed)
+    inputs = []
+    for trial in range(60):
+        n = int(rng.integers(1, 5000))
+        kind = trial % 4
+        if kind == 0:
+            x = rng.standard_normal(n).astype(np.float16).astype(np.float32)
+        elif kind == 1:
+            x = np.repeat(rng.standard_normal(n // 97 + 1), 97)[:n].astype(np.float16).astype(np.float32)
+        elif kind == 2:
+            b = np.ascontiguousarray(rng.standard_normal(n) * np.exp(rng.uniform(-90, 80)), dtype=np.float32)
+            u = b.view(np.uint32).astype(np.uint64)                          # to bf16, RN-even, and back
+            x = (((u + 0x7FFF + ((u >> 16) & 1)) >> 16).astype(np.uint32) << 16).view(np.float32)
+        else:
+            x = (rng.standard_normal(n) * np.exp(rng.uniform(-30, 30, n))).astype(np.float32)
+        inputs.append(x)
+    payloads = []
+    for trial in range(20):
+        p = rng.integers(0, 256, int(rng.integers(0, 400)), dtype=np.uint8)
+        if trial % 2:
+            p[1::2] = rng.integers(0, 4, p[1::2].size)
+        payloads.append((np.float32(rng.uniform(0.001, 3)), p))
+    return inputs, payloads
+
+
 def splitmix64_block(seed: int, n: int) -> np.ndarray:
     """The cross-language integer generator of SURVEY.md section 8c: splitmix64(seed) ->
     k = sum of four 11-bit fields - 4094, x = k / 1024 (exactly representable in fp16)."""

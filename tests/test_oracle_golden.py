@@ -1,11 +1,19 @@
 """CPU: the C restatement (oracle/speckv_oracle.c) against the fixtures produced by the
 reference's own C++ model (tests/golden, see oracle/make_golden.py) and, when
-oracle/_ref is present, against the reference itself on fresh random inputs."""
+oracle/_ref is present, against the reference itself on the same random inputs."""
 import numpy as np
 import pytest
 
 from oracle.oracle import Port, Ref, splitmix64_block
 from tests.helpers import F16, BF16, F32, bf16_from_f32, bf16_to_f32, case_input, f32_bits
+
+
+@pytest.fixture(scope="module")
+def reference_traces():
+    import json
+    import os
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_traces.json")) as f:
+        return json.load(f)
 
 
 def test_codec_fixtures(golden):
@@ -136,32 +144,28 @@ def test_lstm_fixtures(golden):
     assert [L.oracle_kv_address(0, pf["layer"], i + 1) for i in range(pf["depth"])] == pf["va"]
 
 
-@pytest.mark.skipif(not Ref.available(), reason="oracle/_ref not built (needs /root/reference)")
-def test_port_vs_reference_random():
-    rng = np.random.default_rng(11)
-    for trial in range(60):
-        n = int(rng.integers(1, 5000))
-        kind = trial % 4
-        if kind == 0:
-            x = rng.standard_normal(n).astype(np.float16).astype(np.float32)
-        elif kind == 1:
-            x = np.repeat(rng.standard_normal(n // 97 + 1), 97)[:n].astype(np.float16).astype(np.float32)
-        elif kind == 2:
-            x = bf16_to_f32(bf16_from_f32(rng.standard_normal(n) * np.exp(rng.uniform(-90, 80))))
-        else:
-            x = (rng.standard_normal(n) * np.exp(rng.uniform(-30, 30, n))).astype(np.float32)
+def test_port_vs_reference_random(reference_traces):
+    """The restatement on random inputs against the answers recorded in tests/golden/reference_traces.json (its
+    "source" names the reference or the restatement) and, where oracle/_ref is built, against the reference itself."""
+    from oracle.oracle import random_codec_cases
+    want = reference_traces["codec_random"]
+    inputs, payloads = random_codec_cases()
+    assert len(inputs) == len(want["compress"]) and len(payloads) == len(want["decompress"])
+    for x, w in zip(inputs, want["compress"]):
         s1, p1 = Port.compress(x)
-        s2, p2 = Ref.compress(x)
-        assert f32_bits([s1])[0] == f32_bits([s2])[0] and np.array_equal(p1, p2)
-        assert np.array_equal(f32_bits(Port.decompress(s1, p1, n)), f32_bits(Ref.decompress(s2, p2, n)))
-    # arbitrary (not produced by compress) payloads through both decoders
-    for trial in range(20):
-        p = rng.integers(0, 256, int(rng.integers(0, 400)), dtype=np.uint8)
-        if trial % 2:
-            p[1::2] = rng.integers(0, 4, p[1::2].size)
-        s = np.float32(rng.uniform(0.001, 3))
-        a, b = Port.decompress(s, p, 200000), Ref.decompress(s, p, 200000)
-        assert np.array_equal(f32_bits(a), f32_bits(b))
+        y1 = Port.decompress(s1, p1, x.size)
+        assert [int(f32_bits([s1])[0]), int(p1.size), "%016x" % Port.fnv1a64(p1),
+                "%016x" % Port.fnv1a64(f32_bits(y1))] == w, x.size
+        if Ref.available():
+            s2, p2 = Ref.compress(x)
+            assert f32_bits([s1])[0] == f32_bits([s2])[0] and np.array_equal(p1, p2)
+            assert np.array_equal(f32_bits(y1), f32_bits(Ref.decompress(s2, p2, x.size)))
+    # arbitrary (not produced by compress) payloads through the decoder
+    for (s, p), w in zip(payloads, want["decompress"]):
+        a = Port.decompress(s, p, 200000)
+        assert [int(a.size), "%016x" % Port.fnv1a64(f32_bits(a))] == w, p.size
+        if Ref.available():
+            assert np.array_equal(f32_bits(a), f32_bits(Ref.decompress(s, p, 200000)))
 
 
 def test_division_identities_quick():
@@ -177,35 +181,24 @@ def test_division_identities_quick():
     assert out.returncode == 0 and out.stdout.strip().endswith("OK"), out.stdout
 
 
-def test_policy_port_matches_reference_manager():
-    """oracle_policy_* against the reference's CXLMemoryManager (oracle/_ref) on random traces that
-    never fill L1 (its eviction path deadlocks): per-call results, final tiers, LRU order, stats."""
-    import random
-    from oracle.oracle import run_policy_trace
-    for seed in range(4):
-        rng = random.Random(seed)
-        n = rng.choice([8, 64, 300])
-        ops = [("place", g, rng.choice([0, 1, 2, 2])) for g in range(n) if rng.random() < 0.9]
-        for _ in range(3000):
-            r, g = rng.random(), rng.randrange(n)
-            if r < 0.6:
-                ops.append(("touch", g))
-            elif r < 0.7:
-                ops.append(("hot", g))
-            elif r < 0.8:
-                ops.append(("promote", g))
-            elif r < 0.9:
-                ops.append(("demote", g))
-            elif r < 0.93:
-                ops.append(("release", g))
-            else:
-                ops.append(("place", g, rng.choice([0, 1, 2])))
-        a = run_policy_trace(ops, n, impl="port")
-        b = run_policy_trace(ops, n, impl="ref")
-        assert a["results"] == b["results"]
-        assert a["tiers"] == b["tiers"]
-        assert a["lru"] == b["lru"]
-        assert a["stats"] == b["stats"]
+def test_policy_port_matches_reference_manager(reference_traces):
+    """oracle_policy_* against the reference's CXLMemoryManager on random traces that never fill L1 (its eviction
+    path deadlocks): per-call results, final tiers, LRU order, stats -- against the answers recorded in
+    tests/golden/reference_traces.json (its "source" names the reference or the restatement) and, where oracle/_ref
+    is built, against the reference itself."""
+    import json
+    from oracle.oracle import random_policy_trace, run_policy_trace
+    assert len(reference_traces["policy"]) == 4
+    for want in reference_traces["policy"]:
+        ops, n = random_policy_trace(want["seed"])
+        assert (n, len(ops)) == (want["n_pages"], want["n_ops"])
+        a = json.loads(json.dumps(run_policy_trace(ops, n, impl="port")))     # tuples -> lists, as stored
+        refs = [want] + ([json.loads(json.dumps(run_policy_trace(ops, n, impl="ref")))] if Ref.available() else [])
+        for b in refs:
+            assert a["results"] == b["results"]
+            assert a["tiers"] == b["tiers"]
+            assert a["lru"] == b["lru"]
+            assert a["stats"] == b["stats"]
 
 
 def test_policy_port_eviction_semantics():
