@@ -1,5 +1,5 @@
 """Randomised differential run of the CUDA codec against the CPU oracle (test infrastructure, not collected by
-pytest):  python tests/fuzz_codec.py [seconds] [seed]
+pytest):  python tests/fuzz_codec.py [seconds] [seed]  |  decode [seconds] [seed]  |  paths [seconds] [seed]
 Random geometries (tuned and generic kernels), dtypes and value distributions -- mixtures of noise, constant and
 zero stretches of random lengths (around the 8-element lane chunk and the 255 cap), NaN / Inf / denormal
 sprinkles, tiny and huge magnitudes -- compressed and decompressed on the GPU; sizes, scales, payload bytes,
@@ -158,8 +158,123 @@ def main_decode(seconds=60.0, seed=0):
     print(f"decode fuzz ok: {cases} cases in {seconds:.0f} s (seed {seed})")
 
 
+def make_kv(rng, n):
+    """KV-like values: a window of a slow random walk (bench.py smooth_fp16), or N(0,1) with a few outlier channels
+    of a 128-wide head dim; sometimes filled only up to a random token, zeros behind it."""
+    if rng.random() < 0.5:                          # n steps of a 2^20-step walk, its start value drawn directly
+        x0 = 0.01 * np.sqrt(rng.integers(0, 1 << 20)) * rng.standard_normal()
+        x = (x0 + np.cumsum(0.01 * rng.standard_normal(n))).astype(np.float32)
+    else:
+        x = rng.standard_normal(n).astype(np.float32)
+        ch = np.arange(n) % 128
+        for c in rng.integers(0, 128, int(rng.integers(1, 5))):
+            x[ch == c] *= np.float32(rng.uniform(5, 100))
+    if rng.random() < 0.25:
+        x[int(rng.integers(1, n + 1)):] = 0.0
+    return x
+
+
+ENTRIES = ("plain", "gather", "indexed", "routed", "scatter")
+
+
+def main_paths(seconds=60.0, seed=0):
+    """Every scheme through every entry point: plain compress / decompress, paged gather (a block table with
+    repeats), indexed decode (requests with repeats), routed decode (request count on the device, 0 .. past the
+    capacity) and paged scatter (src_index + permuted block table).  Sizes, scales, payload bytes, decoded lengths
+    and decoded bits equal the oracle's; outputs nothing may write keep their sentinel."""
+    rng = np.random.default_rng(seed)
+    t_end = time.time() + seconds
+    counts = {("scheme", s): 0 for s in (1, 2, 3, 4)}
+    counts.update({("entry", e): 0 for e in ENTRIES})
+    cases = 0
+    S = 0x1234
+    while time.time() < t_end:
+        scheme = int(rng.integers(1, 5))
+        entry = ENTRIES[int(rng.integers(0, len(ENTRIES)))]
+        G = 2048 * int(2 ** rng.integers(0, 8)) if rng.random() < 0.75 else int(rng.integers(1, 20000))
+        n_groups = int(max(1, min(64, rng.integers(1, max(2, (3 << 20) // G)))))
+        dtype = F16 if rng.random() < 0.6 else BF16
+        tdt = torch.float16 if dtype == F16 else torch.bfloat16
+        x = np.concatenate([make_kv(rng, G) if rng.random() < 0.4 else make(rng, G) for _ in range(n_groups)])
+        if dtype == BF16 and rng.random() < 0.2:
+            with np.errstate(over="ignore"):
+                x *= np.float32(np.exp(rng.uniform(-70, 80)))
+        if dtype == F16:
+            with np.errstate(over="ignore"):
+                raw = x.astype(np.float16)
+            xd = torch.from_numpy(raw).cuda()
+        else:
+            raw = bf16_from_f32(x)
+            xd = torch.from_numpy(raw.astype(np.int16)).cuda().view(torch.bfloat16)
+        tag = f"paths case {cases}: {entry} scheme={scheme} G={G} n={n_groups} dtype={dtype} seed={seed}"
+        if os.environ.get("FUZZ_VERBOSE"):
+            print(tag, file=sys.stderr, flush=True)
+        sb = codec.slot_bytes(G, scheme)
+        payload, scales, comp = Port.compress_batch(raw, G, dtype=dtype, slot_bytes=sb, threads=8, scheme=scheme)
+        rows = np.arange(n_groups)
+        if entry == "gather":
+            rows = rng.integers(0, n_groups, int(rng.integers(1, n_groups + 4))).astype(np.int32)
+            c = codec.compress_gather(xd.view(n_groups, G), torch.from_numpy(rows).cuda(), scheme=scheme)
+        else:
+            c = codec.compress(xd, G, scheme=scheme)
+        assert np.array_equal(c.scales.cpu().numpy().view(np.uint32), scales[rows].view(np.uint32)), tag
+        assert np.array_equal(c.comp_bytes.cpu().numpy().view(np.uint32), comp[rows]), tag
+        gp = c.payload.cpu().numpy()
+        for i, g in enumerate(rows):
+            assert np.array_equal(gp[i, :comp[g]], payload[g, :comp[g]]), (tag, i)
+        want, want_n = Port.decompress_batch(payload, scales, comp, G, dtype, threads=8, scheme=scheme)
+        want = np.where(np.arange(G)[None, :] < want_n[:, None], want.view(np.uint16).reshape(n_groups, G), np.uint16(S))
+        n_st = rows.size
+        src = rng.integers(0, n_st, n_st).astype(np.int32)          # as many requests as stored blocks, with repeats
+        if rng.random() < 0.5:
+            src[: n_st // 2] = np.arange(n_st)[::-1][: n_st // 2]
+        srcd = torch.from_numpy(src).cuda()
+        oel = torch.full((n_st,), 0x5A5A5A5A, dtype=torch.int32, device="cuda")
+        if entry in ("plain", "gather"):
+            out = torch.full((n_st, G), S, dtype=torch.int16, device="cuda").view(tdt)
+            codec.decompress(c, out=out, out_elems=oel)
+            expect, expect_n = want[rows], want_n[rows]
+        elif entry == "indexed":
+            out = torch.full((n_st, G), S, dtype=torch.int16, device="cuda").view(tdt)
+            codec.decompress_indexed(c, srcd, out=out)
+            expect, expect_n = want[src], None
+        elif entry == "routed":
+            cnt = int(rng.choice([0, 1, max(0, n_st - 1), n_st, n_st + 3, int(rng.integers(0, n_st + 1))]))
+            out = torch.full((n_st, G), S, dtype=torch.int16, device="cuda").view(tdt)
+            codec.decompress_routed(c, srcd, torch.tensor([cnt], dtype=torch.int32, device="cuda"), out)
+            expect, expect_n = np.full((n_st, G), S, np.uint16), None
+            expect[:min(cnt, n_st)] = want[src[:min(cnt, n_st)]]
+            tag += f" count={cnt}"
+        else:
+            nb = n_st + int(rng.integers(0, 9))
+            dst = rng.permutation(nb)[:n_st].astype(np.int32)
+            out = torch.full((nb, G), S, dtype=torch.int16, device="cuda").view(tdt)
+            codec.decompress_scatter(c, out, torch.from_numpy(dst).cuda(), srcd, out_elems=oel)
+            expect = np.full((nb, G), S, np.uint16)
+            expect[dst] = want[src]
+            expect_n = want_n[src]
+        torch.cuda.synchronize()
+        if expect_n is not None:
+            assert np.array_equal(oel.cpu().numpy().view(np.uint32), expect_n), tag
+        got = out.view(torch.int16).cpu().numpy().view(np.uint16)
+        if not np.array_equal(got, expect):
+            bad = np.argwhere(got != expect)
+            r0, e0 = bad[0]
+            raise AssertionError((tag, "mismatches", len(bad), "first at row", r0, "elem", e0, hex(got[r0, e0]),
+                                  hex(expect[r0, e0]), "rows hit", sorted(set(bad[:, 0].tolist()))[:10]))
+        counts[("scheme", scheme)] += 1
+        counts[("entry", entry)] += 1
+        cases += 1
+    per = ", ".join(f"{k[0]} {k[1]}: {v}" for k, v in counts.items())
+    print(f"paths fuzz ok: {cases} cases in {seconds:.0f} s (seed {seed}); {per}")
+    return counts
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "decode":
         main_decode(float(sys.argv[2]) if len(sys.argv) > 2 else 60.0, int(sys.argv[3]) if len(sys.argv) > 3 else 0)
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "paths":
+        main_paths(float(sys.argv[2]) if len(sys.argv) > 2 else 60.0, int(sys.argv[3]) if len(sys.argv) > 3 else 0)
         sys.exit(0)
     main(float(sys.argv[1]) if len(sys.argv) > 1 else 120.0, int(sys.argv[2]) if len(sys.argv) > 2 else 0)
