@@ -103,6 +103,8 @@ def lib() -> C.CDLL:
     L.speckv_ext_compress_gather.restype = C.c_int
     L.speckv_ext_decompress_scatter.argtypes = [vp, sz, vp, vp, vp, vp, sz, sz, C.c_int, vp, vp, C.c_int, vp]
     L.speckv_ext_decompress_scatter.restype = C.c_int
+    L.speckv_ext_compress_ragged.argtypes = [vp, vp, vp, C.c_int, sz, sz, vp, sz, vp, vp, C.c_int, vp]
+    L.speckv_ext_compress_ragged.restype = C.c_int
     L.speckv_ext_compress_host.argtypes = [vp, C.c_int, sz, sz, vp, sz, vp, vp, C.c_int]
     L.speckv_ext_compress_host.restype = C.c_int
     L.speckv_ext_decompress_host.argtypes = [vp, sz, vp, vp, sz, sz, C.c_int, vp, vp, C.c_int]
@@ -138,6 +140,8 @@ def lib() -> C.CDLL:
     L.speckv_ext_tier_offload_paged.restype = C.c_int
     L.speckv_ext_tier_restore_paged.argtypes = [vp, vp, sz, sz, C.c_int, vp, vp, vp]
     L.speckv_ext_tier_restore_paged.restype = C.c_int
+    L.speckv_ext_tier_offload_ragged.argtypes = [vp, vp, vp, vp, C.c_int, sz, sz, vp, vp]
+    L.speckv_ext_tier_offload_ragged.restype = C.c_int
     L.speckv_ext_tier_drop.argtypes = [vp, vp, sz]; L.speckv_ext_tier_drop.restype = C.c_int
     L.speckv_ext_tier_get_stats.argtypes = [vp, C.POINTER(TierStats)]; L.speckv_ext_tier_get_stats.restype = None
     L.speckv_ext_atu_create.argtypes = [C.c_uint32, C.POINTER(vp)]; L.speckv_ext_atu_create.restype = C.c_int

@@ -141,6 +141,45 @@ def compress_gather(cache: torch.Tensor, block_table: torch.Tensor, scheme: int 
     return out
 
 
+def compress_ragged(x: torch.Tensor, group_elems: int, lengths: torch.Tensor,
+                    block_table: Optional[torch.Tensor] = None, scheme: int = COMP_INT8_DELTA_RLE,
+                    out: Optional[CompressedKV] = None) -> CompressedKV:
+    """Compress the filled prefix of each block: group i is the first min(lengths[i], group_elems) elements of block
+    block_table[i] of x (block i when block_table is None), where x is a contiguous CUDA tensor of whole blocks of
+    group_elems elements.  lengths: CUDA int32 tensor of element counts, one per group; it stays on the device (no
+    synchronisation, graph-capturable).  Elements behind a group's length take no part in its scale or payload.
+    Schemes 1-4.  The decoders give lengths[i] elements per group and leave the rest of the destination as it is.
+    The lengths are not read on the host: the kernels take them as unsigned and clamp them to group_elems, so a
+    negative entry stores the whole block.  Callers that cannot rule that out check (lengths >= 0) themselves."""
+    if not x.is_cuda or x.dtype not in _DTYPES or not x.is_contiguous():
+        raise ValueError("compress_ragged() takes a contiguous CUDA fp16/bf16/fp32 tensor")
+    if group_elems <= 0 or x.numel() % group_elems:
+        raise ValueError("numel must be a multiple of group_elems")
+    if not lengths.is_cuda or lengths.dtype != torch.int32 or lengths.device != x.device:
+        raise TypeError("lengths must be an int32 tensor on the device of x")
+    lengths = lengths.contiguous()
+    if block_table is not None:
+        block_table = block_table.to(device=x.device, dtype=torch.int32).contiguous()
+        if block_table.numel() != lengths.numel():
+            raise ValueError("block_table and lengths differ in length")
+    elif lengths.numel() != x.numel() // group_elems:
+        raise ValueError("lengths must hold one entry per block of x")
+    n_groups = lengths.numel()
+    sb = slot_bytes(group_elems, scheme)
+    if out is None:
+        out = CompressedKV(torch.empty((n_groups, sb), dtype=torch.uint8, device=x.device),
+                           torch.empty(n_groups, dtype=torch.float32, device=x.device),
+                           torch.empty(n_groups, dtype=torch.int32, device=x.device),
+                           group_elems, x.dtype, scheme)
+    with torch.cuda.device(x.device):
+        st = lib().speckv_ext_compress_ragged(x.data_ptr(), block_table.data_ptr() if block_table is not None else None,
+                                              lengths.data_ptr(), _DTYPES[x.dtype], group_elems, n_groups,
+                                              out.payload.data_ptr(), out.payload.shape[1], out.scales.data_ptr(),
+                                              out.comp_bytes.data_ptr(), scheme, _stream())
+    check(st, "speckv_ext_compress_ragged")
+    return out
+
+
 def decompress_scatter(c: CompressedKV, cache: torch.Tensor, block_table: torch.Tensor,
                        src_index: Optional[torch.Tensor] = None,
                        out_elems: Optional[torch.Tensor] = None) -> torch.Tensor:

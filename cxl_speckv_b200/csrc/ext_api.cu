@@ -521,6 +521,21 @@ speckv_status_t speckv_ext_compress_gather(const void* d_cache, const uint32_t* 
     return codec_run(false, a, cuda_stream);
 }
 
+speckv_status_t speckv_ext_compress_ragged(const void* d_in, const uint32_t* d_block_table, const uint32_t* d_group_len,
+                                           speckv_dtype_t dtype, size_t group_elems, size_t n_groups, void* d_payload,
+                                           size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
+                                           speckv_comp_scheme_t scheme, void* cuda_stream) {
+    if (scheme == SPECKV_COMP_FP16) return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL;
+    CodecArgs a;
+    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_in);
+    if (rc != SPECKV_OK) return rc;
+    if (n_groups && !d_group_len) return SPECKV_ERR_INVAL;
+    a.in = d_in;
+    a.elem_index = d_block_table;
+    a.group_len = d_group_len;
+    return codec_run(false, a, cuda_stream);
+}
+
 speckv_status_t speckv_ext_decompress_scatter(const void* d_payload, size_t slot_bytes, const float* d_scales,
                                               const uint32_t* d_comp_bytes, const uint32_t* d_src_index,
                                               const uint32_t* d_block_table, size_t n_requests, size_t group_elems,

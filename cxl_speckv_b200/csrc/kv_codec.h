@@ -29,6 +29,9 @@ struct CodecArgs {
     // compress_packed_supported().
     uint64_t* pack_offsets = nullptr;
     uint64_t* pack_total = nullptr;          // receives the stream length, or ~0 when the placement failed (look-back timeout)
+    // compress, optional (device): group g encodes only the first min(group_len[g], group_elems) elements of its
+    // block (the filled prefix of a paged KV block); no packed emission with it
+    const uint32_t* group_len = nullptr;
     size_t slot_bytes = 0;
     uint32_t group_elems = 0;
     uint32_t n_groups = 0;

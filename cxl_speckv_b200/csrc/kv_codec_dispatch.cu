@@ -20,7 +20,7 @@ static bool force_generic() {
 }
 
 bool compress_packed_supported(const CodecArgs& a) {
-    return !force_generic() && scheme_is_rle(a.scheme) && fast_regions(a, false) == 1;
+    return !force_generic() && !a.group_len && scheme_is_rle(a.scheme) && fast_regions(a, false) == 1;
 }
 
 cudaError_t launch_compress(const CodecArgs& a, cudaStream_t st) {

@@ -186,7 +186,8 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
                             uint8_t* __restrict__ payload, size_t slot_bytes,
                             float* __restrict__ scales, uint32_t* __restrict__ comp_bytes,
                             const uint32_t* __restrict__ only_flagged, const uint32_t* __restrict__ elem_index,
-                            bool max_scale, const uint64_t* __restrict__ slot_offsets) {
+                            bool max_scale, const uint64_t* __restrict__ slot_offsets,
+                            const uint32_t* __restrict__ group_len) {
     __shared__ __align__(16) uint16_t stage[kTile + 16];
     __shared__ int wbuf[kWarps];
     __shared__ float fbuf[kWarps];
@@ -200,10 +201,11 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
         const T* gin = in + (size_t)(elem_index ? elem_index[g] : g) * G;
         uint8_t* gout = payload + (slot_offsets ? (size_t)slot_offsets[g] : (size_t)g * slot_bytes);   // packed emission: the slot reserved by the tuned kernel
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gin) & 15) == 0;
+        const uint32_t n = group_len ? min(group_len[g], G) : G;   // ragged calls: the group is the block's first n elements
 
         // second pass behind the tuned kernel: that kernel already took the group max and left its bits in
         // comp_bytes[g] (overwritten with the size below), so the input is read once here, not twice
-        const float m = only_flagged ? __uint_as_float(comp_bytes[g]) : group_absmax<T>(gin, G, vec_ok, fbuf);
+        const float m = only_flagged ? __uint_as_float(comp_bytes[g]) : group_absmax<T>(gin, n, vec_ok, fbuf);
         const float s = scale_for(m, max_scale);
         const bool fast = fast_quant_ok<T>(m);
         float r = 0.0f, rl = 0.0f;
@@ -212,11 +214,11 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
         uint32_t carry_q = 0, carry_d = 0;
         int carry_p0 = 0, carry_lh = 0, carry_nh = 0, stage_base = 0;
 
-        for (uint32_t tile = 0; tile < G; tile += kTile) {
+        for (uint32_t tile = 0; tile < n; tile += kTile) {
             const uint32_t start = tile + tid * kEPT;
-            const int cnt = start < G ? min((uint32_t)kEPT, G - start) : 0;
+            const int cnt = start < n ? min((uint32_t)kEPT, n - start) : 0;
             float x[kEPT];
-            load_elems<T>(gin, start, G, vec_ok, x);
+            load_elems<T>(gin, start, n, vec_ok, x);
             uint32_t q[kEPT];
             if (fast) {
 #pragma unroll
@@ -274,7 +276,7 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
                 }
                 dprev = d[j];
             }
-            const uint32_t last_valid = min(G, tile + kTile) - 1;
+            const uint32_t last_valid = min(n, tile + kTile) - 1;
             if (cnt > 0 && start + cnt - 1 == last_valid) {
                 carry_sm[0] = q[cnt - 1];
                 carry_sm[1] = d[cnt - 1];
@@ -301,10 +303,10 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
         }
 
         __syncthreads();
-        if (G > 0) {
+        if (n > 0) {
             // the run still open at the end of the group (:235-236)
             const int rem = (carry_nh - 1) - stage_base;  // pairs waiting in the stage, < 8
-            if (tid == 0) stage[rem] = (uint16_t)(carry_d | ((uint32_t)((int)G - carry_lh) << 8));
+            if (tid == 0) stage[rem] = (uint16_t)(carry_d | ((uint32_t)((int)n - carry_lh) << 8));
             if (tid > rem && tid < 8) stage[tid] = 0;
             __syncthreads();
             if (tid == 0) *reinterpret_cast<uint4*>(gout + (size_t)stage_base * 2) = *reinterpret_cast<const uint4*>(stage);
@@ -674,7 +676,7 @@ compress_int8_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gr
                              uint8_t* __restrict__ payload, size_t slot_bytes,
                              float* __restrict__ scales, uint32_t* __restrict__ comp_bytes,
                              const uint32_t* __restrict__ only_flagged, const uint32_t* __restrict__ elem_index,
-                             bool max_scale) {
+                             bool max_scale, const uint32_t* __restrict__ group_len) {
     __shared__ float fbuf[kWarps];
     __shared__ uint32_t smask[kWarps];
     const int tid = threadIdx.x;
@@ -683,31 +685,32 @@ compress_int8_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gr
         const T* gin = in + (size_t)(elem_index ? elem_index[g] : g) * G;
         uint8_t* gout = payload + (size_t)g * slot_bytes;
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gin) & 15) == 0;
+        const uint32_t n = group_len ? min(group_len[g], G) : G;
         // behind the tuned kernel the group max is already known (left in comp_bytes[g])
-        const float m = only_flagged ? __uint_as_float(comp_bytes[g]) : group_absmax<T>(gin, G, vec_ok, fbuf);
+        const float m = only_flagged ? __uint_as_float(comp_bytes[g]) : group_absmax<T>(gin, n, vec_ok, fbuf);
         const float s = scale_for(m, max_scale);
         const bool fast = fast_quant_ok<T>(m);
         float r = 0.0f, rl = 0.0f;
         if (fast) recip_hi_lo(s, r, rl);
-        for (uint32_t tile = 0; tile < G; tile += kTile) {
+        for (uint32_t tile = 0; tile < n; tile += kTile) {
             const uint32_t start = tile + tid * kEPT;
             float x[kEPT];
-            load_elems<T>(gin, start, G, vec_ok, x);
+            load_elems<T>(gin, start, n, vec_ok, x);
             uint32_t w[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
             for (int j = 0; j < kEPT; ++j) {
                 const uint32_t q = fast ? quantize_fast(x[j], r, rl) : quantize_exact(x[j], s);
                 w[j >> 2] |= q << (8 * (j & 3));
             }
-            if (start + kEPT <= G) {
+            if (start + kEPT <= n) {
                 *reinterpret_cast<uint4*>(gout + start) = make_uint4(w[0], w[1], w[2], w[3]);
             } else {
-                for (uint32_t j = 0; start + j < G && j < kEPT; ++j) gout[start + j] = (uint8_t)(w[j >> 2] >> (8 * (j & 3)));
+                for (uint32_t j = 0; start + j < n && j < kEPT; ++j) gout[start + j] = (uint8_t)(w[j >> 2] >> (8 * (j & 3)));
             }
         }
         if (tid == 0) {
             scales[g] = s;
-            comp_bytes[g] = G;
+            comp_bytes[g] = n;
         }
     }
 }
@@ -800,11 +803,11 @@ static cudaError_t launch_compress_t(const CodecArgs& a, cudaStream_t st, const 
     if (scheme_is_rle(a.scheme)) {
         compress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(in, a.group_elems, a.n_groups, pay, a.slot_bytes,
                                                                   a.scales, a.comp_bytes, only_flagged, a.elem_index,
-                                                                  scheme_max_scale(a.scheme), a.pack_offsets);
+                                                                  scheme_max_scale(a.scheme), a.pack_offsets, a.group_len);
     } else {
         compress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(in, a.group_elems, a.n_groups, pay, a.slot_bytes,
                                                                    a.scales, a.comp_bytes, only_flagged, a.elem_index,
-                                                                   scheme_max_scale(a.scheme));
+                                                                   scheme_max_scale(a.scheme), a.group_len);
     }
     count_launch();
     return cudaGetLastError();

@@ -88,8 +88,10 @@ struct BlockRec {
     uint32_t comp_bytes;   // bytes held in the pool (payload bytes, or the raw size for raw blocks)
     float scale;
     uint32_t group_elems;  // 0 for raw (uncompressed) blocks
-    int dtype;             // speckv_dtype_t | scheme << 8 (the scheme the block was stored under); -1 = empty map entry
+    int dtype;             // speckv_dtype_t | scheme << 8 (the scheme the block was stored under) | kRagged; -1 = empty map entry
     int scheme() const { return (dtype >> 8) & 0xff; }
+    bool ragged() const { return (dtype & kRagged) != 0; }
+    static constexpr int kRagged = 1 << 16;   // stored from a prefix of its block: decodes to fewer than group_elems elements
 };
 
 struct Extent {
@@ -204,11 +206,13 @@ struct Tier {
     uint32_t* d_comp[kBuf] = {};
     uint64_t* d_offsets[kBuf] = {};
     uint64_t* d_total[kBuf] = {};
+    uint32_t* d_oel[kBuf] = {};                          // restore: decoded lengths of a chunk with ragged blocks
     // pinned host mirrors of the small per-chunk metadata
     float* h_scales[kBuf] = {};
     uint32_t* h_comp[kBuf] = {};
     uint64_t* h_offsets[kBuf] = {};
     uint64_t* h_total[kBuf] = {};
+    uint32_t* h_oel[kBuf] = {};
     size_t cap_groups = 0, cap_slot_bytes = 0;           // per buffer
     int scheme = SPECKV_COMP_INT8_DELTA_RLE;             // what new offloads are stored under (speckv_ext_tier_set_scheme)
     speckv_tier_stats_t stats = {};
@@ -249,11 +253,12 @@ struct Tier {
     void release_staging() {
         for (int b = 0; b < kBuf; ++b) {
             cudaFree(d_slots[b]); cudaFree(d_packed[b]); cudaFree(d_scales[b]); cudaFree(d_comp[b]);
-            cudaFree(d_offsets[b]); cudaFree(d_total[b]);
+            cudaFree(d_offsets[b]); cudaFree(d_total[b]); cudaFree(d_oel[b]);
             cudaFreeHost(h_scales[b]); cudaFreeHost(h_comp[b]); cudaFreeHost(h_offsets[b]); cudaFreeHost(h_total[b]);
+            cudaFreeHost(h_oel[b]);
             d_slots[b] = d_packed[b] = nullptr; d_scales[b] = nullptr; d_comp[b] = nullptr;
             d_offsets[b] = d_total[b] = nullptr; h_scales[b] = nullptr; h_comp[b] = nullptr;
-            h_offsets[b] = h_total[b] = nullptr;
+            h_offsets[b] = h_total[b] = nullptr; d_oel[b] = h_oel[b] = nullptr;
         }
         cap_groups = cap_slot_bytes = 0;
     }
@@ -268,10 +273,12 @@ struct Tier {
             if ((e = cudaMalloc((void**)&d_comp[b], groups * 4)) != cudaSuccess) break;
             if ((e = cudaMalloc((void**)&d_offsets[b], groups * 8)) != cudaSuccess) break;
             if ((e = cudaMalloc((void**)&d_total[b], 8)) != cudaSuccess) break;
+            if ((e = cudaMalloc((void**)&d_oel[b], groups * 4)) != cudaSuccess) break;
             if ((e = cudaHostAlloc((void**)&h_scales[b], groups * 4, cudaHostAllocDefault)) != cudaSuccess) break;
             if ((e = cudaHostAlloc((void**)&h_comp[b], groups * 4, cudaHostAllocDefault)) != cudaSuccess) break;
             if ((e = cudaHostAlloc((void**)&h_offsets[b], groups * 8, cudaHostAllocDefault)) != cudaSuccess) break;
             if ((e = cudaHostAlloc((void**)&h_total[b], 8, cudaHostAllocDefault)) != cudaSuccess) break;
+            if ((e = cudaHostAlloc((void**)&h_oel[b], groups * 4, cudaHostAllocDefault)) != cudaSuccess) break;
         }
         if (e != cudaSuccess) {
             release_staging();
@@ -337,9 +344,10 @@ void speckv_ext_tier_destroy(speckv_tier_t* tier) {
     delete tier;
 }
 
+// d_group_len (device, optional): group i is the first min(d_group_len[i], group_elems) elements of its block
 static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, const uint32_t* d_block_table,
-                                         speckv_dtype_t dtype, size_t group_elems, size_t n_groups,
-                                         const uint64_t* h_block_ids, void* cuda_stream) {
+                                         const uint32_t* d_group_len, speckv_dtype_t dtype, size_t group_elems,
+                                         size_t n_groups, const uint64_t* h_block_ids, void* cuda_stream) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
     if (!tier || !h_block_ids || (!d_in && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0 ||
         group_elems >= (1ull << 31))
@@ -348,7 +356,8 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
     Tier& t = tier->t;
     std::lock_guard<std::mutex> lk(t.mu);
     const int scheme = t.scheme;
-    if (scheme == SPECKV_COMP_FP16 && (d_block_table || dtype == SPECKV_DTYPE_F32)) return SPECKV_ERR_INVAL;   // raw passthrough: no gather form
+    if (scheme == SPECKV_COMP_FP16 && (d_block_table || d_group_len || dtype == SPECKV_DTYPE_F32))
+        return SPECKV_ERR_INVAL;   // raw passthrough: no gather or ragged form
     const size_t slot = speckv_ext_slot_bytes(group_elems, (speckv_comp_scheme_t)scheme);
     const size_t esz = dtype == SPECKV_DTYPE_F32 ? 4 : 2;
     const size_t cg = tier_chunk_groups(slot, n_groups);
@@ -381,7 +390,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
             r.comp_bytes = t.h_comp[b][i];
             r.scale = t.h_scales[b][i];
             r.group_elems = (uint32_t)group_elems;
-            r.dtype = (int)dtype | (scheme << 8);
+            r.dtype = (int)dtype | (scheme << 8) | (d_group_len ? BlockRec::kRagged : 0);
             if (t.blocks.exchange(h_block_ids[g0 + i], r, &old)) {
                 t.stats.used_bytes -= ((uint64_t)old.comp_bytes + 15u) & ~15ull;
                 // an id listed twice in this chunk: its first copy is part of the transfer in flight, so its
@@ -406,6 +415,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         // paged form: the chunk's groups are the cache blocks its slice of the block table names
         a.in = d_block_table ? d_in : (const void*)((const char*)d_in + g0 * group_elems * esz);
         a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
+        a.group_len = d_group_len ? d_group_len + g0 : nullptr;   // ragged: slots + scan + pack (no packed emission)
         a.payload = t.d_slots[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
@@ -448,10 +458,19 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         if (rc == SPECKV_OK && e2 != cudaSuccess) rc = status_of(e2);
     }
     if ((e = cudaGetLastError()) != cudaSuccess && rc == SPECKV_OK) rc = status_of(e);
+    uint64_t raw = (uint64_t)n_groups * group_elems * esz;
+    if (rc == SPECKV_OK && d_group_len) {   // ragged: count the valid bytes (the lengths live on the device)
+        std::vector<uint32_t> len(n_groups);
+        e = cudaMemcpyAsync(len.data(), d_group_len, n_groups * 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) rc = status_of(e);
+        raw = 0;
+        for (uint32_t l : len) raw += (uint64_t)std::min<size_t>(l, group_elems) * esz;
+    }
     const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (rc == SPECKV_OK) {
         t.stats.blocks = t.blocks.size();
-        t.stats.bytes_offloaded_raw += (uint64_t)n_groups * group_elems * esz;
+        t.stats.bytes_offloaded_raw += raw;
         t.stats.bytes_offloaded_stored += stored;
         t.stats.last_offload_ms = ms;
         t.stats.last_offload_stored_bytes = stored;
@@ -461,14 +480,21 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
 
 speckv_status_t speckv_ext_tier_offload(speckv_tier_t* tier, const void* d_in, speckv_dtype_t dtype, size_t group_elems,
                                         size_t n_groups, const uint64_t* h_block_ids, void* cuda_stream) {
-    return tier_offload_impl(tier, d_in, nullptr, dtype, group_elems, n_groups, h_block_ids, cuda_stream);
+    return tier_offload_impl(tier, d_in, nullptr, nullptr, dtype, group_elems, n_groups, h_block_ids, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_offload_paged(speckv_tier_t* tier, const void* d_cache, const uint32_t* d_block_table,
                                               speckv_dtype_t dtype, size_t group_elems, size_t n_blocks,
                                               const uint64_t* h_block_ids, void* cuda_stream) {
     if (!d_block_table && n_blocks) return SPECKV_ERR_INVAL;
-    return tier_offload_impl(tier, d_cache, d_block_table, dtype, group_elems, n_blocks, h_block_ids, cuda_stream);
+    return tier_offload_impl(tier, d_cache, d_block_table, nullptr, dtype, group_elems, n_blocks, h_block_ids, cuda_stream);
+}
+
+speckv_status_t speckv_ext_tier_offload_ragged(speckv_tier_t* tier, const void* d_in, const uint32_t* d_block_table,
+                                               const uint32_t* d_group_len, speckv_dtype_t dtype, size_t group_elems,
+                                               size_t n_blocks, const uint64_t* h_block_ids, void* cuda_stream) {
+    if (!d_group_len && n_blocks) return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL;
+    return tier_offload_impl(tier, d_in, d_block_table, d_group_len, dtype, group_elems, n_blocks, h_block_ids, cuda_stream);
 }
 
 static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_groups,
@@ -486,8 +512,13 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
     if (e != cudaSuccess) return status_of(e);
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     const auto t0 = std::chrono::steady_clock::now();
-    uint64_t moved = 0;
+    uint64_t moved = 0, raw = 0;
     size_t chunk = 0;
+    size_t oel_pending[Tier::kBuf] = {};   // decoded lengths of a chunk with ragged blocks, waiting in h_oel[b]
+    auto take_oel = [&](int b) {
+        for (size_t i = 0; i < oel_pending[b]; ++i) raw += (uint64_t)t.h_oel[b][i] * esz;
+        oel_pending[b] = 0;
+    };
     for (size_t g0 = 0, ng = 0; g0 < n_groups; g0 += ng, ++chunk) {
         ng = std::min(cg, n_groups - g0);
         const int b = (int)(chunk % Tier::kBuf);
@@ -496,6 +527,8 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
         // H2D copies and decompress have completed
         if ((e = cudaStreamSynchronize(t.copy_st[b])) != cudaSuccess) return status_of(e);
         cudaEventSynchronize(t.ev_kernel[b]);
+        take_oel(b);
+        bool any_ragged = false;
         // host: look the blocks up, lay them out back to back in the staging buffer (in request order)
         // and merge copies whose pool ranges are contiguous
         uint64_t dst = 0;
@@ -505,6 +538,7 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
             const BlockRec* rec = t.blocks.find(h_block_ids[g0 + i]);
             if (!rec || rec->group_elems != group_elems) return SPECKV_ERR_GENERAL;   // unknown, raw, or other geometry
             const BlockRec& r = *rec;
+            any_ragged |= r.ragged();
             if (scheme < 0) scheme = r.scheme();
             else if (r.scheme() != scheme) {
                 ng = i;
@@ -545,14 +579,23 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
         a.scheme = scheme;
         a.sm_count = current_sm_count();
         if (scheme == SPECKV_COMP_FP16 && (d_block_table || dtype == SPECKV_DTYPE_F32)) return SPECKV_ERR_INVAL;
+        // a chunk holding ragged blocks counts what was decoded; otherwise every block is a whole group
+        if (any_ragged) a.out_elems = t.d_oel[b];
         if ((e = launch_decompress(a, st)) != cudaSuccess) return status_of(e);
+        if (any_ragged) {
+            if ((e = cudaMemcpyAsync(t.h_oel[b], t.d_oel[b], ng * 4, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return status_of(e);
+            oel_pending[b] = ng;
+        } else {
+            raw += (uint64_t)ng * group_elems * esz;
+        }
         cudaEventRecord(t.ev_kernel[b], st);
     }
     e = cudaStreamSynchronize(st);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) return status_of(e);
+    for (int b = 0; b < Tier::kBuf; ++b) take_oel(b);
     const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    t.stats.bytes_restored_raw += (uint64_t)n_groups * group_elems * esz;
+    t.stats.bytes_restored_raw += raw;
     t.stats.bytes_restored_stored += moved;
     t.stats.last_restore_ms = ms;
     t.stats.last_restore_stored_bytes = moved;

@@ -64,6 +64,28 @@ class HostTier:
                                                       cache[0].numel(), ids.size, ids.ctypes.data, _stream()),
                   "speckv_ext_tier_offload_paged")
 
+    def offload_ragged(self, x: torch.Tensor, group_elems: int, lengths: torch.Tensor, block_ids: np.ndarray,
+                       block_table: Optional[torch.Tensor] = None) -> None:
+        """Store the filled prefix of blocks: block i (block block_table[i] of x, or block i of x without a table) is
+        stored from its first min(lengths[i], group_elems) elements.  lengths: CUDA int32 element counts.  Restores
+        write those elements back and leave the rest of each destination block untouched."""
+        assert x.is_cuda and x.is_contiguous() and x.numel() % group_elems == 0
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
+        lengths = lengths.to(device=x.device, dtype=torch.int32).contiguous()
+        assert ids.size == lengths.numel()
+        if bool((lengths < 0).any()):   # the offload synchronises anyway; a negative length would store the whole block
+            raise ValueError("offload_ragged: negative length")
+        table = None
+        if block_table is not None:
+            table = block_table.to(device=x.device, dtype=torch.int32).contiguous()
+            assert ids.size == table.numel()
+        else:
+            assert ids.size == x.numel() // group_elems
+        with torch.cuda.device(x.device):
+            check(lib().speckv_ext_tier_offload_ragged(self._h, x.data_ptr(), table.data_ptr() if table is not None else None,
+                                                       lengths.data_ptr(), _DTYPES[x.dtype], group_elems, ids.size,
+                                                       ids.ctypes.data, _stream()), "speckv_ext_tier_offload_ragged")
+
     def restore_blocks(self, block_ids: np.ndarray, cache: torch.Tensor, block_table: torch.Tensor) -> torch.Tensor:
         """Paged form: decompress the stored blocks `block_ids` straight into cache blocks `block_table`."""
         assert cache.is_cuda and cache.is_contiguous()

@@ -115,12 +115,23 @@ class CxlSpeckvKVAllocator:
 
     # ---- additive: vLLM block tables (SURVEY.md section 8f row 1) ----
     @staticmethod
-    def offload_kv_blocks(kv_cache, block_table, tier, block_ids=None):
+    def offload_kv_blocks(kv_cache, block_table, tier, block_ids=None, num_tokens=None):
         """Compress the cache blocks `block_table` (CUDA int32 tensor of block numbers) of a paged KV cache
         tensor ([num_blocks, block_size, kv_heads, head_dim], contiguous) out to the host tier, reading them
-        in place.  They are stored under `block_ids` (default: the block numbers themselves)."""
+        in place.  They are stored under `block_ids` (default: the block numbers themselves).
+
+        `num_tokens` (optional, one entry per block of `block_table`, tensor or sequence): the filled tokens of each
+        block.  Only they are stored -- the stale K/V a reused block holds behind them takes no part -- and a restore
+        writes them back and leaves the rest of the block as it is.  None stores whole blocks."""
         ids = block_table.cpu().numpy().astype("uint64") if block_ids is None else block_ids
-        tier.offload_blocks(kv_cache, block_table, ids)
+        if num_tokens is None:
+            tier.offload_blocks(kv_cache, block_table, ids)
+            return
+        import torch
+        token_elems = kv_cache[0, 0].numel()   # kv_heads x head_dim: one token of the block is a contiguous row
+        lengths = torch.as_tensor(num_tokens, device=kv_cache.device).to(torch.int64) * token_elems
+        lengths = lengths.clamp_(0, kv_cache[0].numel()).to(torch.int32)
+        tier.offload_ragged(kv_cache, kv_cache[0].numel(), lengths, ids, block_table=block_table)
 
     @staticmethod
     def restore_kv_blocks(kv_cache, block_table, tier, block_ids=None):

@@ -81,7 +81,10 @@ SPECKV_API speckv_status_t speckv_ext_compress(const void* d_in, speckv_dtype_t 
  * odd trailing byte ignored, count 0 emits nothing), mod-256 prefix sum
  * (:260-273), (float)q / 127.0f * scale (:275-284) rounded to `dtype`.
  * At most group_elems elements are written per group at d_out + g*group_elems;
- * d_out_elems[g] (optional, may be NULL) receives the number produced. */
+ * d_out_elems[g] (optional, may be NULL) receives the number produced.  A ragged
+ * group (speckv_ext_compress_ragged) decodes to its n elements: the destination
+ * past them is left untouched.  The same holds for every decode call below
+ * (_indexed, _routed, _scatter, the tier's restores). */
 SPECKV_API speckv_status_t speckv_ext_decompress(const void* d_payload, size_t slot_bytes,
                                       const float* d_scales, const uint32_t* d_comp_bytes,
                                       size_t group_elems, size_t n_groups,
@@ -127,6 +130,21 @@ SPECKV_API speckv_status_t speckv_ext_decompress_scatter(const void* d_payload, 
                                                          size_t group_elems, speckv_dtype_t dtype, void* d_cache,
                                                          uint32_t* d_out_elems, speckv_comp_scheme_t scheme,
                                                          void* cuda_stream);
+
+/* Ragged groups: the filled prefix of each block.  Group i encodes the first min(d_group_len[i], group_elems)
+ * elements of block d_block_table[i] (or of block i when d_block_table is NULL); lengths above group_elems are
+ * clamped to it, a length of 0 gives scale 1.0 and comp_bytes 0.  Bit-exact with FPGACacheEngine::compress on
+ * that prefix (cache_engine.cpp:40-82 takes a vector of any length): the elements behind it -- stale K/V of an
+ * earlier request in a reused block -- take no part in the scale and never reach the payload.  d_group_len is a
+ * DEVICE array, so the call needs no host synchronisation and can be captured into a CUDA graph.  Schemes 1-4
+ * (FP16 -> SPECKV_ERR_INVAL).  Decoding needs no new call: the decoders produce n elements.  The byte counters of
+ * speckv_ext_get_stats / speckv_ext_engine_stats count group capacity (group_elems) for ragged calls, because the
+ * lengths live on the device. */
+SPECKV_API speckv_status_t speckv_ext_compress_ragged(const void* d_in, const uint32_t* d_block_table,
+                                                      const uint32_t* d_group_len, speckv_dtype_t dtype,
+                                                      size_t group_elems, size_t n_groups, void* d_payload,
+                                                      size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
+                                                      speckv_comp_scheme_t scheme, void* cuda_stream);
 
 /* Same two operations on HOST buffers: chunks are staged through device
  * buffers on internal streams (H2D, kernel, D2H overlapped) and the call
@@ -258,6 +276,14 @@ SPECKV_API speckv_status_t speckv_ext_tier_restore_paged(speckv_tier_t* tier, co
                                                          size_t n_blocks, size_t group_elems, speckv_dtype_t dtype,
                                                          void* d_cache, const uint32_t* d_block_table,
                                                          void* cuda_stream);
+/* Ragged offload (d_block_table may be NULL: block i of d_in): block i is stored from its first
+ * min(d_group_len[i], group_elems) elements, as speckv_ext_compress_ragged encodes them.  Restores decode such a
+ * block to that many elements and leave the rest of the destination untouched.  bytes_offloaded_raw /
+ * bytes_restored_raw count the valid bytes.  The tier's scheme must be 1-4 (FP16 -> SPECKV_ERR_INVAL). */
+SPECKV_API speckv_status_t speckv_ext_tier_offload_ragged(speckv_tier_t* tier, const void* d_in,
+                                                          const uint32_t* d_block_table, const uint32_t* d_group_len,
+                                                          speckv_dtype_t dtype, size_t group_elems, size_t n_blocks,
+                                                          const uint64_t* h_block_ids, void* cuda_stream);
 /* Bring blocks back: output group i (d_out + i*group_elems) = decompressed block h_block_ids[i].
  * Unknown id -> SPECKV_ERR_GENERAL.  Returns when d_out is complete. */
 SPECKV_API speckv_status_t speckv_ext_tier_restore(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_groups,
