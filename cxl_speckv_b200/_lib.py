@@ -143,6 +143,10 @@ def lib() -> C.CDLL:
     L.speckv_ext_tier_offload_ragged.argtypes = [vp, vp, vp, vp, C.c_int, sz, sz, vp, vp]
     L.speckv_ext_tier_offload_ragged.restype = C.c_int
     L.speckv_ext_tier_drop.argtypes = [vp, vp, sz]; L.speckv_ext_tier_drop.restype = C.c_int
+    L.speckv_ext_tier_enable_fetch.argtypes = [vp, vp]; L.speckv_ext_tier_enable_fetch.restype = C.c_int
+    L.speckv_ext_tier_fetch_workspace_bytes.argtypes = [sz, sz]; L.speckv_ext_tier_fetch_workspace_bytes.restype = sz
+    L.speckv_ext_tier_fetch.argtypes = [vp, vp, vp, sz, sz, C.c_int, C.c_int, vp, vp, vp, vp, vp, sz, vp]
+    L.speckv_ext_tier_fetch.restype = C.c_int
     L.speckv_ext_tier_get_stats.argtypes = [vp, C.POINTER(TierStats)]; L.speckv_ext_tier_get_stats.restype = None
     L.speckv_ext_atu_create.argtypes = [C.c_uint32, C.POINTER(vp)]; L.speckv_ext_atu_create.restype = C.c_int
     L.speckv_ext_atu_destroy.argtypes = [vp]; L.speckv_ext_atu_destroy.restype = None

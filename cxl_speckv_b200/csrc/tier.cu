@@ -21,6 +21,7 @@
 #include "../../include/speckv_ext.h"
 #include "device_ctx.h"
 #include "kv_codec.h"
+#include "tier_fetch.h"
 
 namespace speckv {
 
@@ -34,11 +35,13 @@ constexpr uint32_t kTierPage = 4096;
 // exclusive scan of the 16-byte-rounded payload sizes, one CTA of 32 warps: every warp scans one contiguous
 // segment tile by tile with no block barrier in between (its loads do not depend on the running sum, so they
 // pipeline), the 32 segment totals are combined once and added in a second pass (the 44 us of a
-// tile-serial scan with three block barriers per 1024 sizes was 12 % of a paged offload chunk)
+// tile-serial scan with three block barriers per 1024 sizes was 12 % of a paged offload chunk).
+// n_dev (optional, device): only the first min(*n_dev, n) sizes are scanned (the device fetch's request count).
 __global__ void __launch_bounds__(1024)
-pack_offsets_kernel(const uint32_t* __restrict__ comp_bytes, uint32_t n, uint64_t* __restrict__ offsets,
-                    uint64_t* __restrict__ total) {
+pack_offsets_kernel(const uint32_t* __restrict__ comp_bytes, uint32_t n, const uint32_t* __restrict__ n_dev,
+                    uint64_t* __restrict__ offsets, uint64_t* __restrict__ total) {
     __shared__ uint64_t warp_total[32];
+    if (n_dev) n = min(n, *n_dev);
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const uint32_t seg = ((n + 31u) / 32u + 31u) & ~31u;          // per-warp segment, a multiple of 32
     const uint32_t s0 = min(n, (uint32_t)wid * seg), s1 = min(n, s0 + seg);
@@ -83,17 +86,6 @@ pack_kernel(const uint8_t* __restrict__ slots, size_t slot_bytes, const uint32_t
     }
 }
 
-struct BlockRec {
-    uint64_t pool_off;
-    uint32_t comp_bytes;   // bytes held in the pool (payload bytes, or the raw size for raw blocks)
-    float scale;
-    uint32_t group_elems;  // 0 for raw (uncompressed) blocks
-    int dtype;             // speckv_dtype_t | scheme << 8 (the scheme the block was stored under) | kRagged; -1 = empty map entry
-    int scheme() const { return (dtype >> 8) & 0xff; }
-    bool ragged() const { return (dtype & kRagged) != 0; }
-    static constexpr int kRagged = 1 << 16;   // stored from a prefix of its block: decodes to fewer than group_elems elements
-};
-
 struct Extent {
     uint64_t off, len;
 };
@@ -102,12 +94,14 @@ struct Extent {
 // linear probing, backward-shift deletion, software prefetch for batches.  One record per 4 KiB page at the
 // paged geometry (a million per offload call): with std::unordered_map the host bookkeeping (a node
 // allocation and several cache misses per page) took longer than the PCIe copy it overlaps.
+// With tracking on (the tier keeps a device copy for speckv_ext_tier_fetch) every slot a call writes is logged, so
+// that only those go to the device; a grow marks the whole table.
 class BlockMap {
 public:
     BlockRec* find(uint64_t key) {
         if (cap_ == 0) return nullptr;
         for (size_t i = slot_of(key);; i = (i + 1) & (cap_ - 1)) {
-            if (tab_[i].val.dtype == kEmpty) return nullptr;
+            if (tab_[i].val.dtype == kDirEmpty) return nullptr;
             if (tab_[i].key == key) return &tab_[i].val;
         }
     }
@@ -115,15 +109,17 @@ public:
     bool exchange(uint64_t key, const BlockRec& r, BlockRec* old) {
         if ((size_ + 1) * 10 > cap_ * 7) grow(cap_ ? cap_ * 2 : 1024);
         for (size_t i = slot_of(key);; i = (i + 1) & (cap_ - 1)) {
-            if (tab_[i].val.dtype == kEmpty) {
+            if (tab_[i].val.dtype == kDirEmpty) {
                 tab_[i].key = key;
                 tab_[i].val = r;
                 ++size_;
+                mark(i);
                 return false;
             }
             if (tab_[i].key == key) {
                 if (old) *old = tab_[i].val;
                 tab_[i].val = r;
+                mark(i);
                 return true;
             }
         }
@@ -133,19 +129,21 @@ public:
         if (cap_ == 0) return false;
         size_t i = slot_of(key);
         for (;; i = (i + 1) & (cap_ - 1)) {
-            if (tab_[i].val.dtype == kEmpty) return false;
+            if (tab_[i].val.dtype == kDirEmpty) return false;
             if (tab_[i].key == key) break;
         }
         // backward shift: pull later entries of the probe run into the hole
         for (size_t j = (i + 1) & (cap_ - 1);; j = (j + 1) & (cap_ - 1)) {
-            if (tab_[j].val.dtype == kEmpty) break;
+            if (tab_[j].val.dtype == kDirEmpty) break;
             const size_t home = slot_of(tab_[j].key);
             if (((j - home) & (cap_ - 1)) >= ((j - i) & (cap_ - 1))) {
                 tab_[i] = tab_[j];
+                mark(i);
                 i = j;
             }
         }
-        tab_[i].val.dtype = kEmpty;
+        tab_[i].val.dtype = kDirEmpty;
+        mark(i);
         --size_;
         return true;
     }
@@ -158,32 +156,48 @@ public:
         if (cap_) __builtin_prefetch(&tab_[slot_of(key)]);
     }
     size_t size() const { return size_; }
+    size_t capacity() const { return cap_; }
+    const DirEntry* entries() const { return tab_.data(); }
+
+    // dirty log for the device copy
+    void set_tracking(bool on) { track_ = on; }
+    void mark_all() {
+        if (track_) {
+            all_dirty_ = true;
+            dirty_.clear();
+        }
+    }
+    bool all_dirty() const { return all_dirty_; }
+    const std::vector<size_t>& dirty() const { return dirty_; }
+    void clear_dirty() {
+        dirty_.clear();
+        all_dirty_ = false;
+    }
 
 private:
-    static constexpr int kEmpty = -1;
-    struct Entry {
-        uint64_t key;
-        BlockRec val;
-    };
-    size_t slot_of(uint64_t k) const {
-        k ^= k >> 33;
-        k *= 0xff51afd7ed558ccdull;
-        k ^= k >> 33;
-        return (size_t)k & (cap_ - 1);
+    size_t slot_of(uint64_t k) const { return (size_t)dir_hash(k) & (cap_ - 1); }
+    void mark(size_t i) {
+        if (track_ && !all_dirty_) dirty_.push_back(i);
     }
     void grow(size_t ncap) {
-        std::vector<Entry> old;
+        std::vector<DirEntry> old;
         old.swap(tab_);
-        Entry e{};
-        e.val.dtype = kEmpty;
+        DirEntry e{};
+        e.val.dtype = kDirEmpty;
         tab_.assign(ncap, e);
         cap_ = ncap;
         size_ = 0;
-        for (const Entry& o : old)
-            if (o.val.dtype != kEmpty) exchange(o.key, o.val, nullptr);
+        if (track_) {   // slots all move: the device gets the whole table
+            all_dirty_ = true;
+            dirty_.clear();
+        }
+        for (const DirEntry& o : old)
+            if (o.val.dtype != kDirEmpty) exchange(o.key, o.val, nullptr);
     }
-    std::vector<Entry> tab_;
+    std::vector<DirEntry> tab_;
     size_t cap_ = 0, size_ = 0;
+    bool track_ = false, all_dirty_ = false;
+    std::vector<size_t> dirty_;
 };
 constexpr size_t kMapPrefetch = 16;   // look-ups in flight when a call walks a list of block ids
 
@@ -216,6 +230,17 @@ struct Tier {
     size_t cap_groups = 0, cap_slot_bytes = 0;           // per buffer
     int scheme = SPECKV_COMP_INT8_DELTA_RLE;             // what new offloads are stored under (speckv_ext_tier_set_scheme)
     speckv_tier_stats_t stats = {};
+    // device copy of the block directory (speckv_ext_tier_enable_fetch); d_dir stays null while fetch is off, and
+    // then nothing below is touched
+    DeviceDir* d_dir = nullptr;                          // header the fetch kernels read the table through
+    DeviceDir* h_dir = nullptr;                          // pinned source of header writes
+    DirEntry* d_table = nullptr;
+    size_t d_table_cap = 0;
+    DirUpdate* h_upd = nullptr;                          // pinned staging of changed slots
+    DirUpdate* d_upd = nullptr;
+    size_t upd_cap = 0;
+    const uint8_t* d_pool = nullptr;                     // device address of the pinned pool
+    cudaStream_t dir_st = nullptr;                       // drop's updates (drop takes no stream)
 
     size_t alloc_pool(size_t len) {   // first fit in the free list, else bump; returns SIZE_MAX when full
         for (size_t i = 0; i < free_list.size(); ++i) {
@@ -288,6 +313,70 @@ struct Tier {
         cap_slot_bytes = groups * slot_bytes;
         return cudaSuccess;
     }
+
+    // Bring the device directory up to date with the host map on st and wait for it.  Changed slots travel as
+    // (slot, entry) records and are applied by a scatter kernel; after a grow, or when many slots changed, the whole
+    // table goes.  A grown table gets a new device table and the header is pointed at it; the old one is freed once
+    // that has completed, so a graph captured before the grow keeps working.
+    cudaError_t sync_dir(cudaStream_t st) {
+        if (!d_dir) return cudaSuccess;
+        const size_t cap = blocks.capacity();
+        const std::vector<size_t>& dirty = blocks.dirty();
+        cudaError_t e = cudaSuccess;
+        DirEntry* old = nullptr;
+        const size_t old_cap = d_table_cap;
+        const bool moved = cap != d_table_cap;   // a grow (or the first upload): a new device table
+        if (moved || blocks.all_dirty() || dirty.size() * 4 >= cap) {
+            if (moved) {
+                DirEntry* nt = nullptr;
+                if ((e = cudaMalloc((void**)&nt, cap * sizeof(DirEntry))) != cudaSuccess) return e;
+                old = d_table;
+                d_table = nt;
+                d_table_cap = cap;
+                *h_dir = DeviceDir{d_table, cap - 1, d_pool};
+            }
+            e = cudaMemcpyAsync(d_table, blocks.entries(), cap * sizeof(DirEntry), cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess && moved) e = cudaMemcpyAsync(d_dir, h_dir, sizeof(DeviceDir), cudaMemcpyHostToDevice, st);
+        } else if (!dirty.empty()) {
+            const size_t n = dirty.size();
+            if (n > upd_cap) {
+                cudaFreeHost(h_upd);
+                cudaFree(d_upd);
+                h_upd = nullptr;
+                d_upd = nullptr;
+                upd_cap = 0;
+                const size_t c = std::max(n, (size_t)4096);
+                if ((e = cudaHostAlloc((void**)&h_upd, c * sizeof(DirUpdate), cudaHostAllocDefault)) != cudaSuccess) return e;
+                if ((e = cudaMalloc((void**)&d_upd, c * sizeof(DirUpdate))) != cudaSuccess) return e;
+                upd_cap = c;
+            }
+            const DirEntry* tab = blocks.entries();
+            for (size_t k = 0; k < n; ++k) h_upd[k] = DirUpdate{dirty[k], tab[dirty[k]]};
+            e = cudaMemcpyAsync(d_upd, h_upd, n * sizeof(DirUpdate), cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = launch_dir_apply(d_dir, d_upd, n, st);
+        }
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) {
+            if (moved) {   // the header may still name the old table: keep it, retry the whole upload next time
+                cudaFree(d_table);
+                d_table = old;
+                d_table_cap = old_cap;
+            }
+            return e;
+        }
+        if (old) cudaFree(old);
+        blocks.clear_dirty();
+        return cudaSuccess;
+    }
+    void release_dir() {
+        cudaFree(d_dir); cudaFree(d_table); cudaFree(d_upd);
+        cudaFreeHost(h_dir); cudaFreeHost(h_upd);
+        if (dir_st) cudaStreamDestroy(dir_st);
+        d_dir = nullptr; d_table = nullptr; d_upd = nullptr; h_dir = nullptr; h_upd = nullptr; dir_st = nullptr;
+        d_table_cap = upd_cap = 0;
+        blocks.set_tracking(false);
+        blocks.clear_dirty();
+    }
 };
 
 }  // namespace speckv
@@ -334,6 +423,7 @@ void speckv_ext_tier_destroy(speckv_tier_t* tier) {
     speckv::runtime_unbind_tier(tier);   // pools bound to this tier (speckv_ext_bind_pool) forget it before it is freed
     Tier& t = tier->t;
     t.release_staging();
+    t.release_dir();
     for (int b = 0; b < Tier::kBuf; ++b) {
         if (t.copy_st[b]) cudaStreamDestroy(t.copy_st[b]);
         if (t.ev_kernel[b]) cudaEventDestroy(t.ev_kernel[b]);
@@ -436,7 +526,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
             if ((e = launch_compress(a, st)) != cudaSuccess) { rc = status_of(e); break; }
         } else {
             if ((e = launch_compress(a, st)) != cudaSuccess) { rc = status_of(e); break; }
-            pack_offsets_kernel<<<1, 1024, 0, st>>>(t.d_comp[b], (uint32_t)ng, t.d_offsets[b], t.d_total[b]);
+            pack_offsets_kernel<<<1, 1024, 0, st>>>(t.d_comp[b], (uint32_t)ng, nullptr, t.d_offsets[b], t.d_total[b]);
             const int grid = (int)std::min<size_t>((ng + 7) / 8, (size_t)current_sm_count() * 8);
             pack_kernel<<<grid, kPackThreads, 0, st>>>(t.d_slots[b], slot, t.d_comp[b], t.d_offsets[b], (uint32_t)ng, t.d_packed[b]);
             count_launch(2);
@@ -457,6 +547,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         cudaError_t e2 = cudaStreamSynchronize(t.copy_st[b]);
         if (rc == SPECKV_OK && e2 != cudaSuccess) rc = status_of(e2);
     }
+    if ((e = t.sync_dir(st)) != cudaSuccess && rc == SPECKV_OK) rc = status_of(e);   // the records this call changed
     if ((e = cudaGetLastError()) != cudaSuccess && rc == SPECKV_OK) rc = status_of(e);
     uint64_t raw = (uint64_t)n_groups * group_elems * esz;
     if (rc == SPECKV_OK && d_group_len) {   // ragged: count the valid bytes (the lengths live on the device)
@@ -627,7 +718,7 @@ speckv_status_t speckv_ext_tier_drop(speckv_tier_t* tier, const uint64_t* h_bloc
         t.blocks.erase(h_block_ids[i]);
     }
     t.stats.blocks = t.blocks.size();
-    return SPECKV_OK;
+    return status_of(t.sync_dir(t.dir_st));
 }
 
 // ---- descriptor interface (driver/uapi/speckv_ioctl.h:10-15, host/src/speckv_driver.cpp:24-47) ----
@@ -681,6 +772,8 @@ speckv_status_t speckv_ext_submit_dma_batch(speckv_tier_t* tier, const speckv_dm
                     rc = status_of(cudaMemcpyAsync(dev, t.pool + it->pool_off, kTierPage, cudaMemcpyHostToDevice, st));
                 }
             }
+            const speckv_status_t rd = status_of(t.sync_dir(st));
+            if (rc == SPECKV_OK) rc = rd;
             if (rc == SPECKV_OK) rc = status_of(cudaStreamSynchronize(st));
             t.stats.blocks = t.blocks.size();
         }
@@ -703,6 +796,100 @@ void speckv_ext_tier_get_stats(speckv_tier_t* tier, speckv_tier_stats_t* out) {
     if (!tier || !out) return;
     std::lock_guard<std::mutex> lk(tier->t.mu);
     *out = tier->t.stats;
+}
+
+// ---- device-side fetch -----------------------------------------------------------------------------------------
+speckv_status_t speckv_ext_tier_enable_fetch(speckv_tier_t* tier, void* cuda_stream) {
+    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
+    if (!tier) return SPECKV_ERR_INVAL;
+    Tier& t = tier->t;
+    std::lock_guard<std::mutex> lk(t.mu);
+    if (t.d_dir) return SPECKV_OK;
+    int dev = -1;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return status_of(e);
+    if (dev != t.device) return SPECKV_ERR_INVAL;
+    // the fetch kernels read the pinned pool directly: it needs a device address
+    int uva = 0, can_map = 0;
+    cudaDeviceGetAttribute(&uva, cudaDevAttrUnifiedAddressing, dev);
+    cudaDeviceGetAttribute(&can_map, cudaDevAttrCanMapHostMemory, dev);
+    if (!uva || !can_map) return SPECKV_ERR_DRIVER;
+    void* dpool = nullptr;
+    if ((e = cudaHostGetDevicePointer(&dpool, t.pool, 0)) != cudaSuccess) return status_of(e);
+    t.d_pool = static_cast<const uint8_t*>(dpool);
+    e = cudaMalloc((void**)&t.d_dir, sizeof(DeviceDir));
+    if (e == cudaSuccess) e = cudaHostAlloc((void**)&t.h_dir, sizeof(DeviceDir), cudaHostAllocDefault);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&t.dir_st, cudaStreamNonBlocking);
+    if (e == cudaSuccess) {
+        t.blocks.reserve(t.blocks.size());   // a table of at least 1024 slots: the device table is never empty
+        t.blocks.set_tracking(true);
+        t.blocks.mark_all();
+        e = t.sync_dir(static_cast<cudaStream_t>(cuda_stream));
+    }
+    if (e != cudaSuccess) {
+        t.release_dir();
+        return status_of(e);
+    }
+    return SPECKV_OK;
+}
+
+size_t speckv_ext_tier_fetch_workspace_bytes(size_t max_requests, size_t group_elems) {
+    // [staging: one slot per request][offsets u64][pool offsets u64][total u64][sizes u32][scales f32]
+    return max_requests * (speckv_ext_slot_bytes(group_elems, SPECKV_COMP_INT8_DELTA_RLE) + 24) + 8;
+}
+
+speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
+                                      size_t max_requests, size_t group_elems, speckv_dtype_t dtype,
+                                      speckv_comp_scheme_t scheme, void* d_out, const uint32_t* d_block_table,
+                                      uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
+                                      size_t workspace_bytes, void* cuda_stream) {
+    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
+    if (!tier || dtype < 0 || dtype > 2 || (int)scheme < 1 || (int)scheme > 4 || group_elems == 0 ||
+        group_elems >= (1ull << 31) || max_requests >= (1ull << 31))
+        return SPECKV_ERR_INVAL;
+    Tier& t = tier->t;
+    std::lock_guard<std::mutex> lk(t.mu);
+    if (!t.d_dir) return SPECKV_ERR_INVAL;   // speckv_ext_tier_enable_fetch first
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev != t.device) return SPECKV_ERR_INVAL;
+    if (max_requests == 0) return SPECKV_OK;
+    if (!d_block_ids || !d_out || !d_workspace || (reinterpret_cast<uintptr_t>(d_workspace) & 15) ||
+        workspace_bytes < speckv_ext_tier_fetch_workspace_bytes(max_requests, group_elems))
+        return SPECKV_ERR_INVAL;
+    const size_t n = max_requests;
+    const size_t slot = speckv_ext_slot_bytes(group_elems, SPECKV_COMP_INT8_DELTA_RLE);   // the largest of any scheme
+    uint8_t* staging = static_cast<uint8_t*>(d_workspace);
+    uint64_t* offsets = reinterpret_cast<uint64_t*>(staging + n * slot);
+    uint64_t* src_off = offsets + n;
+    uint64_t* total = src_off + n;
+    uint32_t* comp = reinterpret_cast<uint32_t*>(total + 1);
+    float* scales = reinterpret_cast<float*>(comp + n);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    cudaError_t e = launch_fetch_lookup(t.d_dir, d_block_ids, d_n_requests, (uint32_t)n, (uint32_t)group_elems, dtype,
+                                        (int)scheme, slot, src_off, comp, scales, d_status, st);
+    if (e != cudaSuccess) return status_of(e);
+    pack_offsets_kernel<<<1, 1024, 0, st>>>(comp, (uint32_t)n, d_n_requests, offsets, total);
+    count_launch();
+    if ((e = cudaGetLastError()) != cudaSuccess) return status_of(e);
+    e = launch_fetch_gather(t.d_dir, src_off, offsets, d_n_requests, (uint32_t)n, total, staging, current_sm_count(), st);
+    if (e != cudaSuccess) return status_of(e);
+    // the staged payloads form a packed container: the codec's decoders take it as it is
+    CodecArgs a;
+    a.out = d_out;
+    a.elem_index = d_block_table;
+    a.payload = staging;
+    a.slot_offsets = offsets;
+    a.scales = scales;
+    a.comp_bytes = comp;
+    a.out_elems = d_out_elems;
+    a.n_groups_dev = d_n_requests;
+    a.slot_bytes = slot;
+    a.group_elems = (uint32_t)group_elems;
+    a.n_groups = (uint32_t)n;
+    a.dtype = dtype;
+    a.scheme = (int)scheme;
+    a.sm_count = current_sm_count();
+    return status_of(launch_decompress(a, st));
 }
 
 }  // extern "C"

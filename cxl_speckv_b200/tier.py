@@ -9,13 +9,14 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import check, lib
+from ._lib import COMP_INT8_DELTA_RLE, check, lib
 from .codec import _DTYPES, _stream
 
 
 class HostTier:
     def __init__(self, pool_bytes: int):
         self._h = C.c_void_p()
+        self._fetch_ws = {}   # fetch() workspaces by (requests, group_elems, device)
         check(lib().speckv_ext_tier_create(pool_bytes, C.byref(self._h)), "speckv_ext_tier_create")
 
     def close(self):
@@ -101,6 +102,68 @@ class HostTier:
     def drop(self, block_ids: np.ndarray) -> None:
         ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
         check(lib().speckv_ext_tier_drop(self._h, ids.ctypes.data, ids.size), "speckv_ext_tier_drop")
+
+    def enable_fetch(self) -> None:
+        """Keep a device copy of the block directory from now on, so that fetch() finds blocks without the host.
+        Call it on the tier's device (the current one when the tier was created)."""
+        check(lib().speckv_ext_tier_enable_fetch(self._h, _stream()), "speckv_ext_tier_enable_fetch")
+
+    def fetch(self, block_ids: torch.Tensor, group_elems: int, dtype: torch.dtype, scheme: int = COMP_INT8_DELTA_RLE,
+              out: Optional[torch.Tensor] = None, block_table: Optional[torch.Tensor] = None,
+              count: Optional[torch.Tensor] = None, out_elems: Optional[torch.Tensor] = None,
+              status: Optional[torch.Tensor] = None):
+        """Restore blocks named on the device (speckv_ext_tier_fetch): request i < count[0] (all of block_ids without
+        a count) decodes stored block block_ids[i] into out[i], or into cache block block_table[i] of `out` (a paged
+        cache of blocks of group_elems elements).  No host synchronisation, so a warm call can be captured into a CUDA
+        graph.  block_ids: CUDA int64 ids; count: CUDA int32 [1] (e.g. from prefetch.route); block_table: CUDA int32.
+        scheme names the decoder: 1 and 4 decode alike, so do 2 and 3; blocks stored under the other pair are not
+        served.  -> (out, out_elems int32 [n], status uint8 [n]): status 1 = served; an unserved request (unknown id,
+        other geometry, dtype or decoder, raw block) leaves its destination as it is and gets out_elems 0.  Entries
+        at and behind the count are not written.  The workspace is cached per (len(block_ids), group_elems) and
+        allocated on the first eager call of that shape: run one before capturing."""
+        if not block_ids.is_cuda or block_ids.dtype not in (torch.int64, torch.uint64) or not block_ids.is_contiguous():
+            raise TypeError("block_ids must be a contiguous CUDA int64 tensor")
+        if dtype not in _DTYPES:
+            raise TypeError(f"unsupported dtype {dtype}")
+        dev = block_ids.device
+        n = block_ids.numel()
+        if count is not None and (not count.is_cuda or count.dtype != torch.int32 or count.device != dev):
+            raise TypeError("count must be a CUDA int32 tensor on the device of block_ids")
+        if block_table is not None:
+            if out is None:
+                raise ValueError("a block table needs the cache to write into (out)")
+            if not block_table.is_cuda or block_table.dtype != torch.int32 or block_table.numel() < n or \
+                    not block_table.is_contiguous():
+                raise TypeError("block_table must be a contiguous CUDA int32 tensor with one entry per request")
+        if out is None:
+            out = torch.empty((n, group_elems), dtype=dtype, device=dev)
+        if out.dtype != dtype or out.device != dev or not out.is_contiguous() or out.numel() % group_elems or \
+                (block_table is None and out.numel() < n * group_elems):
+            raise ValueError("out must be a contiguous tensor of whole blocks of `dtype` on the device of block_ids")
+        if out_elems is None:
+            out_elems = torch.zeros(n, dtype=torch.int32, device=dev)
+        if status is None:
+            status = torch.zeros(n, dtype=torch.uint8, device=dev)
+        assert out_elems.numel() >= n and status.numel() >= n and out_elems.is_cuda and status.is_cuda
+        ws = self._workspace(n, group_elems, dev)
+        with torch.cuda.device(dev):
+            check(lib().speckv_ext_tier_fetch(self._h, block_ids.data_ptr(), count.data_ptr() if count is not None else None,
+                                              n, group_elems, _DTYPES[dtype], int(scheme), out.data_ptr(),
+                                              block_table.data_ptr() if block_table is not None else None,
+                                              out_elems.data_ptr(), status.data_ptr(), ws.data_ptr(), ws.numel(),
+                                              _stream()), "speckv_ext_tier_fetch")
+        return out, out_elems, status
+
+    def _workspace(self, n: int, group_elems: int, dev: torch.device) -> torch.Tensor:
+        key = (n, group_elems, dev)
+        ws = self._fetch_ws.get(key)
+        if ws is None:
+            if torch.cuda.is_current_stream_capturing():
+                raise RuntimeError("HostTier.fetch: no workspace for this shape yet; run one eager call before capturing")
+            ws = torch.empty(max(lib().speckv_ext_tier_fetch_workspace_bytes(n, group_elems), 1), dtype=torch.uint8,
+                             device=dev)
+            self._fetch_ws[key] = ws
+        return ws
 
     def stats(self) -> dict:
         s = _lib.TierStats()

@@ -298,6 +298,44 @@ SPECKV_API speckv_status_t speckv_ext_tier_set_scheme(speckv_tier_t* tier, speck
 SPECKV_API speckv_status_t speckv_ext_tier_drop(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n);
 SPECKV_API void speckv_ext_tier_get_stats(speckv_tier_t* tier, speckv_tier_stats_t* out);
 
+/* Device-side fetch: blocks named by ids in DEVICE memory come back without the host, so a prefetch step
+ * (speckv_ext_prefetch_emit -> speckv_ext_route_requests -> ids -> fetch) is one CUDA graph.
+ *
+ * Keep a copy of the tier's block directory in device memory from now on, so that speckv_ext_tier_fetch can find
+ * blocks without the host.  Uploads the current directory on cuda_stream and waits for it.  Idempotent; there is no
+ * disable.  While it is on, every offload and drop of this tier also updates the device copy before it returns.
+ * Must run on the tier's device (SPECKV_ERR_INVAL otherwise); SPECKV_ERR_DRIVER on a device that cannot read
+ * mapped pinned host memory (no unified addressing). */
+SPECKV_API speckv_status_t speckv_ext_tier_enable_fetch(speckv_tier_t* tier, void* cuda_stream);
+
+/* Device scratch one fetch call needs for up to max_requests blocks of group_elems elements: the staged payloads at
+ * the largest slot of any scheme plus per-request metadata,
+ *   max_requests * (speckv_ext_slot_bytes(group_elems, SPECKV_COMP_INT8_DELTA_RLE) + 24) + 8.
+ * Arithmetic only: works without a device. */
+SPECKV_API size_t speckv_ext_tier_fetch_workspace_bytes(size_t max_requests, size_t group_elems);
+
+/* Restore blocks named on the DEVICE.  Request i < *d_n_requests (all max_requests when d_n_requests is NULL) names
+ * stored block d_block_ids[i].  It is decoded into d_out + i*group_elems, or into cache block d_block_table[i] when a
+ * table is given (block numbers distinct, as for _restore_paged).  d_status[i] (optional) = 1 when the request was
+ * served, 0 when the id is not in the tier or its block does not fit the call.  A block does not fit when it has
+ * another group_elems or another dtype, when it is raw (scheme 0), or when its scheme decodes differently from
+ * `scheme`: 1 and 4 share a decoder, and so do 2 and 3.  An unserved request writes nothing to its destination and
+ * gets out_elems 0.  d_out_elems[i] (optional) = elements decoded (n for a ragged block).  Entries at and behind the
+ * count are left untouched.  No host synchronisation; capturable into a CUDA graph.  Needs speckv_ext_tier_enable_fetch
+ * first (SPECKV_ERR_INVAL otherwise), a 16-byte aligned d_workspace of workspace_bytes >=
+ * speckv_ext_tier_fetch_workspace_bytes(max_requests, group_elems), and scheme 1-4.  The workspace belongs to the
+ * call while it runs: calls in flight at the same time need their own.  The call must run on the tier's device.
+ * Ordering: a fetch reads the directory and the pool when it runs.  Offloads of the tier on the fetch's stream are
+ * ordered with it through that stream; before an offload on another stream, or a drop, synchronise the streams that
+ * still have fetches of the tier in flight.  Fetched bytes are not counted in speckv_tier_stats_t (bytes_restored_*
+ * count the host-driven restores only). */
+SPECKV_API speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_block_ids,
+                                                 const uint32_t* d_n_requests, size_t max_requests, size_t group_elems,
+                                                 speckv_dtype_t dtype, speckv_comp_scheme_t scheme, void* d_out,
+                                                 const uint32_t* d_block_table, uint32_t* d_out_elems,
+                                                 uint8_t* d_status, void* d_workspace, size_t workspace_bytes,
+                                                 void* cuda_stream);
+
 /* ---- descriptor-level interface (what the reference's ioctl client speaks) ------------------ */
 /* One transfer descriptor, identical to struct speckv_ioctl_dma_desc (driver/uapi/speckv_ioctl.h:
  * 10-15) / SpeckvDmaDesc (host/include/speckv_driver.hpp:8-13): fpga_addr names the first 4 KiB
