@@ -56,6 +56,7 @@ struct Predictor {
     float row_abs_max = 0.0f;    // max_v sum_j |W[v][j]| (rounded up): scales the error bound of the rank-one form
     uint32_t vocab = 0, emb_dim = 0, hidden = 0, layers = 0, hist_len = 0;
     int device = -1;
+    size_t smem_optin = 0;       // the device's shared memory per block (opt-in): bounds the tiled kernel's W_out tile
     // device-side prefetcher state (SpeculativePrefetcher's queue and counters, speculative_prefetcher.h:83-94)
     speckv_prefetch_request_t* d_ring = nullptr;   // the 16 most recent requests (issue_dma_prefetch, :162-172)
     unsigned long long* d_total = nullptr;         // requests emitted so far
@@ -182,6 +183,9 @@ __device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
+// Row stride of a staged W_out tile in words: 16 B aligned rows (the float4 reads below) for any hidden, bank-staggered.
+__host__ __device__ __forceinline__ uint32_t tile_ld(uint32_t hidden) { return ((hidden + 3u) & ~3u) + 4u; }
+
 // One partial per (CTA, sequence): { max, sum of exp(x - max), K values, K ids } = 2 + 2K words.
 // Geometry (host-chosen): seq_lanes lanes of a warp hold different sequence slices (S sequences each), the other
 // lane bits and the warp index select a row subset; a tile has nsub * rps rows, nsub = kScoreWarps * 32 / seq_lanes.
@@ -195,18 +199,19 @@ score_partial_kernel(const float* __restrict__ wout, uint32_t vocab, uint32_t hi
     const uint32_t rsub_per_warp = 32u / seq_lanes, nsub = kScoreWarps * rsub_per_warp;
     const uint32_t ssub = lane % seq_lanes, rsub = warp * rsub_per_warp + lane / seq_lanes;
     const uint32_t tile_rows = nsub * rps;
-    const uint32_t ld = hidden + 4;                    // row stride in words: 16 B aligned rows, bank-staggered
+    const uint32_t ld = tile_ld(hidden);
     const uint32_t sb = seq_lanes * S;                 // sequences per CTA (grid.y walks the batch)
     const uint32_t seq0 = blockIdx.y * sb + ssub * S;
     const uint32_t h4 = hidden & ~3u;
 
-    float hs[S], m[S], se[S], bv[S][K];
+    float hs[S], m[S], bv[S][K];
+    double se[S];   // sum of exp(x - max): fp64, or the many small terms of a peaked softmax round away against the top one
     uint32_t bi[S][K];
 #pragma unroll
     for (int i = 0; i < S; ++i) {
         hs[i] = seq0 + i < batch ? hvec[seq0 + i] : 0.0f;
         m[i] = -FLT_MAX;
-        se[i] = 0.0f;
+        se[i] = 0.0;
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             bv[i][k] = -FLT_MAX;
@@ -278,10 +283,10 @@ score_partial_kernel(const float* __restrict__ wout, uint32_t vocab, uint32_t hi
             for (int i = 0; i < S; ++i) {
                 const float x = acc[i];
                 if (x > m[i]) {   // online softmax: rescale the running sum to the new max
-                    se[i] *= __expf(m[i] - x);
+                    se[i] *= (double)expf(m[i] - x);
                     m[i] = x;
                 }
-                se[i] += __expf(x - m[i]);
+                se[i] += (double)expf(x - m[i]);
                 list_insert<K>(bv[i], bi[i], x, v);
             }
         }
@@ -296,7 +301,7 @@ score_partial_kernel(const float* __restrict__ wout, uint32_t vocab, uint32_t hi
     for (int i = 0; i < S; ++i) {
         float* p = park + ((size_t)rsub * sb + ssub * S + i) * PW;
         p[0] = m[i];
-        p[1] = se[i];
+        p[1] = (float)se[i];
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             p[2 + k] = bv[i][k];
@@ -309,7 +314,8 @@ score_partial_kernel(const float* __restrict__ wout, uint32_t vocab, uint32_t hi
         if (seq >= batch) continue;
         float mm = -FLT_MAX;
         for (uint32_t q = 0; q < nsub; ++q) mm = fmaxf(mm, park[((size_t)q * sb + s) * PW]);
-        float ss = 0.0f, lv[K];
+        float lv[K];
+        double ss = 0.0;
         uint32_t li[K];
 #pragma unroll
         for (int k = 0; k < K; ++k) {
@@ -318,13 +324,13 @@ score_partial_kernel(const float* __restrict__ wout, uint32_t vocab, uint32_t hi
         }
         for (uint32_t q = 0; q < nsub; ++q) {
             const float* p = park + ((size_t)q * sb + s) * PW;
-            ss += p[1] * __expf(p[0] - mm);
+            ss += (double)p[1] * (double)expf(p[0] - mm);
 #pragma unroll
             for (int k = 0; k < K; ++k) list_insert<K>(lv, li, p[2 + k], __float_as_uint(p[2 + K + k]));
         }
         float* o = partials + ((size_t)seq * gridDim.x + blockIdx.x) * PW;
         o[0] = mm;
-        o[1] = ss;
+        o[1] = (float)ss;
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             o[2 + k] = lv[k];
@@ -345,10 +351,14 @@ score_partial_kernel(const float* __restrict__ wout, uint32_t vocab, uint32_t hi
 //      than 2 err below the k-th best, every row outside the list is provably below the true k-th best: the true top-k
 //      are among the candidates;
 //   2. the candidates are re-scored with the reference's exact sequential sum and ranked by that (value, then lower id);
-//   3. the softmax denominator is summed over the approximate logits (relative error <= 2 err ~ 1e-5, far inside the
-//      1e-7 absolute tolerance on confidences of a few 1e-5);
-//   4. otherwise (near-ties wider than the list, h = 0, non-finite weights) the CTA walks the vocabulary with exact
-//      logits, online softmax and per-thread best-KC lists.
+//   3. the softmax denominator is summed over the approximate logits, then the candidates' approximate terms are
+//      replaced by their exact ones: S' = S - sum_c exp(a_c - M) + sum_c exp(x_c - M).  Every remaining term is within a
+//      factor e^(+-err) of its exact value, so |S' - S_exact| <= S_nc (e^err - 1), S_nc the sum over the other rows, and
+//      a confidence c is off by at most c |dS| / S'.  When that could exceed half the tolerance 1e-7 + 2^-22 c at the
+//      largest confidence (a peaked predictor: err grows with |h| max_v sum_j |W[v][j]|), the CTA takes the exact pass
+//      below; for near-uniform predictors (srand(1) weights: ~1e-10) the candidate pass stands;
+//   4. otherwise (near-ties wider than the list, h = 0, non-finite weights, the bound of 3) the CTA walks the vocabulary
+//      with exact logits, online softmax and per-thread best-KC lists.
 // ids are therefore the exact method's ids.  Output: one partial per sequence in score_partial_kernel's format,
 // consumed by score_merge_kernel with n_partials = 1.
 constexpr int kCandMax = 16;
@@ -396,6 +406,7 @@ score_rank1_kernel(const float* __restrict__ wout, const float* __restrict__ row
     __shared__ uint32_t s_i[kScoreWarps][KC];
     constexpr int kRowChunk = 256;
     __shared__ float s_rows[KC][kRowChunk + 1];   // (+1: the lanes read different rows at the same column)
+    __shared__ bool s_flag;                        // the candidate pass cannot bound the confidences: exact pass
     const uint32_t tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const uint32_t seq = blockIdx.x;
     if (seq >= batch) return;
@@ -447,14 +458,40 @@ score_rank1_kernel(const float* __restrict__ wout, const float* __restrict__ row
                 for (uint32_t j = 0; j < nj; ++j) acc = __fadd_rn(acc, s_rows[lane][j]);       // logits[i] += ..., in j order
             __syncthreads();
         }
-        if (warp != 0) return;
-        if (lane < nc) xv = acc;
-        float ss = lane < kScoreWarps ? s_s[lane] : 0.0f;
-        for (int o2 = 16; o2 > 0; o2 >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o2);
-        S = ss;
-    } else {
+        // ---- warp 0: swap the candidates' approximate terms for their exact ones and bound what is left ----
+        if (warp == 0) {
+            if (lane < nc) xv = acc;
+            float ss = lane < kScoreWarps ? s_s[lane] : 0.0f;
+            float ta = lane < nc ? __expf(__fmul_rn(h, __ldg(rowsum + ci)) - M) : 0.0f;   // the term summed above
+            float best = xv;
+            for (int o2 = 16; o2 > 0; o2 >>= 1) {
+                ss += __shfl_xor_sync(0xffffffffu, ss, o2);
+                ta += __shfl_xor_sync(0xffffffffu, ta, o2);
+                best = fmaxf(best, __shfl_xor_sync(0xffffffffu, best, o2));
+            }
+            // the exact terms against the exact maximum: the best candidate contributes exactly 1, so S >= 1 and no
+            // confidence can exceed 1 (a rescale by exp(M - best) rounds either way)
+            float tx = lane < nc ? expf(xv - best) : 0.0f;
+            for (int o2 = 16; o2 > 0; o2 >>= 1) tx += __shfl_xor_sync(0xffffffffu, tx, o2);
+            const float s_nc = fmaxf(ss - ta, 0.0f) * expf(M - best);   // the rows outside the list, still approximate
+            S = s_nc + tx;
+            M = best;
+            // each remaining term is within a factor e^(+-err) of its exact value: |dS| <= s_nc (e^err - 1), which moves
+            // a confidence c by at most c |dS| / S; the largest one, 1 / S, decides (the bar 1e-7 + 2^-22 c grows with c).
+            // The fp32 sum above adds its own relative error, at most (terms per accumulator + 10 tree levels) u.
+            const float c1 = 1.0f / S;
+            const float gsum = (float)((vocab + 4 * kScoreThreads - 1) / (4 * kScoreThreads) + 10) * u;
+            const float dc = c1 * (s_nc * expm1f(err) / S + gsum);
+            if (lane == 0) s_flag = !(dc <= 0.5f * (1e-7f + 2.384185791015625e-07f * c1));   // NaN -> exact pass
+        }
+        __syncthreads();
+        exact = s_flag;
+        if (!exact && warp != 0) return;
+    }
+    if (exact) {
         // ---- exact pass over the vocabulary ----
-        float m = -FLT_MAX, se = 0.0f, bv[KC];
+        float m = -FLT_MAX, bv[KC];
+        double se = 0.0;   // fp64 sums (see score_partial_kernel), fp32 exponentials
         uint32_t bi[KC];
 #pragma unroll
         for (int i = 0; i < KC; ++i) {
@@ -465,23 +502,24 @@ score_rank1_kernel(const float* __restrict__ wout, const float* __restrict__ row
             const float* w = wout + (size_t)v * hidden;
             float x = 0.0f;
             for (uint32_t j = 0; j < hidden; ++j) x = __fadd_rn(x, __fmul_rn(h, __ldg(w + j)));
+            // (accurate expf: this pass's time goes to the sequential logit sums, the approximate one would save nothing)
             if (x > m) {
-                se *= __expf(m - x);
+                se *= (double)expf(m - x);
                 m = x;
             }
-            se += __expf(x - m);
+            se += (double)expf(x - m);
             if (better(x, v, bv[KC - 1], bi[KC - 1])) list_insert<KC>(bv, bi, x, v);
         }
         float wm = m;
         for (int o2 = 16; o2 > 0; o2 >>= 1) wm = fmaxf(wm, __shfl_xor_sync(0xffffffffu, wm, o2));
-        float ws = se * __expf(m - wm);   // a thread without rows has se = 0
+        double ws = se * (double)expf(m - wm);   // a thread without rows has se = 0
         for (int o2 = 16; o2 > 0; o2 >>= 1) ws += __shfl_xor_sync(0xffffffffu, ws, o2);
         float wv;
         uint32_t wi;
         warp_select<KC>(bv, bi, lane, wv, wi);
         if (lane == 0) {
             s_m[warp] = wm;
-            s_s[warp] = ws;
+            s_s[warp] = (float)ws;
         }
         if (lane < KC) {
             s_v[warp][lane] = wv;
@@ -491,7 +529,7 @@ score_rank1_kernel(const float* __restrict__ wout, const float* __restrict__ row
         if (warp != 0) return;
         float mm = lane < kScoreWarps ? s_m[lane] : -FLT_MAX;
         for (int o2 = 16; o2 > 0; o2 >>= 1) mm = fmaxf(mm, __shfl_xor_sync(0xffffffffu, mm, o2));
-        float ss = lane < kScoreWarps ? s_s[lane] * __expf(s_m[lane] - mm) : 0.0f;
+        double ss = lane < kScoreWarps ? (double)s_s[lane] * (double)expf(s_m[lane] - mm) : 0.0;
         for (int o2 = 16; o2 > 0; o2 >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o2);
         float lv[KC];
         uint32_t li[KC];
@@ -502,7 +540,7 @@ score_rank1_kernel(const float* __restrict__ wout, const float* __restrict__ row
         }
         warp_select<KC>(lv, li, lane, xv, ci);
         M = mm;
-        S = ss;
+        S = (float)ss;
     }
     // ---- warp 0: rank by the exact order (all candidates are distinct rows) ----
     uint32_t rank = 0;
@@ -511,7 +549,7 @@ score_rank1_kernel(const float* __restrict__ wout, const float* __restrict__ row
         const uint32_t oi = __shfl_sync(0xffffffffu, ci, r);
         if (lane < KC && (uint32_t)r != lane && better(ov, oi, xv, ci)) ++rank;
     }
-    // exact maximum = the best candidate; the sum was taken against M
+    // exact maximum = the best candidate; both passes took the sum against it (M == best, the factor below is 1)
     float best = lane < KC ? xv : -FLT_MAX;
     for (int o2 = 16; o2 > 0; o2 >>= 1) best = fmaxf(best, __shfl_xor_sync(0xffffffffu, best, o2));
     if (lane == 0) {
@@ -565,16 +603,19 @@ score_merge_kernel(const MergeArgs a) {
         const float* base = a.partials + (size_t)seq * a.n_partials * PW;
         for (uint32_t p = lane; p < a.n_partials; p += 32) mm = fmaxf(mm, base[(size_t)p * PW]);
         for (int o = 16; o > 0; o >>= 1) mm = fmaxf(mm, __shfl_xor_sync(0xffffffffu, mm, o));
-        // (the partial sums are fp32 sums of fp32 exponentials already; the tolerance on a confidence is 1e-7 absolute
-        // on values of a few 1e-5, so fp32 is ample here -- fp64 exp cost this kernel most of its time)
-        float ss = 0.0f;
+        // (fp32 exponentials and per-lane sums, the lanes combined in fp64: an fp32 tree over a few hundred partials of
+        // similar size drifts by several ulps, which a confidence near 1/2 cannot afford; fp64 exp would cost this kernel
+        // most of its time)
+        float sl = 0.0f;   // a lane adds at most ceil(n_partials / 32) partials
         for (uint32_t p = lane; p < a.n_partials; p += 32) {
             const float* q = base + (size_t)p * PW;
-            ss += q[1] * expf(q[0] - mm);
+            sl += q[1] * expf(q[0] - mm);
 #pragma unroll
             for (int k = 0; k < K; ++k) list_insert<K>(lv, li, q[2 + k], __float_as_uint(q[2 + K + k]));
         }
+        double ss = sl;
         for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+        const float denom = (float)ss;
         // global top-k: k rounds of warp arg-max over the list heads, the winner pops its head
         float win_v = 0.0f;
         uint32_t win_i = 0;
@@ -604,7 +645,6 @@ score_merge_kernel(const MergeArgs a) {
             }
         }
         // lanes 0 .. k-1 hold prediction i = lane
-        const float denom = ss;
         bool keep = false;
         speckv_prefetch_request_t rq;
         if (lane < a.k) {
@@ -726,9 +766,10 @@ void harvest_calls_locked(bool wait) {
     }
 }
 
+// plan_only: n_partials and the dynamic shared memory the launch needs (smem), nothing launched
 template <int K, int S>
-cudaError_t launch_partial(uint32_t batch, const float* d_h, float* d_partials, uint32_t& n_partials, uint32_t plan_only,
-                           cudaStream_t st) {
+cudaError_t launch_partial(uint32_t batch, const float* d_h, float* d_partials, uint32_t& n_partials, size_t& smem,
+                           uint32_t plan_only, cudaStream_t st) {
     uint32_t seq_lanes = 4;   // at least 4: a tile (kScoreWarps * 32 / seq_lanes rows, double-buffered) must fit shared memory
     while (seq_lanes < 32 && seq_lanes * S < batch) seq_lanes <<= 1;
     const uint32_t nsub = kScoreWarps * (32u / seq_lanes);
@@ -741,11 +782,11 @@ cudaError_t launch_partial(uint32_t batch, const float* d_h, float* d_partials, 
     if (gx < 1) gx = 1;
     if (gx > n_tiles) gx = n_tiles;
     n_partials = gx;
-    if (plan_only) return cudaSuccess;
     constexpr int PW = 2 + 2 * K;
-    const size_t tile_bytes = 2ull * tile_rows * (g_pred.hidden + 4) * sizeof(float);
+    const size_t tile_bytes = 2ull * tile_rows * tile_ld(g_pred.hidden) * sizeof(float);
     const size_t park_bytes = (size_t)nsub * sb * PW * sizeof(float);
-    const size_t smem = tile_bytes > park_bytes ? tile_bytes : park_bytes;
+    smem = tile_bytes > park_bytes ? tile_bytes : park_bytes;
+    if (plan_only) return cudaSuccess;
     cudaError_t e = cudaFuncSetAttribute(score_partial_kernel<K, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     score_partial_kernel<K, S><<<dim3(gx, gy), kScoreThreads, smem, st>>>(g_pred.d_wout, g_pred.vocab, g_pred.hidden, d_h, batch,
@@ -767,18 +808,28 @@ speckv_status_t score_emit(const uint32_t* d_tokens, uint32_t batch, uint32_t k,
     if (cudaGetDevice(&dev) != cudaSuccess || dev != g_pred.device) return SPECKV_ERR_INVAL;   // weights live on another device
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     // rank-one scoring (candidates from h * rowsum[v], exact re-scoring) keeps k + 2 or more candidates; the tiled
-    // exact kernel remains for k > 14 and for SPECKV_SCORE_EXACT=2 (=1: the rank-one kernel with exact logits only)
+    // exact kernel remains for k > 14 and for SPECKV_SCORE_EXACT=2 (=1: the rank-one kernel with exact logits only).
+    // When a tile of W_out rows would not fit shared memory (wide hidden, small batches sooner), the rank-one kernel's
+    // exact pass takes the tiled kernel's place: it reads W_out from global memory at any width, for any k <= 16.
     const char* ex_env = getenv("SPECKV_SCORE_EXACT");
     const int ex_mode = ex_env ? atoi(ex_env) : 0;
-    const bool rank1 = g_pred.d_rowsum && k <= 14 && ex_mode != 2;
-    const int KK = rank1 ? (k <= 6 ? 8 : 16) : (k <= 4 ? 4 : (k <= 8 ? 8 : 16));
-    const int PW = 2 + 2 * KK;
+    bool rank1 = k <= 14 && ex_mode != 2;
+    bool force_exact = ex_mode == 1;
+    int KK = rank1 ? (k <= 6 ? 8 : 16) : (k <= 4 ? 4 : (k <= 8 ? 8 : 16));
     uint32_t n_partials = 1;
+    size_t tile_smem = 0;
     cudaError_t e = cudaSuccess;
-    if (!rank1)
-        e = KK == 4 ? launch_partial<4, 8>(batch, nullptr, nullptr, n_partials, 1, st)
-          : KK == 8 ? launch_partial<8, 4>(batch, nullptr, nullptr, n_partials, 1, st)
-                    : launch_partial<16, 2>(batch, nullptr, nullptr, n_partials, 1, st);
+    if (!rank1) {
+        e = KK == 4 ? launch_partial<4, 8>(batch, nullptr, nullptr, n_partials, tile_smem, 1, st)
+          : KK == 8 ? launch_partial<8, 4>(batch, nullptr, nullptr, n_partials, tile_smem, 1, st)
+                    : launch_partial<16, 2>(batch, nullptr, nullptr, n_partials, tile_smem, 1, st);
+        if (tile_smem > g_pred.smem_optin) {
+            rank1 = force_exact = true;
+            KK = 16;
+            n_partials = 1;
+        }
+    }
+    const int PW = 2 + 2 * KK;
     // per-call scratch from the stream's persistent buffer (two calls on different streams never share it)
     const size_t off_h = 0, off_p = (((size_t)batch * 4) + 255) & ~(size_t)255;
     const size_t off_s = (off_p + (size_t)batch * n_partials * PW * 4 + 255) & ~(size_t)255;
@@ -829,15 +880,15 @@ speckv_status_t score_emit(const uint32_t* d_tokens, uint32_t batch, uint32_t k,
     if (rank1) {
         if (KK == 8)
             score_rank1_kernel<8><<<batch, kScoreThreads, 0, st>>>(g_pred.d_wout, g_pred.d_rowsum, g_pred.d_cand, g_pred.vocab, g_pred.hidden, d_h,
-                                                                  batch, k, g_pred.row_abs_max, ex_mode == 1, d_partials);
+                                                                  batch, k, g_pred.row_abs_max, force_exact, d_partials);
         else
             score_rank1_kernel<16><<<batch, kScoreThreads, 0, st>>>(g_pred.d_wout, g_pred.d_rowsum, g_pred.d_cand, g_pred.vocab, g_pred.hidden, d_h,
-                                                                   batch, k, g_pred.row_abs_max, ex_mode == 1, d_partials);
+                                                                   batch, k, g_pred.row_abs_max, force_exact, d_partials);
         e = cudaGetLastError();
     } else {
-        e = KK == 4 ? launch_partial<4, 8>(batch, d_h, d_partials, n_partials, 0, st)
-          : KK == 8 ? launch_partial<8, 4>(batch, d_h, d_partials, n_partials, 0, st)
-                    : launch_partial<16, 2>(batch, d_h, d_partials, n_partials, 0, st);
+        e = KK == 4 ? launch_partial<4, 8>(batch, d_h, d_partials, n_partials, tile_smem, 0, st)
+          : KK == 8 ? launch_partial<8, 4>(batch, d_h, d_partials, n_partials, tile_smem, 0, st)
+                    : launch_partial<16, 2>(batch, d_h, d_partials, n_partials, tile_smem, 0, st);
     }
     if (e != cudaSuccess) return status_of(e);
     MergeArgs m;
@@ -882,11 +933,16 @@ speckv_status_t speckv_ext_predictor_load(const float* h_embedding, const float*
                                           uint32_t emb_dim, uint32_t hidden, uint32_t layers, uint32_t history_len) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
     if (!h_embedding || !h_output || !vocab || !emb_dim || !hidden || !history_len) return SPECKV_ERR_INVAL;
-    if (hidden > 4096) return SPECKV_ERR_INVAL;   // a tile of W_out rows must fit shared memory
+    // the rank-one kernel stages candidate rows in chunks and the tiled kernel's tile is checked per call (too wide a
+    // tile falls back to the rank-one exact pass), so no width is unscorable; 4096 bounds the per-row work of a thread
+    if (hidden > 4096) return SPECKV_ERR_INVAL;
     std::lock_guard<std::mutex> lk(g_pred_mu);
     harvest_calls_locked(true);
     free_predictor();
     cudaError_t e = cudaGetDevice(&g_pred.device);
+    int optin = 0;
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, g_pred.device);
+    g_pred.smem_optin = (size_t)optin;
     if (e == cudaSuccess) e = cudaMalloc((void**)&g_pred.d_emb, (size_t)vocab * emb_dim * sizeof(float));
     if (e == cudaSuccess) e = cudaMalloc((void**)&g_pred.d_wout, (size_t)vocab * hidden * sizeof(float));
     if (e == cudaSuccess) e = cudaMalloc((void**)&g_pred.d_ring, kRing * sizeof(speckv_prefetch_request_t));
