@@ -429,15 +429,10 @@ static speckv_status_t codec_args(CodecArgs& a, int dtype, size_t group_elems, s
     if (n_groups == 0) return SPECKV_OK;
     if (!d_payload || !d_scales || !d_comp_bytes || (!d_elems && group_elems)) return SPECKV_ERR_INVAL;
     if (reinterpret_cast<uintptr_t>(d_payload) & 15) return SPECKV_ERR_INVAL;
+    a = CodecArgs(slot_bytes, group_elems, n_groups, dtype, scheme);
     a.payload = const_cast<void*>(d_payload);
     a.scales = const_cast<float*>(d_scales);
     a.comp_bytes = const_cast<uint32_t*>(d_comp_bytes);
-    a.slot_bytes = slot_bytes;
-    a.group_elems = (uint32_t)group_elems;
-    a.n_groups = (uint32_t)n_groups;
-    a.dtype = dtype;
-    a.scheme = scheme;
-    a.sm_count = current_sm_count();
     return SPECKV_OK;
 }
 static speckv_status_t codec_run(bool decompress, const CodecArgs& a, void* cuda_stream) {
@@ -584,17 +579,11 @@ speckv_status_t speckv_ext_compress_host(const void* h_in, speckv_dtype_t dtype,
         cudaStream_t st = g_pipe.st[k];
         if ((e = cudaMemcpyAsync(g_pipe.d_elems[k], (const char*)h_in + g0 * gbytes, ng * gbytes, cudaMemcpyHostToDevice, st)) != cudaSuccess) break;
         moved_up += ng * gbytes;
-        CodecArgs a;
+        CodecArgs a(slot_bytes, group_elems, ng, dtype, scheme);
         a.in = g_pipe.d_elems[k];
         a.payload = g_pipe.d_payload[k];
         a.scales = g_pipe.d_scales[k];
         a.comp_bytes = g_pipe.d_comp[k];
-        a.slot_bytes = slot_bytes;
-        a.group_elems = (uint32_t)group_elems;
-        a.n_groups = (uint32_t)ng;
-        a.dtype = dtype;
-        a.scheme = scheme;
-        a.sm_count = current_sm_count();
         if ((e = launch_compress(a, st)) != cudaSuccess) break;
         if ((e = cudaMemcpyAsync(h_comp_bytes + g0, g_pipe.d_comp[k], ng * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;
         if ((e = cudaEventRecord(g_pipe.ev_meta[k], st)) != cudaSuccess) break;
@@ -645,18 +634,12 @@ speckv_status_t speckv_ext_decompress_host(const void* h_payload, size_t slot_by
         moved_down += ng * gbytes + (h_out_elems ? ng * 4 : 0);
         if ((e = cudaMemcpyAsync(g_pipe.d_scales[k], h_scales + g0, ng * sizeof(float), cudaMemcpyHostToDevice, st)) != cudaSuccess) break;
         if ((e = cudaMemcpyAsync(g_pipe.d_comp[k], h_comp_bytes + g0, ng * sizeof(uint32_t), cudaMemcpyHostToDevice, st)) != cudaSuccess) break;
-        CodecArgs a;
+        CodecArgs a(slot_bytes, group_elems, ng, dtype, scheme);
         a.out = g_pipe.d_elems[k];
         a.payload = g_pipe.d_payload[k];
         a.scales = g_pipe.d_scales[k];
         a.comp_bytes = g_pipe.d_comp[k];
         a.out_elems = g_pipe.d_oel[k];
-        a.slot_bytes = slot_bytes;
-        a.group_elems = (uint32_t)group_elems;
-        a.n_groups = (uint32_t)ng;
-        a.dtype = dtype;
-        a.scheme = scheme;
-        a.sm_count = current_sm_count();
         if ((e = launch_decompress(a, st)) != cudaSuccess) break;
         if ((e = cudaMemcpyAsync((char*)h_out + g0 * gbytes, g_pipe.d_elems[k], ng * gbytes, cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;
         if (h_out_elems && (e = cudaMemcpyAsync(h_out_elems + g0, g_pipe.d_oel[k], ng * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;

@@ -7,6 +7,8 @@
 
 namespace speckv {
 
+// One codec call.  The host fills it and every codec kernel takes it by value: the container addressing below is
+// written once, here, for all of them.
 struct CodecArgs {
     const void* in = nullptr;        // compress: elements in; decompress: unused
     void* out = nullptr;             // decompress: elements out
@@ -15,8 +17,9 @@ struct CodecArgs {
     uint32_t* comp_bytes = nullptr;
     uint32_t* out_elems = nullptr;   // decompress, optional
     const uint32_t* src_index = nullptr;  // decompress, optional: output group i decodes payload group src_index[i]
-    const uint64_t* slot_offsets = nullptr;  // decompress, optional: block b starts at payload + slot_offsets[b]
-                                             // (16 B aligned, packed container) instead of b * slot_bytes
+    const uint64_t* slot_offsets = nullptr;  // optional: block b starts at payload + slot_offsets[b] (16 B aligned, packed
+                                             // container) instead of b * slot_bytes.  Decompress, and the generic compress
+                                             // behind a packed emission (the slots reserved at pack_offsets)
     const uint32_t* elem_index = nullptr;    // optional paged gather / scatter: group i's elements are block
                                              // elem_index[i] of the element buffer (compress reads `in` there,
                                              // decompress writes `out` there) instead of block i
@@ -37,14 +40,37 @@ struct CodecArgs {
     uint32_t n_groups = 0;
     int dtype = 0;                   // DT_F16 / DT_BF16 / DT_F32
     int scheme = 2;                  // speckv_comp_scheme_t, or one of the extension ids 3 / 4 (speckv_ext.h)
-    int sm_count = 148;
+
+    CodecArgs() = default;
+    CodecArgs(size_t slot_bytes_, size_t group_elems_, size_t n_groups_, int dtype_, int scheme_)
+        : slot_bytes(slot_bytes_), group_elems((uint32_t)group_elems_), n_groups((uint32_t)n_groups_), dtype(dtype_),
+          scheme(scheme_) {}
+
+    // ---- container addressing (device).  The index arrays stay unchanged during a launch: non-coherent loads.
+    // group g's elements: block elem_index[g] of `base`, else block g (blocks of G elements)
+    template <typename T>
+    __device__ __forceinline__ T* elem_block(T* base, uint32_t g, uint32_t G) const {
+        return base + (size_t)(elem_index ? __ldg(elem_index + g) : g) * G;
+    }
+    // the stored block output group g decodes
+    __device__ __forceinline__ uint32_t stored_block(uint32_t g) const { return src_index ? __ldg(src_index + g) : g; }
+    // the payload of stored block b
+    __device__ __forceinline__ uint8_t* block_payload(uint32_t b) const {
+        return static_cast<uint8_t*>(payload) + (slot_offsets ? (size_t)__ldg(slot_offsets + b) : (size_t)b * slot_bytes);
+    }
+    // groups to process: n_groups, or fewer when the request count lives on the device
+    __device__ __forceinline__ uint32_t live_groups() const { return n_groups_dev ? min(n_groups, __ldg(n_groups_dev)) : n_groups; }
+    // elements group g encodes (blocks of G elements): a ragged call's filled prefix, else the whole block
+    __device__ __forceinline__ uint32_t group_length(uint32_t g, uint32_t G) const {
+        return group_len ? min(__ldg(group_len + g), G) : G;
+    }
 };
 
 // scheme ids: 0 raw 16-bit passthrough, 1 codes only, 2 codes + delta + RLE (the reference's three), and the clamped
 // variants of 2 and 1 that store s = max|x| (3, 4)
-inline bool scheme_is_rle(int s) { return s == 2 || s == 3; }
-inline bool scheme_is_codes(int s) { return s == 1 || s == 4; }
-inline bool scheme_max_scale(int s) { return s == 3 || s == 4; }
+__host__ __device__ inline bool scheme_is_rle(int s) { return s == 2 || s == 3; }
+__host__ __device__ inline bool scheme_is_codes(int s) { return s == 1 || s == 4; }
+__host__ __device__ inline bool scheme_max_scale(int s) { return s == 3 || s == 4; }
 
 // What the tuned decompress kernel leaves for the second pass (one buffer per stream, kept across calls):
 //   flags[g]   0 = done, 1 = the generic kernel decodes group g, 2 = the run-expansion path does

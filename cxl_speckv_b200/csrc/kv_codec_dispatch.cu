@@ -35,7 +35,9 @@ cudaError_t launch_compress(const CodecArgs& a, cudaStream_t st) {
         if (e == cudaSuccess) e = scratch_persistent(reinterpret_cast<void**>(&status), n_ctas * sizeof(unsigned long long), st, 2);
         if (e == cudaSuccess) e = cudaMemsetAsync(status, 0, n_ctas * sizeof(unsigned long long), st);
         if (e == cudaSuccess) e = launch_compress_fast(R, a, flags, st, status);
-        if (e == cudaSuccess) e = launch_compress_generic(a, st, flags);   // writes at pack_offsets[g] (a whole slot was reserved)
+        CodecArgs second = a;
+        second.slot_offsets = a.pack_offsets;   // the generic kernel writes into the whole slot reserved at pack_offsets[g]
+        if (e == cudaSuccess) e = launch_compress_generic(second, st, flags);
         return e;
     }
     if (R == 0) return launch_compress_generic(a, st, nullptr);

@@ -841,15 +841,12 @@ __device__ __noinline__ unsigned long long pack_place(FastSmem& sm, const PackOu
 // ===================================================================================
 // compress
 // ===================================================================================
-// RAGGED: group g is the first n = min(group_len[g], G) elements of its block.  Regions at or past n are neither
+// RAGGED: group g is the first n = a.group_length(g, G) elements of its block.  Regions at or past n are neither
 // loaded nor emitted but still take part in every exchange (a cluster CTA stays until its peers' words have landed);
 // the region holding element n - 1 masks its tail out of the max, forces run heads from n on and ends the group.
 template <typename T, int R, bool PACKED = false, bool RAGGED = false>
 __global__ void __launch_bounds__(kThreadsF, kCtasPerSm)
-compress_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t* __restrict__ payload, size_t slot_bytes,
-                     float* __restrict__ scales, uint32_t* __restrict__ comp_bytes,
-                     uint32_t* __restrict__ needs_generic, const uint32_t* __restrict__ elem_index, uint32_t max_scale,
-                     const PackOut pk, const uint32_t* __restrict__ group_len) {
+compress_fast_kernel(const __grid_constant__ CodecArgs a, uint32_t* __restrict__ needs_generic, const PackOut pk) {
     static_assert(!PACKED || R == 1, "packed emission is built for page groups");
     static_assert(!(PACKED && RAGGED), "ragged groups use the slot form");
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -858,7 +855,6 @@ compress_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t* __res
     constexpr int GPC = R >= kW ? 1 : kW / R;     // groups per CTA
     constexpr uint32_t G = (uint32_t)R * kRegion;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const unsigned lt_mask = (1u << lane) - 1u;
 
     uint32_t g;
     int ridx;
@@ -870,13 +866,13 @@ compress_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t* __res
         g = blockIdx.x * GPC + warp / R;
         ridx = warp % R;
     }
-    const bool active = g < n_groups;
-    const uint32_t n_len = (RAGGED && active) ? min(group_len[g], G) : G;
+    const bool active = g < a.n_groups;
+    const uint32_t n_len = (RAGGED && active) ? a.group_length(g, G) : G;
     const int lim = (int)n_len - ridx * kRegion;                 // elements of this region inside the group (>= 2048: all)
-    const int r_last = RAGGED ? ((int)n_len - 1) >> 11 : R - 1;   // region of the group's last element (-1: empty group)
     const bool live = active && (!RAGGED || lim > 0);
-    // paged gather: the group's elements are block elem_index[g] of the element buffer
-    const T* rin = in + (size_t)((elem_index && active) ? elem_index[g] : g) * G + (size_t)ridx * kRegion;
+    const T* in = static_cast<const T*>(a.in);
+    // a group past the end has no elem_index entry to read: its (never loaded) address stays block g
+    const T* rin = (active ? a.elem_block(in, g, G) : in + (size_t)g * G) + (size_t)ridx * kRegion;
     uint8_t* reg = sm.tile[warp] + kPadBytes;
     const uint32_t reg_s = smem_u32(reg);
     const uint32_t mb = smem_u32(&sm.mbar[warp]);
@@ -923,7 +919,7 @@ compress_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t* __res
     // max / 127 (the reference), or max for the clamped scheme.  For the groups this kernel encodes itself (fast) the
     // IEEE division by 127 is the two-operation form RN(m * r127 + RN(m * d127)) of codec_math.cuh: exact for every
     // fp16 value and every bf16 value >= 2^-118 (oracle/verify_fastdiv.c, "scale"), a dozen instructions shorter
-    const float s = max_scale != 0u ? (gmax > 0.0f ? gmax : 1.0f)
+    const float s = scheme_max_scale(a.scheme) ? (gmax > 0.0f ? gmax : 1.0f)
                                     : (fast ? __fmaf_rn(gmax, __uint_as_float(0x3c010204u), __fmul_rn(gmax, __uint_as_float(0x2e010204u)))
                                             : scale_from_max(gmax));
     // a group whose max-abs is 0 (zeros, possibly NaNs: cache_engine.cpp:176-179 skips them and the cast maps
@@ -1036,39 +1032,39 @@ compress_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t* __res
         // the closed form of a zero group, a whole slot for a group the generic kernel will encode
         constexpr uint32_t zfull = G / 255u, zrem = G % 255u, znp = zfull + (zrem ? 1u : 0u);
         uint32_t my = 0;
-        if (active) my = cplx ? (uint32_t)slot_bytes : (zero_group ? 2u * znp : 2u * (h_total & 0xfffffu));
+        if (active) my = cplx ? (uint32_t)a.slot_bytes : (zero_group ? 2u * znp : 2u * (h_total & 0xfffffu));
         out_off = (size_t)pack_place(sm, pk, (my + 15u) & ~15u, warp, lane);
         if (active && lane == 0) pk.offsets[g] = out_off;
     }
     if (!active) return;
     if (ridx == 0 && lane == 0) {
         needs_generic[g] = any_cplx ? 1u : 0u;
-        if (any_cplx) comp_bytes[g] = gmax_bits;   // hand the group max to the generic kernel: it skips its own max pass
+        if (any_cplx) a.comp_bytes[g] = gmax_bits;   // hand the group max to the generic kernel: it skips its own max pass
     }
     if (any_cplx) return;
     if (zero_group) {
         if (ridx == 0) {
             const uint32_t full = n_len / 255u, rem = n_len % 255u, npairs = full + (rem ? 1u : 0u);
-            uint16_t* go = reinterpret_cast<uint16_t*>(payload + (PACKED ? out_off : (size_t)g * slot_bytes));
+            uint16_t* go = reinterpret_cast<uint16_t*>(static_cast<uint8_t*>(a.payload) + (PACKED ? out_off : (size_t)g * a.slot_bytes));
             for (uint32_t i = lane; i < npairs; i += 32u) go[i] = i < full ? (uint16_t)0xff00u : (uint16_t)(rem << 8);
             if (lane == 0) {
-                scales[g] = s;   // 1.0f
-                comp_bytes[g] = 2u * npairs;
+                a.scales[g] = s;   // 1.0f
+                a.comp_bytes[g] = 2u * npairs;
             }
         }
         return;
     }
 
-    uint8_t* gout = payload + (PACKED ? out_off : (size_t)g * slot_bytes);
-    const bool last = ridx == r_last;
+    uint8_t* gout = static_cast<uint8_t*>(a.payload) + (PACKED ? out_off : (size_t)g * a.slot_bytes);
+    const bool last = RAGGED ? lim > 0 && lim <= kRegion : ridx == R - 1;   // the region holds the group's last element
     if (any_long) {   // groups with long runs: everything else happens in long_path (not inlined)
-        long_path<R, RAGGED>(sm, reg, reg_s, warp, lane, ridx, longr, carry_d1, halo_tail, s, gout, scales + g, comp_bytes + g,
+        long_path<R, RAGGED>(sm, reg, reg_s, warp, lane, ridx, longr, carry_d1, halo_tail, s, gout, a.scales + g, a.comp_bytes + g,
                              live, last, lim);
         return;
     }
     if (RAGGED && !live) return;
 
-    emit_common<R, RAGGED>(reg, reg_s, lane, lt_mask, ridx, h_before, halo_tail, carry_d1, s, gout, scales + g, comp_bytes + g,
+    emit_common<R, RAGGED>(reg, reg_s, lane, (1u << lane) - 1u, ridx, h_before, halo_tail, carry_d1, s, gout, a.scales + g, a.comp_bytes + g,
                            last, lim);
 }
 
@@ -1118,12 +1114,7 @@ __device__ __noinline__ uint32_t zero_tail_blank(uint8_t* reg, int lane, uint32_
 
 template <typename T, int R>
 __global__ void __launch_bounds__(kThreadsF, kCtasPerSm)
-decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, const float* __restrict__ scales,
-                       const uint32_t* __restrict__ comp_bytes, uint32_t n_groups, T* __restrict__ out,
-                       uint32_t* __restrict__ out_elems, uint32_t* __restrict__ needs_generic,
-                       const uint32_t* __restrict__ src_index, const uint64_t* __restrict__ slot_offsets,
-                       const uint32_t* __restrict__ elem_index, const uint32_t* __restrict__ n_groups_dev,
-                       uint32_t* __restrict__ runs_list, uint32_t* __restrict__ runs_counters, uint2* __restrict__ runs_prefix) {
+decompress_fast_kernel(const __grid_constant__ CodecArgs a, const DecodeScratch scr) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     FastSmem& sm = *reinterpret_cast<FastSmem*>(smem_raw);
     constexpr int C = R > kW ? R / kW : 1;
@@ -1144,8 +1135,8 @@ decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, c
     }
     // the request count may live on the device (prefetch requests routed by a kernel): the grid covers the
     // capacity n_groups, groups at or above the count only clear their flag for the generic second pass
-    const bool in_grid = g < n_groups;
-    const bool active = in_grid && (!n_groups_dev || g < *n_groups_dev);
+    const bool in_grid = g < a.n_groups;
+    const bool active = in_grid && g < a.live_groups();
     uint8_t* reg = sm.tile[warp] + kPadBytes;
     const uint32_t reg_s = smem_u32(reg);
     const uint32_t mb = smem_u32(&sm.mbar[warp]);
@@ -1154,20 +1145,19 @@ decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, c
     uint32_t np = 0;
     float s = 1.0f;
     bool cplx = false;
-    uint32_t gi = g;   // stored block decoded by output group g
+    const uint8_t* rp = nullptr;   // the region's pairs
     if (active) {
-        if (src_index) gi = src_index[g];
-        const uint32_t cb = comp_bytes[gi];
+        const uint32_t gi = a.stored_block(g);
+        const uint32_t cb = __ldg(a.comp_bytes + gi);
         uint32_t npairs = cb >> 1;                            // a trailing odd byte is ignored (:245-247)
-        if ((size_t)cb > slot_bytes) cplx = true;             // malformed: leave it to the generic kernel's clamping
+        if ((size_t)cb > a.slot_bytes) cplx = true;           // malformed: leave it to the generic kernel's clamping
         npairs = min(npairs, (uint32_t)(R * kRegion));
         const uint32_t first = (uint32_t)ridx * kRegion;
         np = npairs > first ? min(npairs - first, (uint32_t)kRegion) : 0u;
-        s = scales[gi];
+        s = __ldg(a.scales + gi);
         cplx |= scale_is_special(s);
+        rp = a.block_payload(gi) + (size_t)ridx * kRegionBytes;
     }
-    const uint8_t* rp = payload + ((slot_offsets && active) ? (size_t)slot_offsets[gi] : (size_t)gi * slot_bytes) +
-                        (size_t)ridx * kRegionBytes;
 
     if (lane == 0) {
         mbar_init(mb, 1);
@@ -1310,12 +1300,12 @@ decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, c
         mbar_wait(mb, 0);
         const bool ok = expand(std::false_type{}, std::true_type{}) && ecur <= G;
         if (lane == 0) {
-            needs_generic[g] = ok ? 0u : 1u;
-            if (out_elems && ok) out_elems[g] = ecur;
+            scr.flags[g] = ok ? 0u : 1u;
+            if (a.out_elems && ok) a.out_elems[g] = ecur;
         }
         if (!ok) return;
         __syncwarp();
-        flush_region(sbase, reinterpret_cast<uint8_t*>(out + (size_t)(elem_index ? elem_index[g] : g) * G), 0, (int)ecur, lane);
+        flush_region(sbase, reinterpret_cast<uint8_t*>(a.elem_block(static_cast<T*>(a.out), g, G)), 0, (int)ecur, lane);
         return;
     }
 
@@ -1394,24 +1384,24 @@ decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, c
     group_reduce<R>(sm.xa, warp, lane, ridx, e_before, e_total, t0);
     group_reduce<R>(sm.xb, warp, lane, ridx, q_before, xb_total, xb_max);
     if (!active) {
-        if (in_grid && ridx == 0 && lane == 0) needs_generic[g] = 0u;
+        if (in_grid && ridx == 0 && lane == 0) scr.flags[g] = 0u;
         return;
     }
     const bool any_cplx = ((xb_total >> 16) & 0xffu) != 0 || e_total > G;   // output longer than the group: generic kernel clips
     const bool any_runs = !any_cplx && (xb_max >> 31) != 0u;
     const bool short_deq = ((xb_total >> 24) & 0x7fu) == 0;
     if (ridx == 0 && lane == 0) {
-        needs_generic[g] = any_cplx ? 1u : (any_runs ? 2u : 0u);
-        if (out_elems && !any_cplx) out_elems[g] = e_total;
+        scr.flags[g] = any_cplx ? 1u : (any_runs ? 2u : 0u);
+        if (a.out_elems && !any_cplx) a.out_elems[g] = e_total;
     }
     if (any_runs) {
         // hand the group over with what phase A found: where every pairs-region starts in the output and with which
         // code; the second pass expands output region by output region (kv_codec_generic.cu, decode_runs_region)
         if (lane == 0) {
-            runs_prefix[(size_t)g * (R + 1) + ridx] = make_uint2(e_before, q_before & 0xffu);
+            scr.prefix[(size_t)g * (R + 1) + ridx] = make_uint2(e_before, q_before & 0xffu);
             if (ridx == 0) {
-                runs_prefix[(size_t)g * (R + 1) + R] = make_uint2(e_total, 0u);
-                runs_list[atomicAdd(runs_counters, 1u)] = g;
+                scr.prefix[(size_t)g * (R + 1) + R] = make_uint2(e_total, 0u);
+                scr.list[atomicAdd(scr.counters, 1u)] = g;
             }
         }
         return;
@@ -1419,7 +1409,7 @@ decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, c
     if (any_cplx || np == 0) return;
 
     // ---- C. expand in place: element e of run j carries code q_before + ... + v_j * (e - start_j + 1) ----
-    uint8_t* gout = reinterpret_cast<uint8_t*>(out + (size_t)(elem_index ? elem_index[g] : g) * G);   // paged scatter
+    uint8_t* gout = reinterpret_cast<uint8_t*>(a.elem_block(static_cast<T*>(a.out), g, G));
     const uint32_t e0 = e_before;
     // constant fill: elements [ea, ea + n) all carry `code` (zero blocks, long runs of one value, zero tails)
     auto fill_const = [&](uint32_t ea, uint32_t n, uint32_t code) {
@@ -1455,13 +1445,10 @@ decompress_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, c
 // bulk-TMA store of the region's 2 KiB.  Decompress has no dependency between regions at all: no cluster, no exchange.
 // Algorithmic traffic: 2n + n bytes per group either way.
 // ===================================================================================
-// RAGGED: group g is the first n = min(group_len[g], G) elements of its block; n codes are written.
+// RAGGED: group g is the first n = a.group_length(g, G) elements of its block; n codes are written.
 template <typename T, int R, bool RAGGED = false>
 __global__ void __launch_bounds__(kThreadsF, kCtasPerSm)
-compress_codes_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t* __restrict__ payload, size_t slot_bytes,
-                           float* __restrict__ scales, uint32_t* __restrict__ comp_bytes,
-                           uint32_t* __restrict__ needs_generic, const uint32_t* __restrict__ elem_index, uint32_t max_scale,
-                           const uint32_t* __restrict__ group_len) {
+compress_codes_fast_kernel(const __grid_constant__ CodecArgs a, uint32_t* __restrict__ needs_generic) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     FastSmem& sm = *reinterpret_cast<FastSmem*>(smem_raw);
     constexpr int C = R > kW ? R / kW : 1;
@@ -1478,11 +1465,13 @@ compress_codes_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t*
         g = blockIdx.x * GPC + warp / R;
         ridx = warp % R;
     }
-    const bool active = g < n_groups;
-    const uint32_t n_len = (RAGGED && active) ? min(group_len[g], G) : G;
+    const bool active = g < a.n_groups;
+    const uint32_t n_len = (RAGGED && active) ? a.group_length(g, G) : G;
     const int lim = (int)n_len - ridx * kRegion;   // elements of this region inside the group (>= 2048: all)
     const bool live = active && (!RAGGED || lim > 0);
-    const T* rin = in + (size_t)((elem_index && active) ? elem_index[g] : g) * G + (size_t)ridx * kRegion;
+    const T* in = static_cast<const T*>(a.in);
+    // a group past the end has no elem_index entry to read: its (never loaded) address stays block g
+    const T* rin = (active ? a.elem_block(in, g, G) : in + (size_t)g * G) + (size_t)ridx * kRegion;
     uint8_t* reg = sm.tile[warp] + kPadBytes;
     const uint32_t reg_s = smem_u32(reg);
     const uint32_t mb = smem_u32(&sm.mbar[warp]);
@@ -1516,18 +1505,18 @@ compress_codes_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t*
     group_reduce<R>(sm.xa, warp, lane, ridx, t0, t1, gmax_bits);
     if (!active) return;
     const float gmax = __uint_as_float(gmax_bits);
-    const float s = scale_for(gmax, max_scale != 0u);
+    const float s = scale_for(gmax, scheme_max_scale(a.scheme));
     const bool zero_group = gmax_bits == 0u;                 // zeros / NaNs only: every code is 0 (scale 1)
     const bool fast = fast_quant_ok<T>(gmax) || zero_group;
     if (ridx == 0 && lane == 0) {
         needs_generic[g] = fast ? 0u : 1u;
-        if (!fast) comp_bytes[g] = gmax_bits;                // the generic second pass skips its own max pass
+        if (!fast) a.comp_bytes[g] = gmax_bits;              // the generic second pass skips its own max pass
     }
     if (!fast) return;
     if (RAGGED && !live) {   // past the end (an empty group: region 0 reports it)
         if (ridx == 0 && lane == 0) {
-            scales[g] = s;
-            comp_bytes[g] = 0u;
+            a.scales[g] = s;
+            a.comp_bytes[g] = 0u;
         }
         return;
     }
@@ -1555,7 +1544,7 @@ compress_codes_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t*
     // ragged: the codes before the group's end, whole 16-byte vectors in the bulk store, the rest byte by byte
     const uint32_t nb = RAGGED ? (uint32_t)min(lim, kRegion) : (uint32_t)kRegion;
     const uint32_t nb16 = nb & ~15u;
-    uint8_t* gout = payload + (size_t)g * slot_bytes + (size_t)ridx * kRegion;
+    uint8_t* gout = static_cast<uint8_t*>(a.payload) + (size_t)g * a.slot_bytes + (size_t)ridx * kRegion;
     if (RAGGED && (uint32_t)lane < nb - nb16) gout[nb16 + lane] = reg[nb16 + lane];
     if (lane == 0) {
         if (nb16)
@@ -1563,51 +1552,47 @@ compress_codes_fast_kernel(const T* __restrict__ in, uint32_t n_groups, uint8_t*
                          : "memory");
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         if (ridx == 0) {
-            scales[g] = s;
-            comp_bytes[g] = n_len;
+            a.scales[g] = s;
+            a.comp_bytes[g] = n_len;
         }
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
     }
 }
 
-// one warp per region of 2048 codes; `regions` = R of the group geometry (any value: regions are independent)
+// one warp per region of 2048 codes; scr.regions = R of the group geometry (any value: regions are independent)
 template <typename T>
 __global__ void __launch_bounds__(kThreadsF, kCtasPerSm)
-decompress_codes_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes, const float* __restrict__ scales,
-                             const uint32_t* __restrict__ comp_bytes, uint32_t n_groups, uint32_t regions, T* __restrict__ out,
-                             uint32_t* __restrict__ out_elems, uint32_t* __restrict__ needs_generic,
-                             const uint32_t* __restrict__ src_index, const uint64_t* __restrict__ slot_offsets,
-                             const uint32_t* __restrict__ elem_index, const uint32_t* __restrict__ n_groups_dev) {
+decompress_codes_fast_kernel(const __grid_constant__ CodecArgs a, const DecodeScratch scr) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     FastSmem& sm = *reinterpret_cast<FastSmem*>(smem_raw);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint64_t rid = (uint64_t)blockIdx.x * kW + warp;
-    const uint32_t g = (uint32_t)(rid / regions), ridx = (uint32_t)(rid % regions);
-    const uint32_t G = regions * (uint32_t)kRegion;
-    const bool in_grid = g < n_groups;
-    const bool active = in_grid && (!n_groups_dev || g < *n_groups_dev);
+    const uint32_t g = (uint32_t)(rid / scr.regions), ridx = (uint32_t)(rid % scr.regions);
+    const uint32_t G = scr.regions * (uint32_t)kRegion;
+    const bool in_grid = g < a.n_groups;
+    const bool active = in_grid && g < a.live_groups();
     if (!in_grid) return;
     uint32_t gi = g, n = 0;
     float s = 1.0f;
     bool cplx = false;
     if (active) {
-        if (src_index) gi = src_index[g];
-        s = scales[gi];
+        gi = a.stored_block(g);
+        s = __ldg(a.scales + gi);
         // oversized payloads and non-finite scales: the generic kernel's clamping / special values.  A shorter payload
         // (a ragged group) decodes to its comp_bytes elements here; the rest of the destination is left as it is.
-        n = comp_bytes[gi];
-        cplx = n > G || (size_t)G > slot_bytes || scale_is_special(s);
+        n = __ldg(a.comp_bytes + gi);
+        cplx = n > G || (size_t)G > a.slot_bytes || scale_is_special(s);
     }
     if (ridx == 0 && lane == 0) {
-        needs_generic[g] = (active && cplx) ? 1u : 0u;
-        if (out_elems && active && !cplx) out_elems[g] = n;
+        scr.flags[g] = (active && cplx) ? 1u : 0u;
+        if (a.out_elems && active && !cplx) a.out_elems[g] = n;
     }
     const uint32_t nr = n > ridx * (uint32_t)kRegion ? min(n - ridx * (uint32_t)kRegion, (uint32_t)kRegion) : 0u;   // codes of this region
     if (!active || cplx || nr == 0) return;
     uint8_t* reg = sm.tile[warp] + kPadBytes;
     const uint32_t reg_s = smem_u32(reg);
     const uint32_t mb = smem_u32(&sm.mbar[warp]);
-    const uint8_t* rp = payload + (slot_offsets ? (size_t)slot_offsets[gi] : (size_t)gi * slot_bytes) + (size_t)ridx * kRegion;
+    const uint8_t* rp = a.block_payload(gi) + (size_t)ridx * kRegion;
     if (lane == 0) {
         mbar_init(mb, 1);
         const uint32_t bytes = (nr + 15u) & ~15u;   // within the slot: slot_bytes >= G
@@ -1627,7 +1612,7 @@ decompress_codes_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_by
         *reinterpret_cast<uint4*>(reg + k * 512 + lane * 16) =
             make_uint4(pack2_out<T>(y[0], y[1]), pack2_out<T>(y[2], y[3]), pack2_out<T>(y[4], y[5]), pack2_out<T>(y[6], y[7]));
     }
-    T* gout = out + (size_t)(elem_index ? elem_index[g] : g) * G + (size_t)ridx * kRegion;
+    T* gout = a.elem_block(static_cast<T*>(a.out), g, G) + (size_t)ridx * kRegion;
     if (nr < (uint32_t)kRegion) {   // the region holding the end of a short payload: exactly nr elements
         __syncwarp();
         flush_region(reg_s, reinterpret_cast<uint8_t*>(gout), 0, (int)nr, lane);
@@ -1644,8 +1629,8 @@ decompress_codes_fast_kernel(const uint8_t* __restrict__ payload, size_t slot_by
 }
 
 // ---- launch -------------------------------------------------------------------------
-template <typename K>
-cudaError_t launch_clustered(K kernel, int R, uint32_t n_groups, cudaStream_t st, void** args) {
+template <typename... P, typename... Args>
+cudaError_t launch_clustered(void (*kernel)(P...), int R, uint32_t n_groups, cudaStream_t st, Args... args) {
     const int C = R > kW ? R / kW : 1;
     const int gpc = R >= kW ? 1 : kW / R;
     const size_t smem = sizeof(FastSmem);
@@ -1672,45 +1657,35 @@ cudaError_t launch_clustered(K kernel, int R, uint32_t n_groups, cudaStream_t st
             policy == 1 ? cudaClusterSchedulingPolicySpread : cudaClusterSchedulingPolicyLoadBalancing;
         cfg.numAttrs = 2;
     }
-    e = cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(kernel), args);
+    e = cudaLaunchKernelEx(&cfg, kernel, args...);
     count_launch();
     return e;
 }
 
 template <typename T>
 cudaError_t compress_fast_t(int R, const CodecArgs& a, uint32_t* flags, cudaStream_t st, unsigned long long* pack_status) {
-    const T* in = static_cast<const T*>(a.in);
-    uint32_t n = a.n_groups;
-    uint8_t* pay = static_cast<uint8_t*>(a.payload);
-    size_t sb = a.slot_bytes;
-    float* sc = a.scales;
-    uint32_t* cb = a.comp_bytes;
-    const uint32_t* ei = a.elem_index;
-    uint32_t ms = scheme_max_scale(a.scheme) ? 1u : 0u;
-    PackOut pko;
-    pko.offsets = a.pack_offsets;
-    pko.total = a.pack_total;
-    pko.status = pack_status;
-    const uint32_t* gl = a.group_len;
-    void* args[] = {&in, &n, &pay, &sb, &sc, &cb, &flags, &ei, &ms, &pko, &gl};
-    void* cargs[] = {&in, &n, &pay, &sb, &sc, &cb, &flags, &ei, &ms, &gl};   // the codes-only kernels: no packed emission
+    const uint32_t n = a.n_groups;
     if (pack_status) {
-        if (R != 1 || scheme_is_codes(a.scheme) || !a.pack_offsets || !a.pack_total || gl) return cudaErrorInvalidValue;
-        return launch_clustered(compress_fast_kernel<T, 1, true>, 1, n, st, args);
+        if (R != 1 || scheme_is_codes(a.scheme) || !a.pack_offsets || !a.pack_total || a.group_len) return cudaErrorInvalidValue;
+        PackOut pk;
+        pk.offsets = a.pack_offsets;
+        pk.total = a.pack_total;
+        pk.status = pack_status;
+        return launch_clustered(compress_fast_kernel<T, 1, true>, 1, n, st, a, flags, pk);
     }
     // ragged calls (a.group_len) run their own instantiations: the dense ones keep their code and registers
     if (scheme_is_codes(a.scheme)) {
         switch (R) {
-#define SPECKV_CASE(RR) case RR: return gl ? launch_clustered(compress_codes_fast_kernel<T, RR, true>, RR, n, st, cargs) \
-                                           : launch_clustered(compress_codes_fast_kernel<T, RR>, RR, n, st, cargs);
+#define SPECKV_CASE(RR) case RR: return a.group_len ? launch_clustered(compress_codes_fast_kernel<T, RR, true>, RR, n, st, a, flags) \
+                                                    : launch_clustered(compress_codes_fast_kernel<T, RR>, RR, n, st, a, flags);
             SPECKV_CASE(1) SPECKV_CASE(2) SPECKV_CASE(4) SPECKV_CASE(8) SPECKV_CASE(16) SPECKV_CASE(32) SPECKV_CASE(64) SPECKV_CASE(128)
 #undef SPECKV_CASE
             default: return cudaErrorInvalidValue;
         }
     }
     switch (R) {
-#define SPECKV_CASE(RR) case RR: return gl ? launch_clustered(compress_fast_kernel<T, RR, false, true>, RR, n, st, args) \
-                                       : launch_clustered(compress_fast_kernel<T, RR>, RR, n, st, args);
+#define SPECKV_CASE(RR) case RR: return a.group_len ? launch_clustered(compress_fast_kernel<T, RR, false, true>, RR, n, st, a, flags, PackOut{}) \
+                                                : launch_clustered(compress_fast_kernel<T, RR>, RR, n, st, a, flags, PackOut{});
         SPECKV_CASE(1) SPECKV_CASE(2) SPECKV_CASE(4) SPECKV_CASE(8) SPECKV_CASE(16) SPECKV_CASE(32) SPECKV_CASE(64) SPECKV_CASE(128)
 #undef SPECKV_CASE
         default: return cudaErrorInvalidValue;
@@ -1719,34 +1694,17 @@ cudaError_t compress_fast_t(int R, const CodecArgs& a, uint32_t* flags, cudaStre
 
 template <typename T>
 cudaError_t decompress_fast_t(int R, const CodecArgs& a, const DecodeScratch& scr, cudaStream_t st) {
-    uint32_t* flags = scr.flags;
-    uint32_t* rl = scr.list;
-    uint32_t* rc = scr.counters;
-    uint2* rp = scr.prefix;
-    const uint8_t* pay = static_cast<const uint8_t*>(a.payload);
-    size_t sb = a.slot_bytes;
-    const float* sc = a.scales;
-    const uint32_t* cb = a.comp_bytes;
-    uint32_t n = a.n_groups;
-    T* out = static_cast<T*>(a.out);
-    uint32_t* oe = a.out_elems;
-    const uint32_t* si = a.src_index;
-    const uint64_t* so = a.slot_offsets;
-    const uint32_t* ei = a.elem_index;
-    const uint32_t* nd = a.n_groups_dev;
     if (scheme_is_codes(a.scheme)) {
         const size_t smem = sizeof(FastSmem);
         cudaError_t e = cudaFuncSetAttribute(decompress_codes_fast_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        const uint64_t regions = (uint64_t)n * (uint32_t)R;
-        decompress_codes_fast_kernel<T><<<(unsigned)((regions + kW - 1) / kW), kThreadsF, smem, st>>>(
-            pay, sb, sc, cb, n, (uint32_t)R, out, oe, flags, si, so, ei, nd);
+        const uint64_t regions = (uint64_t)a.n_groups * (uint32_t)R;
+        decompress_codes_fast_kernel<T><<<(unsigned)((regions + kW - 1) / kW), kThreadsF, smem, st>>>(a, scr);
         count_launch();
         return cudaGetLastError();
     }
-    void* args[] = {&pay, &sb, &sc, &cb, &n, &out, &oe, &flags, &si, &so, &ei, &nd, &rl, &rc, &rp};
     switch (R) {
-#define SPECKV_CASE(RR) case RR: return launch_clustered(decompress_fast_kernel<T, RR>, RR, n, st, args);
+#define SPECKV_CASE(RR) case RR: return launch_clustered(decompress_fast_kernel<T, RR>, RR, a.n_groups, st, a, scr);
         SPECKV_CASE(1) SPECKV_CASE(2) SPECKV_CASE(4) SPECKV_CASE(8) SPECKV_CASE(16) SPECKV_CASE(32) SPECKV_CASE(64) SPECKV_CASE(128)
 #undef SPECKV_CASE
         default: return cudaErrorInvalidValue;

@@ -182,12 +182,7 @@ __device__ __forceinline__ void load_elems(const T* __restrict__ gin, uint32_t s
 // ---------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
-compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_groups,
-                            uint8_t* __restrict__ payload, size_t slot_bytes,
-                            float* __restrict__ scales, uint32_t* __restrict__ comp_bytes,
-                            const uint32_t* __restrict__ only_flagged, const uint32_t* __restrict__ elem_index,
-                            bool max_scale, const uint64_t* __restrict__ slot_offsets,
-                            const uint32_t* __restrict__ group_len) {
+compress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged) {
     __shared__ __align__(16) uint16_t stage[kTile + 16];
     __shared__ int wbuf[kWarps];
     __shared__ float fbuf[kWarps];
@@ -196,17 +191,18 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
     const int tid = threadIdx.x;
 
     __shared__ uint32_t smask[kWarps];
-    GroupIter it(only_flagged, n_groups, smask);
+    const uint32_t G = a.group_elems;
+    GroupIter it(only_flagged, a.n_groups, smask);
     for (uint32_t g; it.next(g);) {
-        const T* gin = in + (size_t)(elem_index ? elem_index[g] : g) * G;
-        uint8_t* gout = payload + (slot_offsets ? (size_t)slot_offsets[g] : (size_t)g * slot_bytes);   // packed emission: the slot reserved by the tuned kernel
+        const T* gin = a.elem_block(static_cast<const T*>(a.in), g, G);
+        uint8_t* gout = a.block_payload(g);   // packed emission: the slot reserved by the tuned kernel
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gin) & 15) == 0;
-        const uint32_t n = group_len ? min(group_len[g], G) : G;   // ragged calls: the group is the block's first n elements
+        const uint32_t n = a.group_length(g, G);
 
         // second pass behind the tuned kernel: that kernel already took the group max and left its bits in
         // comp_bytes[g] (overwritten with the size below), so the input is read once here, not twice
-        const float m = only_flagged ? __uint_as_float(comp_bytes[g]) : group_absmax<T>(gin, n, vec_ok, fbuf);
-        const float s = scale_for(m, max_scale);
+        const float m = only_flagged ? __uint_as_float(a.comp_bytes[g]) : group_absmax<T>(gin, n, vec_ok, fbuf);
+        const float s = scale_for(m, scheme_max_scale(a.scheme));
         const bool fast = fast_quant_ok<T>(m);
         float r = 0.0f, rl = 0.0f;
         if (fast) recip_hi_lo(s, r, rl);
@@ -312,8 +308,8 @@ compress_rle_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gro
             if (tid == 0) *reinterpret_cast<uint4*>(gout + (size_t)stage_base * 2) = *reinterpret_cast<const uint4*>(stage);
         }
         if (tid == 0) {
-            scales[g] = s;
-            comp_bytes[g] = 2u * (uint32_t)carry_nh;
+            a.scales[g] = s;
+            a.comp_bytes[g] = 2u * (uint32_t)carry_nh;
         }
         __syncthreads();
     }
@@ -357,7 +353,7 @@ __device__ __forceinline__ void decode_runs_region(RunsSmem& rs, int wid, int la
                                                    uint32_t o, T* __restrict__ gout) {
     constexpr unsigned kAll = 0xffffffffu;
     const uint32_t O0 = o * 2048u;
-    const uint32_t e_total = pre[R].x;
+    const uint32_t e_total = __ldg(pre + R).x;
     if (O0 >= e_total) return;
     const uint32_t n_out = min(2048u, e_total - O0), Oend = O0 + n_out;
     uint32_t* bm = rs.bitmap[wid];
@@ -372,7 +368,7 @@ __device__ __forceinline__ void decode_runs_region(RunsSmem& rs, int wid, int la
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         const uint32_t r = (uint32_t)lane + 32u * i;
-        mine[i] = r < R ? pre[r + 1] : make_uint2(0xffffffffu, 0u);
+        mine[i] = r < R ? __ldg(pre + r + 1) : make_uint2(0xffffffffu, 0u);
         cnt += (r < R && mine[i].x <= O0) ? 1u : 0u;
     }
     const uint32_t r0 = __reduce_add_sync(kAll, cnt);
@@ -519,19 +515,13 @@ __device__ __forceinline__ void decode_runs_region(RunsSmem& rs, int wid, int la
 // ---------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
-decompress_rle_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes,
-                              const float* __restrict__ scales, const uint32_t* __restrict__ comp_bytes,
-                              uint32_t G, uint32_t n_groups, T* __restrict__ out,
-                              uint32_t* __restrict__ out_elems, const uint32_t* __restrict__ only_flagged,
-                              const uint32_t* __restrict__ src_index, const uint64_t* __restrict__ slot_offsets,
-                              const uint32_t* __restrict__ elem_index, const uint32_t* __restrict__ n_groups_dev,
-                              const uint32_t* __restrict__ runs_list, uint32_t* __restrict__ runs_counters,
-                              const uint2* __restrict__ runs_prefix, uint32_t runs_R) {
-    if (n_groups_dev) n_groups = min(n_groups, *n_groups_dev);   // request count held on the device
+decompress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged, const DecodeScratch runs) {
+    const uint32_t G = a.group_elems, n_groups = a.live_groups();
+    T* out = static_cast<T*>(a.out);
     // ---- first the groups flagged for run expansion: warps of the whole grid stride over (group, output region) ----
-    if (runs_counters) {
+    if (runs.counters) {
         __shared__ RunsSmem rs;
-        const uint32_t n_runs = *reinterpret_cast<const volatile uint32_t*>(runs_counters);
+        const uint32_t n_runs = *reinterpret_cast<const volatile uint32_t*>(runs.counters);
         if (n_runs) {
             {   // selectors: output j of a chunk takes table byte popc(heads up to and including j) - (head at 0)
                 const uint32_t hb = threadIdx.x;
@@ -544,14 +534,14 @@ decompress_rle_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_b
             }
             __syncthreads();
             const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
-            const uint64_t n_items = (uint64_t)n_runs * runs_R;
+            const uint32_t R = runs.regions;
+            const uint64_t n_items = (uint64_t)n_runs * R;
             for (uint64_t it = (uint64_t)blockIdx.x * kWarps + wid; it < n_items; it += (uint64_t)gridDim.x * kWarps) {
-                const uint32_t g = runs_list[it / runs_R], o = (uint32_t)(it % runs_R);
-                const uint32_t gi = src_index ? src_index[g] : g;
-                const uint8_t* gp = payload + (slot_offsets ? (size_t)slot_offsets[gi] : (size_t)gi * slot_bytes);
-                const uint32_t npairs = min(comp_bytes[gi] >> 1, runs_R * 2048u);
-                decode_runs_region<T>(rs, wid, lane, gp, npairs, scales[gi], runs_prefix + (size_t)g * (runs_R + 1), runs_R, o,
-                                      out + (size_t)(elem_index ? elem_index[g] : g) * G);
+                const uint32_t g = __ldg(runs.list + it / R), o = (uint32_t)(it % R);
+                const uint32_t gi = a.stored_block(g);
+                const uint32_t npairs = min(__ldg(a.comp_bytes + gi) >> 1, R * 2048u);
+                decode_runs_region<T>(rs, wid, lane, a.block_payload(gi), npairs, __ldg(a.scales + gi), runs.prefix + (size_t)g * (R + 1),
+                                      R, o, a.elem_block(out, g, G));
             }
             // the last CTA to get here clears the list for the next call (every CTA has read the count by then).  Only
             // when there was a list: with n_runs == 0 both counters are zero already, and one atomic per CTA on the same
@@ -559,9 +549,9 @@ decompress_rle_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_b
             __syncthreads();
             if (threadIdx.x == 0) {
                 __threadfence();
-                if (atomicAdd(runs_counters + 1, 1u) == gridDim.x - 1) {
-                    runs_counters[0] = 0u;
-                    runs_counters[1] = 0u;
+                if (atomicAdd(runs.counters + 1, 1u) == gridDim.x - 1) {
+                    runs.counters[0] = 0u;
+                    runs.counters[1] = 0u;
                 }
             }
         }
@@ -581,13 +571,13 @@ decompress_rle_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_b
     __shared__ uint32_t smask[kWarps];
     GroupIter it(only_flagged, n_groups, smask);
     for (uint32_t g; it.next(g);) {
-        const uint32_t gi = src_index ? src_index[g] : g; // which stored block this output group decodes
-        const uint8_t* gp = payload + (slot_offsets ? (size_t)slot_offsets[gi] : (size_t)gi * slot_bytes);
-        uint32_t npairs = comp_bytes[gi] >> 1;  // a trailing odd byte is ignored (:245-247)
-        npairs = min(npairs, (uint32_t)(slot_bytes >> 1));
-        const float s = scales[gi];
+        const uint32_t gi = a.stored_block(g);
+        const uint8_t* gp = a.block_payload(gi);
+        uint32_t npairs = __ldg(a.comp_bytes + gi) >> 1;  // a trailing odd byte is ignored (:245-247)
+        npairs = min(npairs, (uint32_t)(a.slot_bytes >> 1));
+        const float s = __ldg(a.scales + gi);
         const bool special = scale_is_special(s);
-        T* gout = out + (size_t)(elem_index ? elem_index[g] : g) * G;
+        T* gout = a.elem_block(out, g, G);
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gout) & 15) == 0;
         const bool in_vec_ok = (reinterpret_cast<uintptr_t>(gp) & 15) == 0;
 
@@ -663,7 +653,7 @@ decompress_rle_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_b
             out_pos = chunk_end;
             acc = (acc + (uint32_t)totS) & 0xffu;
         }
-        if (tid == 0 && out_elems) out_elems[g] = out_pos;
+        if (tid == 0 && a.out_elems) a.out_elems[g] = out_pos;
     }
 }
 
@@ -672,23 +662,20 @@ decompress_rle_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_b
 // ---------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
-compress_int8_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_groups,
-                             uint8_t* __restrict__ payload, size_t slot_bytes,
-                             float* __restrict__ scales, uint32_t* __restrict__ comp_bytes,
-                             const uint32_t* __restrict__ only_flagged, const uint32_t* __restrict__ elem_index,
-                             bool max_scale, const uint32_t* __restrict__ group_len) {
+compress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged) {
     __shared__ float fbuf[kWarps];
     __shared__ uint32_t smask[kWarps];
     const int tid = threadIdx.x;
-    GroupIter it(only_flagged, n_groups, smask);
+    const uint32_t G = a.group_elems;
+    GroupIter it(only_flagged, a.n_groups, smask);
     for (uint32_t g; it.next(g);) {
-        const T* gin = in + (size_t)(elem_index ? elem_index[g] : g) * G;
-        uint8_t* gout = payload + (size_t)g * slot_bytes;
+        const T* gin = a.elem_block(static_cast<const T*>(a.in), g, G);
+        uint8_t* gout = static_cast<uint8_t*>(a.payload) + (size_t)g * a.slot_bytes;   // no packed emission with codes only
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gin) & 15) == 0;
-        const uint32_t n = group_len ? min(group_len[g], G) : G;
+        const uint32_t n = a.group_length(g, G);
         // behind the tuned kernel the group max is already known (left in comp_bytes[g])
-        const float m = only_flagged ? __uint_as_float(comp_bytes[g]) : group_absmax<T>(gin, n, vec_ok, fbuf);
-        const float s = scale_for(m, max_scale);
+        const float m = only_flagged ? __uint_as_float(a.comp_bytes[g]) : group_absmax<T>(gin, n, vec_ok, fbuf);
+        const float s = scale_for(m, scheme_max_scale(a.scheme));
         const bool fast = fast_quant_ok<T>(m);
         float r = 0.0f, rl = 0.0f;
         if (fast) recip_hi_lo(s, r, rl);
@@ -709,42 +696,40 @@ compress_int8_generic_kernel(const T* __restrict__ in, uint32_t G, uint32_t n_gr
             }
         }
         if (tid == 0) {
-            scales[g] = s;
-            comp_bytes[g] = n;
+            a.scales[g] = s;
+            a.comp_bytes[g] = n;
         }
     }
 }
 
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
-decompress_int8_generic_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes,
-                               const float* __restrict__ scales, const uint32_t* __restrict__ comp_bytes,
-                               uint32_t G, uint32_t n_groups, T* __restrict__ out,
-                               uint32_t* __restrict__ out_elems, const uint32_t* __restrict__ only_flagged,
-                               const uint32_t* __restrict__ src_index, const uint64_t* __restrict__ slot_offsets,
-                               const uint32_t* __restrict__ elem_index, const uint32_t* __restrict__ n_groups_dev) {
+decompress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged) {
     __shared__ uint32_t smask[kWarps];
     const int tid = threadIdx.x;
-    if (n_groups_dev) n_groups = min(n_groups, *n_groups_dev);
-    GroupIter it(only_flagged, n_groups, smask);
+    const uint32_t G = a.group_elems;
+    GroupIter it(only_flagged, a.live_groups(), smask);
     for (uint32_t g; it.next(g);) {
-        const uint32_t gi = src_index ? src_index[g] : g;
-        const uint8_t* gp = payload + (slot_offsets ? (size_t)slot_offsets[gi] : (size_t)gi * slot_bytes);
-        const uint32_t n = min(min(comp_bytes[gi], G), (uint32_t)slot_bytes);
-        const float s = scales[gi];
-        T* gout = out + (size_t)(elem_index ? elem_index[g] : g) * G;
+        const uint32_t gi = a.stored_block(g);
+        const uint8_t* gp = a.block_payload(gi);
+        const uint32_t n = min(min(__ldg(a.comp_bytes + gi), G), (uint32_t)a.slot_bytes);
+        const float s = __ldg(a.scales + gi);
+        T* gout = a.elem_block(static_cast<T*>(a.out), g, G);
         const bool special = scale_is_special(s);
         for (uint32_t i = tid; i < n; i += kThreads)
-            gout[i] = special ? narrow_special<T>(dequantize_special(gp[i], s)) : narrow<T>(dequantize(gp[i], s));
-        if (tid == 0 && out_elems) out_elems[g] = n;
+            gout[i] = special ? narrow_special<T>(dequantize_special(__ldg(gp + i), s)) : narrow<T>(dequantize(__ldg(gp + i), s));
+        if (tid == 0 && a.out_elems) a.out_elems[g] = n;
     }
 }
 
 // scheme FP16: raw 16-bit passthrough of fp16 / bf16 groups
 // raw copy of whole groups into their slots (and the metadata), 16 bytes per thread and step when both sides allow
 __global__ void __launch_bounds__(kThreads)
-passthrough_in_kernel(const uint16_t* __restrict__ in, uint32_t G, uint32_t n_groups, uint8_t* __restrict__ payload,
-                      size_t slot_bytes, float* __restrict__ scales, uint32_t* __restrict__ comp_bytes) {
+passthrough_in_kernel(const __grid_constant__ CodecArgs a) {
+    const uint16_t* in = static_cast<const uint16_t*>(a.in);
+    uint8_t* payload = static_cast<uint8_t*>(a.payload);
+    const size_t slot_bytes = a.slot_bytes;
+    const uint32_t G = a.group_elems, n_groups = a.n_groups;
     const bool vec_ok = ((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(payload) | slot_bytes) & 15) == 0 && G % 8 == 0;
     const uint64_t vec_per_group = G / 8;
     if (vec_ok) {
@@ -761,24 +746,21 @@ passthrough_in_kernel(const uint16_t* __restrict__ in, uint32_t G, uint32_t n_gr
         }
     }
     for (uint32_t g = blockIdx.x * kThreads + threadIdx.x; g < n_groups; g += gridDim.x * kThreads) {
-        scales[g] = 1.0f;
-        comp_bytes[g] = G * 2u;
+        a.scales[g] = 1.0f;
+        a.comp_bytes[g] = G * 2u;
     }
 }
 
 __global__ void __launch_bounds__(kThreads)
-passthrough_out_kernel(const uint8_t* __restrict__ payload, size_t slot_bytes,
-                       const uint32_t* __restrict__ comp_bytes, uint32_t G, uint32_t n_groups,
-                       uint16_t* __restrict__ out, uint32_t* __restrict__ out_elems,
-                       const uint32_t* __restrict__ src_index, const uint64_t* __restrict__ slot_offsets,
-                       const uint32_t* __restrict__ n_groups_dev) {
-    if (n_groups_dev) n_groups = min(n_groups, *n_groups_dev);
+passthrough_out_kernel(const __grid_constant__ CodecArgs a) {
+    const uint32_t G = a.group_elems, n_groups = a.live_groups();
+    uint16_t* out = static_cast<uint16_t*>(a.out);
     for (uint32_t g = blockIdx.x; g < n_groups; g += gridDim.x) {
-        const uint32_t gi = src_index ? src_index[g] : g;
-        const uint16_t* gp = reinterpret_cast<const uint16_t*>(payload + (slot_offsets ? (size_t)slot_offsets[gi] : (size_t)gi * slot_bytes));
-        const uint32_t n = min(min(comp_bytes[gi] >> 1, G), (uint32_t)(slot_bytes >> 1));
-        for (uint32_t i = threadIdx.x; i < n; i += kThreads) out[(size_t)g * G + i] = gp[i];
-        if (threadIdx.x == 0 && out_elems) out_elems[g] = n;
+        const uint32_t gi = a.stored_block(g);
+        const uint16_t* gp = reinterpret_cast<const uint16_t*>(a.block_payload(gi));
+        const uint32_t n = min(min(__ldg(a.comp_bytes + gi) >> 1, G), (uint32_t)(a.slot_bytes >> 1));
+        for (uint32_t i = threadIdx.x; i < n; i += kThreads) out[(size_t)g * G + i] = __ldg(gp + i);
+        if (threadIdx.x == 0 && a.out_elems) a.out_elems[g] = n;
     }
 }
 
@@ -795,45 +777,26 @@ inline int grid_for(uint32_t n_groups, int sm_count, int per_sm) {
 
 template <typename T>
 static cudaError_t launch_compress_t(const CodecArgs& a, cudaStream_t st, const uint32_t* only_flagged) {
-    const T* in = static_cast<const T*>(a.in);
-    uint8_t* pay = static_cast<uint8_t*>(a.payload);
     // as the second pass behind a tuned kernel almost nothing is flagged: a smaller grid (its launch and drain are
     // what an empty pass costs) still spreads the few flagged groups over every SM
-    const int grid = grid_for(a.n_groups, a.sm_count, only_flagged ? kSecondPassPerSm : 8);
-    if (scheme_is_rle(a.scheme)) {
-        compress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(in, a.group_elems, a.n_groups, pay, a.slot_bytes,
-                                                                  a.scales, a.comp_bytes, only_flagged, a.elem_index,
-                                                                  scheme_max_scale(a.scheme), a.pack_offsets, a.group_len);
-    } else {
-        compress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(in, a.group_elems, a.n_groups, pay, a.slot_bytes,
-                                                                   a.scales, a.comp_bytes, only_flagged, a.elem_index,
-                                                                   scheme_max_scale(a.scheme), a.group_len);
-    }
+    const int grid = grid_for(a.n_groups, current_sm_count(), only_flagged ? kSecondPassPerSm : 8);
+    if (scheme_is_rle(a.scheme)) compress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged);
+    else compress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged);
     count_launch();
     return cudaGetLastError();
 }
 
 template <typename T>
 static cudaError_t launch_decompress_t(const CodecArgs& a, cudaStream_t st, const uint32_t* only_flagged, const DecodeScratch* runs) {
-    T* out = static_cast<T*>(a.out);
-    const uint8_t* pay = static_cast<const uint8_t*>(a.payload);
-    int grid = grid_for(a.n_groups, a.sm_count, only_flagged ? kSecondPassPerSm : 8);
+    const int sm_count = current_sm_count();
+    int grid = grid_for(a.n_groups, sm_count, only_flagged ? kSecondPassPerSm : 8);
     if (runs) {   // a few flagged groups still spread over the device: one warp per output region, up to 2 CTAs per SM
         const long long want = ((long long)a.n_groups * runs->regions + kWarps - 1) / kWarps;
-        const long long cap = (long long)a.sm_count * 2;
+        const long long cap = (long long)sm_count * 2;
         grid = (int)std::max<long long>(grid, std::min(want, cap));
     }
-    if (scheme_is_rle(a.scheme)) {
-        decompress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(pay, a.slot_bytes, a.scales, a.comp_bytes,
-                                                                    a.group_elems, a.n_groups, out, a.out_elems, only_flagged, a.src_index,
-                                                                    a.slot_offsets, a.elem_index, a.n_groups_dev,
-                                                                    runs ? runs->list : nullptr, runs ? runs->counters : nullptr,
-                                                                    runs ? runs->prefix : nullptr, runs ? runs->regions : 0u);
-    } else {
-        decompress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(pay, a.slot_bytes, a.scales, a.comp_bytes,
-                                                                     a.group_elems, a.n_groups, out, a.out_elems, only_flagged,
-                                                                     a.src_index, a.slot_offsets, a.elem_index, a.n_groups_dev);
-    }
+    if (scheme_is_rle(a.scheme)) decompress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged, runs ? *runs : DecodeScratch{});
+    else decompress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged);
     count_launch();
     return cudaGetLastError();
 }
@@ -842,9 +805,7 @@ cudaError_t launch_compress_generic(const CodecArgs& a, cudaStream_t st, const u
     if (a.n_groups == 0) return cudaSuccess;
     if (a.scheme == 0) {
         if (a.elem_index) return cudaErrorInvalidValue;   // the raw passthrough has no gather form
-        passthrough_in_kernel<<<a.sm_count * 8, kThreads, 0, st>>>(static_cast<const uint16_t*>(a.in), a.group_elems, a.n_groups,
-                                                                   static_cast<uint8_t*>(a.payload), a.slot_bytes, a.scales,
-                                                                   a.comp_bytes);
+        passthrough_in_kernel<<<current_sm_count() * 8, kThreads, 0, st>>>(a);
         count_launch();
         return cudaGetLastError();
     }
@@ -859,9 +820,7 @@ cudaError_t launch_decompress_generic(const CodecArgs& a, cudaStream_t st, const
     if (a.n_groups == 0) return cudaSuccess;
     if (a.scheme == 0) {
         if (a.elem_index) return cudaErrorInvalidValue;
-        passthrough_out_kernel<<<grid_for(a.n_groups, a.sm_count, 8), kThreads, 0, st>>>(
-            static_cast<const uint8_t*>(a.payload), a.slot_bytes, a.comp_bytes, a.group_elems, a.n_groups,
-            static_cast<uint16_t*>(a.out), a.out_elems, a.src_index, a.slot_offsets, a.n_groups_dev);
+        passthrough_out_kernel<<<grid_for(a.n_groups, current_sm_count(), 8), kThreads, 0, st>>>(a);
         count_launch();
         return cudaGetLastError();
     }

@@ -501,7 +501,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         const int b = (int)(chunk % Tier::kBuf);
         // buffer b is free once the payload copy of chunk - 2 has completed
         cudaStreamWaitEvent(st, t.ev_copy[b], 0);
-        CodecArgs a;
+        CodecArgs a(slot, group_elems, ng, dtype, scheme);
         // paged form: the chunk's groups are the cache blocks its slice of the block table names
         a.in = d_block_table ? d_in : (const void*)((const char*)d_in + g0 * group_elems * esz);
         a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
@@ -509,12 +509,6 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         a.payload = t.d_slots[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
-        a.slot_bytes = slot;
-        a.group_elems = (uint32_t)group_elems;
-        a.n_groups = (uint32_t)ng;
-        a.dtype = dtype;
-        a.scheme = scheme;
-        a.sm_count = current_sm_count();
         if (compress_packed_supported(a)) {
             // 4 KiB page groups: the compress kernel places the payloads itself (look-back over per-CTA totals), the
             // packed stream is written once.  A group the generic kernel encodes keeps a whole slot inside the
@@ -656,19 +650,13 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
         cudaMemcpyAsync(t.d_scales[b], t.h_scales[b], ng * 4, cudaMemcpyHostToDevice, t.copy_st[b]);
         cudaEventRecord(t.ev_copy[b], t.copy_st[b]);
         cudaStreamWaitEvent(st, t.ev_copy[b], 0);
-        CodecArgs a;
+        CodecArgs a(slot, group_elems, ng, dtype, scheme);
         a.out = d_block_table ? d_out : (void*)((char*)d_out + g0 * group_elems * esz);
         a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
         a.payload = t.d_packed[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
         a.slot_offsets = t.d_offsets[b];
-        a.slot_bytes = slot;
-        a.group_elems = (uint32_t)group_elems;
-        a.n_groups = (uint32_t)ng;
-        a.dtype = dtype;
-        a.scheme = scheme;
-        a.sm_count = current_sm_count();
         if (scheme == SPECKV_COMP_FP16 && (d_block_table || dtype == SPECKV_DTYPE_F32)) return SPECKV_ERR_INVAL;
         // a chunk holding ragged blocks counts what was decoded; otherwise every block is a whole group
         if (any_ragged) a.out_elems = t.d_oel[b];
@@ -874,7 +862,7 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
     e = launch_fetch_gather(t.d_dir, src_off, offsets, d_n_requests, (uint32_t)n, total, staging, current_sm_count(), st);
     if (e != cudaSuccess) return status_of(e);
     // the staged payloads form a packed container: the codec's decoders take it as it is
-    CodecArgs a;
+    CodecArgs a(slot, group_elems, n, dtype, (int)scheme);
     a.out = d_out;
     a.elem_index = d_block_table;
     a.payload = staging;
@@ -883,12 +871,6 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
     a.comp_bytes = comp;
     a.out_elems = d_out_elems;
     a.n_groups_dev = d_n_requests;
-    a.slot_bytes = slot;
-    a.group_elems = (uint32_t)group_elems;
-    a.n_groups = (uint32_t)n;
-    a.dtype = dtype;
-    a.scheme = (int)scheme;
-    a.sm_count = current_sm_count();
     return status_of(launch_decompress(a, st));
 }
 
