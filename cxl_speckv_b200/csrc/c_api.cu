@@ -62,7 +62,6 @@ static std::unique_ptr<Runtime> g_rt;
 static speckv_status_t fetch_pages_locked(Runtime& rt, uint64_t handle, KvAllocation& a, const PoolBinding& pb,
                                           uint64_t p0, uint64_t p1, cudaStream_t st) {
     (void)rt;
-    (void)handle;
     std::vector<uint64_t> ids;
     uint64_t run_start = p0;
     // a run of pages to restore: they are marked resident only once their restore has succeeded (a failed restore
@@ -85,7 +84,7 @@ static speckv_status_t fetch_pages_locked(Runtime& rt, uint64_t handle, KvAlloca
                 return SPECKV_ERR_INVAL;
             }
             if (ids.empty()) run_start = p;
-            ids.push_back(pg.virt_page_id);
+            ids.push_back(PageTable::tier_key(handle, p));
         } else {
             speckv_status_t rc = flush();
             if (rc != SPECKV_OK) return rc;
@@ -173,8 +172,8 @@ speckv_status_t speckv_free(speckv_handle_t handle) {
         KvAllocation* a = g_rt->table.find(handle);
         if (a && pit->second.tier) {
             std::vector<uint64_t> ids;
-            for (const KvPage& pg : a->pages)
-                if (pg.flags & kFlagCompressed) ids.push_back(pg.virt_page_id);
+            for (uint64_t p = 0; p < a->pages.size(); ++p)
+                if (a->pages[p].flags & kFlagCompressed) ids.push_back(PageTable::tier_key(handle, p));
             if (!ids.empty()) speckv_ext_tier_drop(pit->second.tier, ids.data(), ids.size());
         }
         g_rt->pools.erase(pit);
@@ -405,7 +404,7 @@ speckv_status_t speckv_ext_offload_pages(speckv_handle_t handle, uint64_t first_
     for (uint64_t p = first_page; p < last; ++p) {
         if (a->pages[p].flags & (kFlagL1 | kFlagL2)) {
             if (ids.empty()) run_start = p;
-            ids.push_back(a->pages[p].virt_page_id);
+            ids.push_back(PageTable::tier_key(handle, p));
         } else {
             speckv_status_t rc = flush();
             if (rc != SPECKV_OK) return rc;

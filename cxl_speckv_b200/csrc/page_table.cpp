@@ -29,7 +29,8 @@ KvAllocation* PageTable::find(uint64_t handle) {
 
 KvPage* PageTable::find_page(uint64_t virt) {
     // ids are unambiguous for allocations below 4 GiB (page index < 2^20); beyond that
-    // the reference's own map keys collide across handles as well.
+    // the reference's own map keys collide across handles as well.  (The host tier keys pool pages by
+    // tier_key, which stays unique there.)
     KvAllocation* a = find(virt >> 32);
     if (!a) return nullptr;
     const uint64_t i = (virt & 0xFFFFFFFFULL) >> 12;

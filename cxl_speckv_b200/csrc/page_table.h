@@ -54,6 +54,13 @@ public:
 
     static uint64_t virt_page_id(uint64_t handle, uint64_t i) { return (handle << 32) | (i << 12); }
     static uint64_t phys_page_id(uint64_t handle, uint64_t i) { return kPhysBase + (handle << 20) + (i << 12); }
+    // The id a bound pool's page i is stored under in the host tier.  virt_page_id for i < 2^20; from there on
+    // i << 12 reaches the handle bits and virt_page_id repeats the id of page i - 2^20 of the same handle (h odd) or
+    // of handle h + 1 (h even).  Those pages take (h << 32) | ((i mod 2^20) << 12) | (i >> 20): its low 12 bits are
+    // non-zero, so it equals no page-aligned id, and it is unique per (handle, page) for i < 2^32 (16 TiB).
+    static uint64_t tier_key(uint64_t handle, uint64_t i) {
+        return i < (1ull << 20) ? virt_page_id(handle, i) : (handle << 32) | ((i & 0xFFFFFull) << 12) | (i >> 20);
+    }
     // gpu_addr of the fetch descriptor, speckv_allocator.cpp:124
     static uint64_t fetch_gpu_addr(uint64_t virt) { return 0x8000000000ULL + (virt & 0xFFFFFFFFFFFFULL); }
 

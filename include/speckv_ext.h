@@ -397,7 +397,12 @@ SPECKV_API speckv_status_t speckv_ext_set_pool_dtype(speckv_handle_t handle, spe
 SPECKV_API speckv_status_t speckv_ext_get_compression_scheme(int* out_scheme);
 /* Demote pages to the host tier (compress + move; flags: L1/L2 cleared, compressed set) /
  * promote them back (restore; flags: L2 set; a page is marked resident only after its restore succeeded).
- * Pages are groups of the pool's element type, stored under the current compression scheme. */
+ * Pages are groups of the pool's element type, stored under the current compression scheme.
+ * Block ids in the tier: page i of handle h is stored under its virt_page_id, (h << 32) | (i << 12), for
+ * i < 2^20.  Pages past the first 4 GiB of an allocation (i >= 2^20) would repeat another page's virt_page_id there,
+ * so they are stored under (h << 32) | ((i & 0xFFFFF) << 12) | (i >> 20), whose low 12 bits are non-zero: unique
+ * per (handle, page) for i < 2^32.  The page table (speckv_ext_page_table_export, speckv_ext_page_lookup) keeps the
+ * reference's ids. */
 SPECKV_API speckv_status_t speckv_ext_offload_pages(speckv_handle_t handle, uint64_t first_page, uint64_t n_pages,
                                                     void* cuda_stream);
 SPECKV_API speckv_status_t speckv_ext_fetch_pages(speckv_handle_t handle, uint64_t first_page, uint64_t n_pages,
