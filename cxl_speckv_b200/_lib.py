@@ -148,6 +148,17 @@ def lib() -> C.CDLL:
     L.speckv_ext_tier_fetch.argtypes = [vp, vp, vp, sz, sz, C.c_int, C.c_int, vp, vp, vp, vp, vp, sz, vp]
     L.speckv_ext_tier_fetch.restype = C.c_int
     L.speckv_ext_tier_get_stats.argtypes = [vp, C.POINTER(TierStats)]; L.speckv_ext_tier_get_stats.restype = None
+    L.speckv_ext_cache_set_create.argtypes = [vp, sz, sz, sz, C.c_int, C.POINTER(vp)]
+    L.speckv_ext_cache_set_create.restype = C.c_int
+    L.speckv_ext_cache_set_destroy.argtypes = [vp]; L.speckv_ext_cache_set_destroy.restype = None
+    L.speckv_ext_compress_gather_set.argtypes = [vp, vp, vp, vp, sz, vp, sz, vp, vp, C.c_int, vp]
+    L.speckv_ext_compress_gather_set.restype = C.c_int
+    L.speckv_ext_decompress_scatter_set.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp, sz, vp, C.c_int, vp]
+    L.speckv_ext_decompress_scatter_set.restype = C.c_int
+    L.speckv_ext_tier_offload_set.argtypes = [vp, vp, vp, vp, vp, sz, vp, vp]; L.speckv_ext_tier_offload_set.restype = C.c_int
+    L.speckv_ext_tier_restore_set.argtypes = [vp, vp, sz, vp, vp, vp, vp]; L.speckv_ext_tier_restore_set.restype = C.c_int
+    L.speckv_ext_tier_fetch_set.argtypes = [vp, vp, vp, sz, vp, vp, vp, C.c_int, vp, vp, vp, sz, vp]
+    L.speckv_ext_tier_fetch_set.restype = C.c_int
     L.speckv_ext_atu_create.argtypes = [C.c_uint32, C.POINTER(vp)]; L.speckv_ext_atu_create.restype = C.c_int
     L.speckv_ext_atu_destroy.argtypes = [vp]; L.speckv_ext_atu_destroy.restype = None
     L.speckv_ext_atu_translate.argtypes = [vp, vp, vp, sz, vp]; L.speckv_ext_atu_translate.restype = C.c_int

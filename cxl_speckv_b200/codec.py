@@ -209,6 +209,145 @@ def decompress_scatter(c: CompressedKV, cache: torch.Tensor, block_table: torch.
     return cache
 
 
+class KVCacheSet:
+    """A model's paged KV caches registered as one set (speckv_ext_cache_set_create): one tensor per layer and K|V,
+    all of the same shape, dtype, strides and device, each [num_blocks, ...] with block b at index b.  A block must be
+    contiguous; consecutive blocks may lie further apart (a K or V view of vLLM's [num_blocks, 2, ...] layout).
+
+    Calls through the set name each group by (cache index, block number): see groups().  The set keeps the tensors
+    alive; close() (or garbage collection) releases the native set, which must not happen while calls that use it
+    are in flight or captured in a graph that is still replayed.  On CPU tensors only the geometry and groups() are
+    available (no native set is created)."""
+
+    def __init__(self, caches):
+        caches = list(caches)
+        if not caches:
+            raise ValueError("KVCacheSet needs at least one cache")
+        c0 = caches[0]
+        for c in caches:
+            if not isinstance(c, torch.Tensor):
+                raise TypeError("KVCacheSet takes tensors")
+            if c.dtype not in _DTYPES:
+                raise TypeError(f"unsupported dtype {c.dtype}")
+            if c.dim() < 2 or c.shape[0] == 0 or c[0].numel() == 0:
+                raise ValueError("each cache must be [num_blocks, ...] with non-empty blocks")
+            if c.shape != c0.shape or c.dtype != c0.dtype or c.stride() != c0.stride() or c.device != c0.device:
+                raise ValueError("the caches of a set must agree in shape, dtype, strides and device")
+        if not c0[0].is_contiguous():
+            raise ValueError("a cache block must be contiguous")
+        self.caches = caches
+        self.num_blocks = c0.shape[0]
+        self.block_elems = c0[0].numel()
+        self.block_stride = c0.stride(0)
+        if self.block_stride < self.block_elems:
+            raise ValueError("the blocks of a cache overlap (stride(0) < block size)")
+        self.dtype = c0.dtype
+        self.device = c0.device
+        self._h = C.c_void_p()
+        if c0.is_cuda:
+            bases = (C.c_void_p * len(caches))(*[c.data_ptr() for c in caches])
+            with torch.cuda.device(self.device):
+                check(lib().speckv_ext_cache_set_create(bases, len(caches), self.block_elems, self.block_stride,
+                                                        _DTYPES[self.dtype], C.byref(self._h)),
+                      "speckv_ext_cache_set_create")
+
+    def __len__(self) -> int:
+        return len(self.caches)
+
+    def handle(self) -> C.c_void_p:
+        if not self._h:
+            raise ValueError("this KVCacheSet has no native set (CPU tensors, or closed)")
+        return self._h
+
+    def groups(self, block_table: torch.Tensor):
+        """The cache-major cross product of all caches with block_table: (cache_index, block_index), int32 tensors of
+        len(self) * block_table.numel() entries on block_table's device, all blocks of cache 0 first.  Torch ops only
+        (capturable)."""
+        b = block_table.reshape(-1).to(torch.int32)
+        n, nc = b.numel(), len(self.caches)
+        cache_index = torch.arange(nc, dtype=torch.int32, device=b.device).view(nc, 1).expand(nc, n).reshape(-1)
+        return cache_index, b.view(1, n).expand(nc, n).reshape(-1)
+
+    def close(self):
+        if self._h:
+            lib().speckv_ext_cache_set_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):  # pragma: no cover
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _set_groups(cset: KVCacheSet, cache_index: torch.Tensor, block_table: torch.Tensor):
+    """Checked (cache_index, block_table) of a set call: contiguous int32 on the set's device, equal lengths."""
+    if not isinstance(cset, KVCacheSet):
+        raise TypeError("expected a KVCacheSet")
+    dev = cset.device
+    cache_index = cache_index.to(device=dev, dtype=torch.int32).contiguous()
+    block_table = block_table.to(device=dev, dtype=torch.int32).contiguous()
+    if cache_index.numel() != block_table.numel():
+        raise ValueError("cache_index and block_table differ in length")
+    return cache_index, block_table
+
+
+def compress_gather_set(cset: KVCacheSet, cache_index: torch.Tensor, block_table: torch.Tensor,
+                        lengths: Optional[torch.Tensor] = None, scheme: int = COMP_INT8_DELTA_RLE,
+                        out: Optional[CompressedKV] = None) -> CompressedKV:
+    """compress_gather across a cache set: stored group i encodes block block_table[i] of cache cache_index[i]
+    (e.g. from cset.groups(table)).  lengths (optional, CUDA int32, one per group) stores only the first lengths[i]
+    elements of each block, as compress_ragged does.  Schemes 1-4."""
+    cache_index, block_table = _set_groups(cset, cache_index, block_table)
+    n_groups = block_table.numel()
+    if lengths is not None:
+        if not lengths.is_cuda or lengths.dtype != torch.int32 or lengths.device != cset.device:
+            raise TypeError("lengths must be an int32 tensor on the device of the set")
+        lengths = lengths.contiguous()
+        if lengths.numel() != n_groups:
+            raise ValueError("lengths must hold one entry per group")
+    dev = cset.device
+    sb = slot_bytes(cset.block_elems, scheme)
+    if out is None:
+        out = CompressedKV(torch.empty((n_groups, sb), dtype=torch.uint8, device=dev),
+                           torch.empty(n_groups, dtype=torch.float32, device=dev),
+                           torch.empty(n_groups, dtype=torch.int32, device=dev),
+                           cset.block_elems, cset.dtype, scheme)
+    with torch.cuda.device(dev):
+        st = lib().speckv_ext_compress_gather_set(cset.handle(), cache_index.data_ptr(), block_table.data_ptr(),
+                                                  lengths.data_ptr() if lengths is not None else None, n_groups,
+                                                  out.payload.data_ptr(), out.payload.shape[1], out.scales.data_ptr(),
+                                                  out.comp_bytes.data_ptr(), scheme, _stream())
+    check(st, "speckv_ext_compress_gather_set")
+    return out
+
+
+def decompress_scatter_set(c: CompressedKV, cset: KVCacheSet, cache_index: torch.Tensor, block_table: torch.Tensor,
+                           src_index: Optional[torch.Tensor] = None,
+                           out_elems: Optional[torch.Tensor] = None) -> KVCacheSet:
+    """decompress_scatter across a cache set: request i decodes stored block src_index[i] (block i when src_index is
+    None) into block block_table[i] of cache cache_index[i].  (cache, block) pairs must be distinct."""
+    if cset.block_elems != c.group_elems:
+        raise ValueError("cache block size differs from the stored group size")
+    cache_index, block_table = _set_groups(cset, cache_index, block_table)
+    n = block_table.numel()
+    if src_index is not None:
+        src_index = src_index.to(device=cset.device, dtype=torch.int32).contiguous()
+        if src_index.numel() != n:
+            raise ValueError("src_index and block_table differ in length")
+    elif n != c.n_groups:
+        raise ValueError("block_table must name one cache block per stored block")
+    with torch.cuda.device(cset.device):
+        st = lib().speckv_ext_decompress_scatter_set(c.payload.data_ptr(), c.payload.shape[1], c.scales.data_ptr(),
+                                                     c.comp_bytes.data_ptr(),
+                                                     src_index.data_ptr() if src_index is not None else None,
+                                                     cset.handle(), cache_index.data_ptr(), block_table.data_ptr(), n,
+                                                     out_elems.data_ptr() if out_elems is not None else None,
+                                                     c.scheme, _stream())
+    check(st, "speckv_ext_decompress_scatter_set")
+    return cset
+
+
 def translate(va: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Batched FPGACacheEngine::translate_address over an int64 tensor of (uint64) addresses."""
     if va.dtype != torch.int64 or not va.is_cuda:

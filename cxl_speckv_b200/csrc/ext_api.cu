@@ -13,6 +13,7 @@
 
 #include "../../include/speckv_ext.h"
 #include "atu.h"
+#include "cache_set.h"
 #include "codec_math.cuh"
 #include "device_ctx.h"
 #include "kv_codec.h"
@@ -543,6 +544,79 @@ speckv_status_t speckv_ext_decompress_scatter(const void* d_payload, size_t slot
     if (n_requests && !d_block_table) return SPECKV_ERR_INVAL;
     a.out = d_cache;
     a.elem_index = d_block_table;
+    a.out_elems = d_out_elems;
+    a.src_index = d_src_index;
+    return codec_run(true, a, cuda_stream);
+}
+
+// ---- KV cache sets ---------------------------------------------------------------------------------------------
+speckv_status_t speckv_ext_cache_set_create(const void* const* h_bases, size_t n_caches, size_t block_elems,
+                                            size_t block_stride_elems, speckv_dtype_t dtype, speckv_cache_set_t** out) {
+    if (!out || !h_bases || n_caches == 0 || n_caches >= (1ull << 32) || block_elems == 0 ||
+        block_elems >= (1ull << 31) || block_stride_elems < block_elems || dtype < 0 || dtype > 2)
+        return SPECKV_ERR_INVAL;
+    for (size_t c = 0; c < n_caches; ++c)
+        if (!h_bases[c]) return SPECKV_ERR_INVAL;
+    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
+    speckv_cache_set* s = new speckv_cache_set();
+    s->n_caches = (uint32_t)n_caches;
+    s->block_elems = block_elems;
+    s->block_stride = block_stride_elems;
+    s->dtype = (int)dtype;
+    uintptr_t bits = (uintptr_t)(block_stride_elems * elem_bytes(dtype));
+    std::vector<uint64_t> bases(n_caches);
+    for (size_t c = 0; c < n_caches; ++c) {
+        bases[c] = reinterpret_cast<uint64_t>(h_bases[c]);
+        bits |= reinterpret_cast<uintptr_t>(h_bases[c]);
+    }
+    s->aligned = (bits & 15) == 0;
+    cudaError_t e = cudaGetDevice(&s->device);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_bases, n_caches * sizeof(uint64_t));
+    if (e == cudaSuccess) e = cudaMemcpy(s->d_bases, bases.data(), n_caches * sizeof(uint64_t), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) {
+        speckv_ext_cache_set_destroy(s);
+        return status_of(e);
+    }
+    *out = s;
+    return SPECKV_OK;
+}
+
+void speckv_ext_cache_set_destroy(speckv_cache_set_t* set) {
+    if (!set) return;
+    if (set->d_bases) cudaFree(set->d_bases);
+    cudaGetLastError();
+    delete set;
+}
+
+speckv_status_t speckv_ext_compress_gather_set(const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                               const uint32_t* d_block_table, const uint32_t* d_group_len, size_t n_groups,
+                                               void* d_payload, size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
+                                               speckv_comp_scheme_t scheme, void* cuda_stream) {
+    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
+    if (!set || scheme == SPECKV_COMP_FP16 || !cache_set_on_current_device(*set)) return SPECKV_ERR_INVAL;
+    CodecArgs a;
+    const speckv_status_t rc = codec_args(a, set->dtype, set->block_elems, n_groups, d_payload, slot_bytes, d_scales,
+                                          d_comp_bytes, scheme, set->d_bases);
+    if (rc != SPECKV_OK) return rc;
+    if (n_groups && (!d_cache_index || !d_block_table)) return SPECKV_ERR_INVAL;
+    use_cache_set(a, *set, d_cache_index, d_block_table);
+    a.group_len = d_group_len;
+    return codec_run(false, a, cuda_stream);
+}
+
+speckv_status_t speckv_ext_decompress_scatter_set(const void* d_payload, size_t slot_bytes, const float* d_scales,
+                                                  const uint32_t* d_comp_bytes, const uint32_t* d_src_index,
+                                                  const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                                  const uint32_t* d_block_table, size_t n_requests, uint32_t* d_out_elems,
+                                                  speckv_comp_scheme_t scheme, void* cuda_stream) {
+    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
+    if (!set || scheme == SPECKV_COMP_FP16 || !cache_set_on_current_device(*set)) return SPECKV_ERR_INVAL;
+    CodecArgs a;
+    const speckv_status_t rc = codec_args(a, set->dtype, set->block_elems, n_requests, d_payload, slot_bytes, d_scales,
+                                          d_comp_bytes, scheme, set->d_bases);
+    if (rc != SPECKV_OK) return rc;
+    if (n_requests && (!d_cache_index || !d_block_table)) return SPECKV_ERR_INVAL;
+    use_cache_set(a, *set, d_cache_index, d_block_table);
     a.out_elems = d_out_elems;
     a.src_index = d_src_index;
     return codec_run(true, a, cuda_stream);

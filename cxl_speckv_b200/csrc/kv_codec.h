@@ -35,6 +35,15 @@ struct CodecArgs {
     // compress, optional (device): group g encodes only the first min(group_len[g], group_elems) elements of its
     // block (the filled prefix of a paged KV block); no packed emission with it
     const uint32_t* group_len = nullptr;
+    // optional KV cache set (speckv_ext_cache_set_create): group g's elements are block elem_index[g] of cache
+    // cache_index[g], at cache_bases[cache_index[g]] + elem_index[g] * block_stride; `in` / `out` are unused.  Always
+    // with elem_index.  An index >= n_caches addresses cache 0 (never read or written: the fetch leaves such a request
+    // with an empty payload, and the other forms take it as a caller error)
+    const uint64_t* cache_bases = nullptr;   // device: element address of each cache
+    const uint32_t* cache_index = nullptr;   // device: per group
+    uint64_t block_stride = 0;               // elements between consecutive blocks of a cache
+    uint32_t n_caches = 0;
+    bool set_unaligned = false;              // host: a base or the stride in bytes is not a multiple of 16 (generic kernels)
     size_t slot_bytes = 0;
     uint32_t group_elems = 0;
     uint32_t n_groups = 0;
@@ -47,9 +56,16 @@ struct CodecArgs {
           scheme(scheme_) {}
 
     // ---- container addressing (device).  The index arrays stay unchanged during a launch: non-coherent loads.
-    // group g's elements: block elem_index[g] of `base`, else block g (blocks of G elements)
-    template <typename T>
+    // group g's elements: block elem_index[g] of `base`, else block g (blocks of G elements); with a cache set, block
+    // elem_index[g] of cache cache_index[g].  SET = false: a kernel instantiated for calls without a set (the generic
+    // kernels have one instantiation per form, so that the set branch costs their single-cache forms nothing)
+    template <bool SET = true, typename T>
     __device__ __forceinline__ T* elem_block(T* base, uint32_t g, uint32_t G) const {
+        if (SET && cache_bases) {
+            const uint32_t c = __ldg(cache_index + g);
+            return reinterpret_cast<T*>(__ldg(cache_bases + (c < n_caches ? c : 0u))) +
+                   (size_t)__ldg(elem_index + g) * block_stride;
+        }
         return base + (size_t)(elem_index ? __ldg(elem_index + g) : g) * G;
     }
     // the stored block output group g decodes

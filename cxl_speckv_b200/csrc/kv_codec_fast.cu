@@ -1720,7 +1720,9 @@ int fast_regions(const CodecArgs& a, bool decompress) {
     const uint32_t R = a.group_elems / kRegion;
     if (R > 128 || (R & (R - 1))) return 0;
     if (R > (uint32_t)kW * 8) return 0;   // portable cluster size limit (8 CTAs)
-    const void* elems = decompress ? a.out : a.in;
+    // a cache set: the alignment of its bases and stride, recorded when it was created
+    const void* elems = a.cache_bases ? nullptr : decompress ? a.out : a.in;
+    if (a.cache_bases && a.set_unaligned) return 0;
     if ((reinterpret_cast<uintptr_t>(elems) | reinterpret_cast<uintptr_t>(a.payload)) & 15) return 0;
     if (a.slot_bytes < (size_t)R * (scheme_is_codes(a.scheme) ? kRegion : kRegionBytes)) return 0;
     if ((uint64_t)a.n_groups * R >= (1ull << 31) * (uint64_t)kW) return 0;   // grid of the codes-only decode

@@ -180,7 +180,7 @@ __device__ __forceinline__ void load_elems(const T* __restrict__ gin, uint32_t s
 // ---------------------------------------------------------------------------------
 // compress, scheme INT8_DELTA_RLE
 // ---------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool SET>
 __global__ void __launch_bounds__(kThreads)
 compress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged) {
     __shared__ __align__(16) uint16_t stage[kTile + 16];
@@ -194,7 +194,7 @@ compress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t*
     const uint32_t G = a.group_elems;
     GroupIter it(only_flagged, a.n_groups, smask);
     for (uint32_t g; it.next(g);) {
-        const T* gin = a.elem_block(static_cast<const T*>(a.in), g, G);
+        const T* gin = a.elem_block<SET>(static_cast<const T*>(a.in), g, G);
         uint8_t* gout = a.block_payload(g);   // packed emission: the slot reserved by the tuned kernel
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gin) & 15) == 0;
         const uint32_t n = a.group_length(g, G);
@@ -513,7 +513,7 @@ __device__ __forceinline__ void decode_runs_region(RunsSmem& rs, int wid, int la
 // ---------------------------------------------------------------------------------
 // decompress, scheme INT8_DELTA_RLE
 // ---------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool SET>
 __global__ void __launch_bounds__(kThreads)
 decompress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged, const DecodeScratch runs) {
     const uint32_t G = a.group_elems, n_groups = a.live_groups();
@@ -541,7 +541,7 @@ decompress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_
                 const uint32_t gi = a.stored_block(g);
                 const uint32_t npairs = min(__ldg(a.comp_bytes + gi) >> 1, R * 2048u);
                 decode_runs_region<T>(rs, wid, lane, a.block_payload(gi), npairs, __ldg(a.scales + gi), runs.prefix + (size_t)g * (R + 1),
-                                      R, o, a.elem_block(out, g, G));
+                                      R, o, a.elem_block<SET>(out, g, G));
             }
             // the last CTA to get here clears the list for the next call (every CTA has read the count by then).  Only
             // when there was a list: with n_runs == 0 both counters are zero already, and one atomic per CTA on the same
@@ -577,7 +577,7 @@ decompress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_
         npairs = min(npairs, (uint32_t)(a.slot_bytes >> 1));
         const float s = __ldg(a.scales + gi);
         const bool special = scale_is_special(s);
-        T* gout = a.elem_block(out, g, G);
+        T* gout = a.elem_block<SET>(out, g, G);
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gout) & 15) == 0;
         const bool in_vec_ok = (reinterpret_cast<uintptr_t>(gp) & 15) == 0;
 
@@ -660,7 +660,7 @@ decompress_rle_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_
 // ---------------------------------------------------------------------------------
 // scheme INT8: codes only (quantize_to_int8 / dequantize_from_int8)
 // ---------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool SET>
 __global__ void __launch_bounds__(kThreads)
 compress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged) {
     __shared__ float fbuf[kWarps];
@@ -669,7 +669,7 @@ compress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t
     const uint32_t G = a.group_elems;
     GroupIter it(only_flagged, a.n_groups, smask);
     for (uint32_t g; it.next(g);) {
-        const T* gin = a.elem_block(static_cast<const T*>(a.in), g, G);
+        const T* gin = a.elem_block<SET>(static_cast<const T*>(a.in), g, G);
         uint8_t* gout = static_cast<uint8_t*>(a.payload) + (size_t)g * a.slot_bytes;   // no packed emission with codes only
         const bool vec_ok = (reinterpret_cast<uintptr_t>(gin) & 15) == 0;
         const uint32_t n = a.group_length(g, G);
@@ -702,7 +702,7 @@ compress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t
     }
 }
 
-template <typename T>
+template <typename T, bool SET>
 __global__ void __launch_bounds__(kThreads)
 decompress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32_t* __restrict__ only_flagged) {
     __shared__ uint32_t smask[kWarps];
@@ -714,7 +714,7 @@ decompress_int8_generic_kernel(const __grid_constant__ CodecArgs a, const uint32
         const uint8_t* gp = a.block_payload(gi);
         const uint32_t n = min(min(__ldg(a.comp_bytes + gi), G), (uint32_t)a.slot_bytes);
         const float s = __ldg(a.scales + gi);
-        T* gout = a.elem_block(static_cast<T*>(a.out), g, G);
+        T* gout = a.elem_block<SET>(static_cast<T*>(a.out), g, G);
         const bool special = scale_is_special(s);
         for (uint32_t i = tid; i < n; i += kThreads)
             gout[i] = special ? narrow_special<T>(dequantize_special(__ldg(gp + i), s)) : narrow<T>(dequantize(__ldg(gp + i), s));
@@ -775,18 +775,18 @@ inline int grid_for(uint32_t n_groups, int sm_count, int per_sm) {
 
 }  // namespace
 
-template <typename T>
+template <typename T, bool SET>
 static cudaError_t launch_compress_t(const CodecArgs& a, cudaStream_t st, const uint32_t* only_flagged) {
     // as the second pass behind a tuned kernel almost nothing is flagged: a smaller grid (its launch and drain are
     // what an empty pass costs) still spreads the few flagged groups over every SM
     const int grid = grid_for(a.n_groups, current_sm_count(), only_flagged ? kSecondPassPerSm : 8);
-    if (scheme_is_rle(a.scheme)) compress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged);
-    else compress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged);
+    if (scheme_is_rle(a.scheme)) compress_rle_generic_kernel<T, SET><<<grid, kThreads, 0, st>>>(a, only_flagged);
+    else compress_int8_generic_kernel<T, SET><<<grid, kThreads, 0, st>>>(a, only_flagged);
     count_launch();
     return cudaGetLastError();
 }
 
-template <typename T>
+template <typename T, bool SET>
 static cudaError_t launch_decompress_t(const CodecArgs& a, cudaStream_t st, const uint32_t* only_flagged, const DecodeScratch* runs) {
     const int sm_count = current_sm_count();
     int grid = grid_for(a.n_groups, sm_count, only_flagged ? kSecondPassPerSm : 8);
@@ -795,8 +795,8 @@ static cudaError_t launch_decompress_t(const CodecArgs& a, cudaStream_t st, cons
         const long long cap = (long long)sm_count * 2;
         grid = (int)std::max<long long>(grid, std::min(want, cap));
     }
-    if (scheme_is_rle(a.scheme)) decompress_rle_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged, runs ? *runs : DecodeScratch{});
-    else decompress_int8_generic_kernel<T><<<grid, kThreads, 0, st>>>(a, only_flagged);
+    if (scheme_is_rle(a.scheme)) decompress_rle_generic_kernel<T, SET><<<grid, kThreads, 0, st>>>(a, only_flagged, runs ? *runs : DecodeScratch{});
+    else decompress_int8_generic_kernel<T, SET><<<grid, kThreads, 0, st>>>(a, only_flagged);
     count_launch();
     return cudaGetLastError();
 }
@@ -804,30 +804,32 @@ static cudaError_t launch_decompress_t(const CodecArgs& a, cudaStream_t st, cons
 cudaError_t launch_compress_generic(const CodecArgs& a, cudaStream_t st, const uint32_t* only_flagged) {
     if (a.n_groups == 0) return cudaSuccess;
     if (a.scheme == 0) {
-        if (a.elem_index) return cudaErrorInvalidValue;   // the raw passthrough has no gather form
+        if (a.elem_index || a.cache_bases) return cudaErrorInvalidValue;   // the raw passthrough has no gather form
         passthrough_in_kernel<<<current_sm_count() * 8, kThreads, 0, st>>>(a);
         count_launch();
         return cudaGetLastError();
     }
+    const bool set = a.cache_bases != nullptr;   // a cache set runs its own instantiations (kv_codec.h, elem_block)
     switch (a.dtype) {
-        case DT_F16: return launch_compress_t<__half>(a, st, only_flagged);
-        case DT_BF16: return launch_compress_t<__nv_bfloat16>(a, st, only_flagged);
-        default: return launch_compress_t<float>(a, st, only_flagged);
+        case DT_F16: return set ? launch_compress_t<__half, true>(a, st, only_flagged) : launch_compress_t<__half, false>(a, st, only_flagged);
+        case DT_BF16: return set ? launch_compress_t<__nv_bfloat16, true>(a, st, only_flagged) : launch_compress_t<__nv_bfloat16, false>(a, st, only_flagged);
+        default: return set ? launch_compress_t<float, true>(a, st, only_flagged) : launch_compress_t<float, false>(a, st, only_flagged);
     }
 }
 
 cudaError_t launch_decompress_generic(const CodecArgs& a, cudaStream_t st, const uint32_t* only_flagged, const DecodeScratch* runs) {
     if (a.n_groups == 0) return cudaSuccess;
     if (a.scheme == 0) {
-        if (a.elem_index) return cudaErrorInvalidValue;
+        if (a.elem_index || a.cache_bases) return cudaErrorInvalidValue;
         passthrough_out_kernel<<<grid_for(a.n_groups, current_sm_count(), 8), kThreads, 0, st>>>(a);
         count_launch();
         return cudaGetLastError();
     }
+    const bool set = a.cache_bases != nullptr;
     switch (a.dtype) {
-        case DT_F16: return launch_decompress_t<__half>(a, st, only_flagged, runs);
-        case DT_BF16: return launch_decompress_t<__nv_bfloat16>(a, st, only_flagged, runs);
-        default: return launch_decompress_t<float>(a, st, only_flagged, runs);
+        case DT_F16: return set ? launch_decompress_t<__half, true>(a, st, only_flagged, runs) : launch_decompress_t<__half, false>(a, st, only_flagged, runs);
+        case DT_BF16: return set ? launch_decompress_t<__nv_bfloat16, true>(a, st, only_flagged, runs) : launch_decompress_t<__nv_bfloat16, false>(a, st, only_flagged, runs);
+        default: return set ? launch_decompress_t<float, true>(a, st, only_flagged, runs) : launch_decompress_t<float, false>(a, st, only_flagged, runs);
     }
 }
 

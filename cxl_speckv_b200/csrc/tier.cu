@@ -19,6 +19,7 @@
 #include <vector>
 
 #include "../../include/speckv_ext.h"
+#include "cache_set.h"
 #include "device_ctx.h"
 #include "kv_codec.h"
 #include "tier_fetch.h"
@@ -435,11 +436,13 @@ void speckv_ext_tier_destroy(speckv_tier_t* tier) {
 }
 
 // d_group_len (device, optional): group i is the first min(d_group_len[i], group_elems) elements of its block
+// set (optional): group i is block d_block_table[i] of cache d_cache_index[i] of the set (d_in unused)
 static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, const uint32_t* d_block_table,
                                          const uint32_t* d_group_len, speckv_dtype_t dtype, size_t group_elems,
-                                         size_t n_groups, const uint64_t* h_block_ids, void* cuda_stream) {
+                                         size_t n_groups, const uint64_t* h_block_ids, void* cuda_stream,
+                                         const speckv_cache_set* set = nullptr, const uint32_t* d_cache_index = nullptr) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!tier || !h_block_ids || (!d_in && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0 ||
+    if (!tier || !h_block_ids || (!d_in && !set && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0 ||
         group_elems >= (1ull << 31))
         return SPECKV_ERR_INVAL;
     if (n_groups == 0) return SPECKV_OK;
@@ -506,6 +509,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         a.in = d_block_table ? d_in : (const void*)((const char*)d_in + g0 * group_elems * esz);
         a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
         a.group_len = d_group_len ? d_group_len + g0 : nullptr;   // ragged: slots + scan + pack (no packed emission)
+        if (set) use_cache_set(a, *set, d_cache_index + g0, d_block_table + g0);
         a.payload = t.d_slots[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
@@ -584,9 +588,11 @@ speckv_status_t speckv_ext_tier_offload_ragged(speckv_tier_t* tier, const void* 
 
 static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_groups,
                                          size_t group_elems, speckv_dtype_t dtype, void* d_out,
-                                         const uint32_t* d_block_table, void* cuda_stream) {
+                                         const uint32_t* d_block_table, void* cuda_stream,
+                                         const speckv_cache_set* set = nullptr, const uint32_t* d_cache_index = nullptr) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!tier || !h_block_ids || (!d_out && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0) return SPECKV_ERR_INVAL;
+    if (!tier || !h_block_ids || (!d_out && !set && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0)
+        return SPECKV_ERR_INVAL;
     if (n_groups == 0) return SPECKV_OK;
     Tier& t = tier->t;
     std::lock_guard<std::mutex> lk(t.mu);
@@ -653,6 +659,7 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
         CodecArgs a(slot, group_elems, ng, dtype, scheme);
         a.out = d_block_table ? d_out : (void*)((char*)d_out + g0 * group_elems * esz);
         a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
+        if (set) use_cache_set(a, *set, d_cache_index + g0, d_block_table + g0);
         a.payload = t.d_packed[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
@@ -691,6 +698,33 @@ speckv_status_t speckv_ext_tier_restore_paged(speckv_tier_t* tier, const uint64_
                                               const uint32_t* d_block_table, void* cuda_stream) {
     if (!d_block_table && n_blocks) return SPECKV_ERR_INVAL;
     return tier_restore_impl(tier, h_block_ids, n_blocks, group_elems, dtype, d_cache, d_block_table, cuda_stream);
+}
+
+// the set forms: geometry and dtype from the set, the rest shared with the single-cache forms
+static speckv_status_t check_set_call(const speckv_cache_set* set, const uint32_t* d_cache_index,
+                                      const uint32_t* d_block_table, size_t n) {
+    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
+    if (!set || !cache_set_on_current_device(*set) || (n && (!d_cache_index || !d_block_table))) return SPECKV_ERR_INVAL;
+    return SPECKV_OK;
+}
+
+speckv_status_t speckv_ext_tier_offload_set(speckv_tier_t* tier, const speckv_cache_set_t* set,
+                                            const uint32_t* d_cache_index, const uint32_t* d_block_table,
+                                            const uint32_t* d_group_len, size_t n_blocks, const uint64_t* h_block_ids,
+                                            void* cuda_stream) {
+    const speckv_status_t rc = check_set_call(set, d_cache_index, d_block_table, n_blocks);
+    if (rc != SPECKV_OK) return rc;
+    return tier_offload_impl(tier, nullptr, d_block_table, d_group_len, (speckv_dtype_t)set->dtype, set->block_elems,
+                             n_blocks, h_block_ids, cuda_stream, set, d_cache_index);
+}
+
+speckv_status_t speckv_ext_tier_restore_set(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_blocks,
+                                            const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                            const uint32_t* d_block_table, void* cuda_stream) {
+    const speckv_status_t rc = check_set_call(set, d_cache_index, d_block_table, n_blocks);
+    if (rc != SPECKV_OK) return rc;
+    return tier_restore_impl(tier, h_block_ids, n_blocks, set->block_elems, (speckv_dtype_t)set->dtype, nullptr,
+                             d_block_table, cuda_stream, set, d_cache_index);
 }
 
 speckv_status_t speckv_ext_tier_drop(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n) {
@@ -826,11 +860,12 @@ size_t speckv_ext_tier_fetch_workspace_bytes(size_t max_requests, size_t group_e
     return max_requests * (speckv_ext_slot_bytes(group_elems, SPECKV_COMP_INT8_DELTA_RLE) + 24) + 8;
 }
 
-speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
-                                      size_t max_requests, size_t group_elems, speckv_dtype_t dtype,
-                                      speckv_comp_scheme_t scheme, void* d_out, const uint32_t* d_block_table,
-                                      uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
-                                      size_t workspace_bytes, void* cuda_stream) {
+static speckv_status_t tier_fetch_impl(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
+                                       size_t max_requests, size_t group_elems, speckv_dtype_t dtype,
+                                       speckv_comp_scheme_t scheme, void* d_out, const uint32_t* d_block_table,
+                                       uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
+                                       size_t workspace_bytes, void* cuda_stream, const speckv_cache_set* set = nullptr,
+                                       const uint32_t* d_cache_index = nullptr) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
     if (!tier || dtype < 0 || dtype > 2 || (int)scheme < 1 || (int)scheme > 4 || group_elems == 0 ||
         group_elems >= (1ull << 31) || max_requests >= (1ull << 31))
@@ -841,7 +876,7 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess || dev != t.device) return SPECKV_ERR_INVAL;
     if (max_requests == 0) return SPECKV_OK;
-    if (!d_block_ids || !d_out || !d_workspace || (reinterpret_cast<uintptr_t>(d_workspace) & 15) ||
+    if (!d_block_ids || (!d_out && !set) || !d_workspace || (reinterpret_cast<uintptr_t>(d_workspace) & 15) ||
         workspace_bytes < speckv_ext_tier_fetch_workspace_bytes(max_requests, group_elems))
         return SPECKV_ERR_INVAL;
     const size_t n = max_requests;
@@ -854,7 +889,8 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
     float* scales = reinterpret_cast<float*>(comp + n);
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     cudaError_t e = launch_fetch_lookup(t.d_dir, d_block_ids, d_n_requests, (uint32_t)n, (uint32_t)group_elems, dtype,
-                                        (int)scheme, slot, src_off, comp, scales, d_status, st);
+                                        (int)scheme, slot, src_off, comp, scales, d_status, st, d_cache_index,
+                                        set ? set->n_caches : 0u);
     if (e != cudaSuccess) return status_of(e);
     pack_offsets_kernel<<<1, 1024, 0, st>>>(comp, (uint32_t)n, d_n_requests, offsets, total);
     count_launch();
@@ -865,6 +901,7 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
     CodecArgs a(slot, group_elems, n, dtype, (int)scheme);
     a.out = d_out;
     a.elem_index = d_block_table;
+    if (set) use_cache_set(a, *set, d_cache_index, d_block_table);
     a.payload = staging;
     a.slot_offsets = offsets;
     a.scales = scales;
@@ -872,6 +909,27 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
     a.out_elems = d_out_elems;
     a.n_groups_dev = d_n_requests;
     return status_of(launch_decompress(a, st));
+}
+
+speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
+                                      size_t max_requests, size_t group_elems, speckv_dtype_t dtype,
+                                      speckv_comp_scheme_t scheme, void* d_out, const uint32_t* d_block_table,
+                                      uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
+                                      size_t workspace_bytes, void* cuda_stream) {
+    return tier_fetch_impl(tier, d_block_ids, d_n_requests, max_requests, group_elems, dtype, scheme, d_out, d_block_table,
+                           d_out_elems, d_status, d_workspace, workspace_bytes, cuda_stream);
+}
+
+speckv_status_t speckv_ext_tier_fetch_set(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
+                                          size_t max_requests, const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                          const uint32_t* d_block_table, speckv_comp_scheme_t scheme,
+                                          uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
+                                          size_t workspace_bytes, void* cuda_stream) {
+    const speckv_status_t rc = check_set_call(set, d_cache_index, d_block_table, max_requests);
+    if (rc != SPECKV_OK) return rc;
+    return tier_fetch_impl(tier, d_block_ids, d_n_requests, max_requests, set->block_elems, (speckv_dtype_t)set->dtype,
+                           scheme, nullptr, d_block_table, d_out_elems, d_status, d_workspace, workspace_bytes,
+                           cuda_stream, set, d_cache_index);
 }
 
 }  // extern "C"

@@ -20,11 +20,13 @@ constexpr int kGatherVec = 8;                                               // 1
 constexpr uint64_t kGatherPiece = (uint64_t)kGatherThreads * kGatherVec * 16;   // 32 KiB of staging per CTA step
 constexpr int kGatherCtasPerSm = 4;
 
+// SET: request i names a block of a cache set; cache_index[i] >= n_caches is not served
+template <bool SET>
 __global__ void __launch_bounds__(kLookupThreads)
 fetch_lookup_kernel(const DeviceDir* __restrict__ dir, const uint64_t* __restrict__ ids, const uint32_t* __restrict__ n_dev,
                     uint32_t n, uint32_t group_elems, int dtype, bool rle, uint64_t max_comp_bytes,
                     uint64_t* __restrict__ src_off, uint32_t* __restrict__ comp_bytes, float* __restrict__ scales,
-                    uint8_t* __restrict__ status) {
+                    uint8_t* __restrict__ status, const uint32_t* __restrict__ cache_index, uint32_t n_caches) {
     const uint32_t i = blockIdx.x * kLookupThreads + threadIdx.x;
     const uint32_t count = n_dev ? min(*n_dev, n) : n;
     if (i >= count) return;
@@ -34,8 +36,9 @@ fetch_lookup_kernel(const DeviceDir* __restrict__ dir, const uint64_t* __restric
     uint32_t cb = 0;
     float s = 1.0f;
     bool served = false;
+    const bool in_set = !SET || cache_index[i] < n_caches;
     // the host map keeps its load under 0.7, so an empty slot ends every probe run; the bound only guards the loop
-    for (uint64_t h = dir_hash(key) & d.mask, probes = 0; probes <= d.mask; h = (h + 1) & d.mask, ++probes) {
+    for (uint64_t h = dir_hash(key) & d.mask, probes = 0; in_set && probes <= d.mask; h = (h + 1) & d.mask, ++probes) {
         const uint4* e = reinterpret_cast<const uint4*>(d.table + h);
         const uint4 lo = e[0];   // key, pool_off
         const uint4 hi = e[1];   // comp_bytes, scale, group_elems, dtype | scheme << 8 | ragged
@@ -126,10 +129,16 @@ cudaError_t launch_dir_apply(const DeviceDir* d_dir, const DirUpdate* d_upd, siz
 
 cudaError_t launch_fetch_lookup(const DeviceDir* d_dir, const uint64_t* ids, const uint32_t* n_dev, uint32_t n,
                                 uint32_t group_elems, int dtype, int scheme, size_t max_comp_bytes, uint64_t* src_off,
-                                uint32_t* comp_bytes, float* scales, uint8_t* status, cudaStream_t st) {
+                                uint32_t* comp_bytes, float* scales, uint8_t* status, cudaStream_t st,
+                                const uint32_t* cache_index, uint32_t n_caches) {
     const bool rle = scheme == 2 || scheme == 3;
-    fetch_lookup_kernel<<<(n + kLookupThreads - 1) / kLookupThreads, kLookupThreads, 0, st>>>(
-        d_dir, ids, n_dev, n, group_elems, dtype, rle, max_comp_bytes, src_off, comp_bytes, scales, status);
+    const unsigned grid = (n + kLookupThreads - 1) / kLookupThreads;
+    if (cache_index)
+        fetch_lookup_kernel<true><<<grid, kLookupThreads, 0, st>>>(d_dir, ids, n_dev, n, group_elems, dtype, rle, max_comp_bytes,
+                                                                    src_off, comp_bytes, scales, status, cache_index, n_caches);
+    else
+        fetch_lookup_kernel<false><<<grid, kLookupThreads, 0, st>>>(d_dir, ids, n_dev, n, group_elems, dtype, rle, max_comp_bytes,
+                                                                     src_off, comp_bytes, scales, status, nullptr, 0u);
     count_launch();
     return cudaGetLastError();
 }

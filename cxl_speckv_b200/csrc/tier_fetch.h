@@ -56,11 +56,13 @@ cudaError_t launch_dir_apply(const DeviceDir* d_dir, const DirUpdate* d_upd, siz
 // Fetch pipeline on the device.  Request i < min(*n_dev, n) (all n when n_dev is null) names block ids[i].
 //   lookup: probe the directory, check the block fits (group_elems, dtype, scheme family, not raw), write the pool
 //           offset, payload size and scale of a served request, size 0 and scale 1 of an unserved one, status[i]
+//           (with cache_index: also unserved when cache_index[i] >= n_caches, a cache set's request past the set)
 //   gather: copy the served payloads out of the pinned pool into `staging`, back to back at offsets[i]
 // Between the two the caller scans the sizes (pack_offsets_kernel, tier.cu) into offsets / *total.
 cudaError_t launch_fetch_lookup(const DeviceDir* d_dir, const uint64_t* ids, const uint32_t* n_dev, uint32_t n,
                                 uint32_t group_elems, int dtype, int scheme, size_t max_comp_bytes, uint64_t* src_off,
-                                uint32_t* comp_bytes, float* scales, uint8_t* status, cudaStream_t st);
+                                uint32_t* comp_bytes, float* scales, uint8_t* status, cudaStream_t st,
+                                const uint32_t* cache_index = nullptr, uint32_t n_caches = 0);
 cudaError_t launch_fetch_gather(const DeviceDir* d_dir, const uint64_t* src_off, const uint64_t* offsets,
                                 const uint32_t* n_dev, uint32_t n, const uint64_t* total, uint8_t* staging,
                                 int sm_count, cudaStream_t st);

@@ -10,7 +10,7 @@ import torch
 
 from . import _lib
 from ._lib import COMP_INT8_DELTA_RLE, check, lib
-from .codec import _DTYPES, _stream
+from .codec import _DTYPES, KVCacheSet, _set_groups, _stream
 
 
 class HostTier:
@@ -98,6 +98,74 @@ class HostTier:
                                                       _DTYPES[cache.dtype], cache.data_ptr(), table.data_ptr(), _stream()),
                   "speckv_ext_tier_restore_paged")
         return cache
+
+    def offload_set(self, cset: KVCacheSet, cache_index: torch.Tensor, block_table: torch.Tensor, block_ids: np.ndarray,
+                    lengths: Optional[torch.Tensor] = None) -> None:
+        """offload_blocks / offload_ragged across a cache set in one call: block block_table[i] of cache cache_index[i]
+        (e.g. from cset.groups(table)) is stored under block_ids[i], from its first lengths[i] elements when lengths
+        (CUDA int32, one per block) is given.  Stored blocks are the records offload_blocks makes: restore_blocks and
+        fetch find them too."""
+        cache_index, block_table = _set_groups(cset, cache_index, block_table)
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
+        if ids.size != block_table.numel():
+            raise ValueError("block_ids must hold one id per block")
+        if lengths is not None:
+            lengths = lengths.to(device=cset.device, dtype=torch.int32).contiguous()
+            if lengths.numel() != ids.size:
+                raise ValueError("lengths must hold one entry per block")
+            if bool((lengths < 0).any()):   # the offload synchronises anyway; a negative length would store the whole block
+                raise ValueError("offload_set: negative length")
+        with torch.cuda.device(cset.device):
+            check(lib().speckv_ext_tier_offload_set(self._h, cset.handle(), cache_index.data_ptr(), block_table.data_ptr(),
+                                                    lengths.data_ptr() if lengths is not None else None, ids.size,
+                                                    ids.ctypes.data, _stream()), "speckv_ext_tier_offload_set")
+
+    def restore_set(self, block_ids: np.ndarray, cset: KVCacheSet, cache_index: torch.Tensor,
+                    block_table: torch.Tensor) -> KVCacheSet:
+        """restore_blocks across a cache set: stored block block_ids[i] is decompressed into block block_table[i] of
+        cache cache_index[i].  (cache, block) pairs must be distinct."""
+        cache_index, block_table = _set_groups(cset, cache_index, block_table)
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
+        if ids.size != block_table.numel():
+            raise ValueError("block_ids must hold one id per block")
+        with torch.cuda.device(cset.device):
+            check(lib().speckv_ext_tier_restore_set(self._h, ids.ctypes.data, ids.size, cset.handle(),
+                                                    cache_index.data_ptr(), block_table.data_ptr(), _stream()),
+                  "speckv_ext_tier_restore_set")
+        return cset
+
+    def fetch_set(self, block_ids: torch.Tensor, cset: KVCacheSet, cache_index: torch.Tensor, block_table: torch.Tensor,
+                  scheme: int = COMP_INT8_DELTA_RLE, count: Optional[torch.Tensor] = None,
+                  out_elems: Optional[torch.Tensor] = None, status: Optional[torch.Tensor] = None):
+        """fetch across a cache set: request i < count[0] (all of block_ids without a count) decodes stored block
+        block_ids[i] into block block_table[i] of cache cache_index[i].  -> (out_elems int32 [n], status uint8 [n]);
+        a request is unserved (status 0, its block untouched) as in fetch(), and also when cache_index[i] >= len(cset).
+        No host synchronisation: a warm call can be captured into a CUDA graph (the workspace is shared with fetch()
+        calls of the same shape)."""
+        if not block_ids.is_cuda or block_ids.dtype not in (torch.int64, torch.uint64) or not block_ids.is_contiguous():
+            raise TypeError("block_ids must be a contiguous CUDA int64 tensor")
+        dev = block_ids.device
+        if dev != cset.device:
+            raise ValueError("block_ids must be on the device of the set")
+        n = block_ids.numel()
+        for name, t in (("cache_index", cache_index), ("block_table", block_table)):
+            if not t.is_cuda or t.dtype != torch.int32 or t.numel() < n or not t.is_contiguous() or t.device != dev:
+                raise TypeError(f"{name} must be a contiguous CUDA int32 tensor with one entry per request")
+        if count is not None and (not count.is_cuda or count.dtype != torch.int32 or count.device != dev):
+            raise TypeError("count must be a CUDA int32 tensor on the device of block_ids")
+        if out_elems is None:
+            out_elems = torch.zeros(n, dtype=torch.int32, device=dev)
+        if status is None:
+            status = torch.zeros(n, dtype=torch.uint8, device=dev)
+        assert out_elems.numel() >= n and status.numel() >= n and out_elems.is_cuda and status.is_cuda
+        ws = self._workspace(n, cset.block_elems, dev)
+        with torch.cuda.device(dev):
+            check(lib().speckv_ext_tier_fetch_set(self._h, block_ids.data_ptr(),
+                                                  count.data_ptr() if count is not None else None, n, cset.handle(),
+                                                  cache_index.data_ptr(), block_table.data_ptr(), int(scheme),
+                                                  out_elems.data_ptr(), status.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                  _stream()), "speckv_ext_tier_fetch_set")
+        return out_elems, status
 
     def drop(self, block_ids: np.ndarray) -> None:
         ids = np.ascontiguousarray(block_ids, dtype=np.uint64)

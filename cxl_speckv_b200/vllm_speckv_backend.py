@@ -10,6 +10,8 @@ token history to speckv_prefetch.
 import ctypes
 from typing import Any, Dict, List, Optional
 
+import numpy as np
+
 try:  # the reference imports it relatively (:5); its tests import it top-level
     from .speckv_ctypes import SpeckvLib
 except ImportError:  # pragma: no cover
@@ -31,6 +33,7 @@ class CxlSpeckvKVAllocator:
         self._pool = None      # CUDA tensor backing the region (bind_pool)
         self._tier = None      # keeps the HostTier alive as long as the binding refers to it
         self._policy = None    # TierPolicy (attach_policy)
+        self._kv_set = None    # KVCacheSet of the registered per-layer caches (register_kv_caches)
         lib = self._speckv.lib
         if hasattr(lib, "speckv_ext_bind_pool"):   # additive entry points of the B200 library, declared once
             lib.speckv_ext_bind_pool.argtypes = [ctypes.c_uint64, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
@@ -138,6 +141,78 @@ class CxlSpeckvKVAllocator:
         """Bring stored blocks back into the cache blocks `block_table` (decompressed in place)."""
         ids = block_table.cpu().numpy().astype("uint64") if block_ids is None else block_ids
         tier.restore_blocks(ids, kv_cache, block_table)
+
+    # ---- additive: whole requests across all layers (one KV cache set) ----
+    def register_kv_caches(self, kv_caches):
+        """Register the model's per-layer KV caches once (a list, or vLLM's layer name -> tensor dict, in layer
+        order).  Each tensor is [2, num_blocks, ...] (FlashAttention backend: K = kv[0], V = kv[1]) or
+        [num_blocks, 2, ...] (FlashInfer backend: K = kv[:, 0], V = kv[:, 1]); a tensor whose first two dimensions are
+        both 2 is taken as the first.  Cache 2 * layer is the layer's K, cache 2 * layer + 1 its V.  Returns the
+        KVCacheSet that offload_request / restore_request move blocks through."""
+        from .codec import KVCacheSet
+        tensors = list(kv_caches.values()) if isinstance(kv_caches, dict) else list(kv_caches)
+        views = []
+        for kv in tensors:
+            if kv.dim() >= 3 and kv.shape[0] == 2:
+                views += [kv[0], kv[1]]
+            elif kv.dim() >= 3 and kv.shape[1] == 2:
+                views += [kv[:, 0], kv[:, 1]]
+            else:
+                raise ValueError(f"register_kv_caches: {tuple(kv.shape)} is neither [2, num_blocks, ...] nor "
+                                 "[num_blocks, 2, ...]")
+        if self._kv_set is not None:
+            self._kv_set.close()
+        self._kv_set = KVCacheSet(views)
+        return self._kv_set
+
+    def request_block_ids(self, block_table):
+        """The default ids of a request's blocks: (cache c, block b) -> (c << 40) | b, a uint64 [n_caches, n_blocks]
+        array.  Block numbers are below 2^32 (the tables are int32), so the cache index in bits 40 and up never meets
+        them; cache 0's ids are the block numbers themselves, the ids offload_kv_blocks gives by default."""
+        b = np.asarray(block_table.cpu() if hasattr(block_table, "cpu") else block_table).reshape(-1).astype(np.uint64)
+        c = np.arange(len(self._registered()), dtype=np.uint64)
+        return (c[:, None] << np.uint64(40)) | b[None, :]
+
+    def offload_request(self, block_table, tier, block_ids=None, num_tokens=None):
+        """Compress one request's blocks `block_table` (CUDA int32, the request's block numbers) of every registered
+        cache out to the host tier in one call, cache-major.  block_ids: uint64 [n_caches, n_blocks] (default
+        request_block_ids).  num_tokens (optional, one entry per block): the filled tokens of each block, as in
+        offload_kv_blocks, applied to every cache."""
+        import torch
+        cset = self._registered()
+        table = torch.as_tensor(block_table).to(device=cset.device, dtype=torch.int32).reshape(-1)
+        ids = self._request_ids(cset, table, block_ids)
+        cache_index, blocks = cset.groups(table)
+        lengths = None
+        if num_tokens is not None:
+            token_elems = cset.caches[0][0, 0].numel()   # kv_heads x head_dim: one token of the block
+            lengths = torch.as_tensor(num_tokens, device=cset.device).to(torch.int64).reshape(-1) * token_elems
+            if lengths.numel() != table.numel():
+                raise ValueError("num_tokens must hold one entry per block")
+            lengths = lengths.clamp_(0, cset.block_elems).to(torch.int32).repeat(len(cset))
+        tier.offload_set(cset, cache_index, blocks, ids, lengths=lengths)
+
+    def restore_request(self, block_table, tier, block_ids=None):
+        """Bring one request's blocks of every registered cache back from the host tier in one call."""
+        import torch
+        cset = self._registered()
+        table = torch.as_tensor(block_table).to(device=cset.device, dtype=torch.int32).reshape(-1)
+        ids = self._request_ids(cset, table, block_ids)
+        cache_index, blocks = cset.groups(table)
+        tier.restore_set(ids, cset, cache_index, blocks)
+
+    def _registered(self):
+        if self._kv_set is None:
+            raise RuntimeError("no KV caches registered (register_kv_caches)")
+        return self._kv_set
+
+    def _request_ids(self, cset, table, block_ids):
+        if block_ids is None:
+            return self.request_block_ids(table).reshape(-1)
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
+        if ids.shape != (len(cset), table.numel()):
+            raise ValueError(f"block_ids must be [{len(cset)}, {table.numel()}] (caches x blocks)")
+        return ids.reshape(-1)
 
     # ---- additive: residency policy driving the data path (SURVEY.md section 8f row 2) ----
     def attach_policy(self, policy):

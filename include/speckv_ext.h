@@ -336,6 +336,66 @@ SPECKV_API speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint
                                                  uint8_t* d_status, void* d_workspace, size_t workspace_bytes,
                                                  void* cuda_stream);
 
+/* ---- KV cache sets: one call for a request's blocks across all layers ----------------------------------------
+ * A KV cache set is the list of a model's paged KV caches (one per layer and K|V), all with the same dtype, block
+ * size and block stride.  It is registered once; the calls below then name each group by a (cache index, block
+ * number) pair held in two DEVICE arrays: group i is block d_block_table[i] of cache d_cache_index[i], whose
+ * elements start at h_bases[d_cache_index[i]] + d_block_table[i] * block_stride_elems.  The stride makes both
+ * usual vLLM layouts addressable: [2, num_blocks, ...] per layer (K = kv[0], V = kv[1], stride = block_elems) and
+ * [num_blocks, 2, ...] (K = kv[:, 0], V = kv[:, 1], stride = 2 * block_elems).
+ *
+ * _create validates its arguments (n_caches >= 1, no NULL base, block_elems >= 1, block_stride_elems >=
+ * block_elems, dtype 0-2) before it looks for a device, uploads the bases to device memory the set owns (on the
+ * current device, which every call through the set must run on) and records whether every base and the stride in
+ * bytes are multiples of 16.  Only then do the tuned kernels run; an unaligned set takes the generic kernels and
+ * gives the same bits.  The set is immutable: register a new one when the caches move.  Destroying a set while
+ * calls that use it are in flight (in a stream, or in a graph that will be replayed) is a caller error, as for the
+ * fetch workspace.
+ *
+ * Each form takes the argument checks and status codes of its single-cache counterpart, with the geometry and
+ * dtype of the set.  A cache index >= n_caches is a caller error (the fetch reports it as unserved instead).
+ * (cache, block) pairs must be distinct within a scatter, a restore and a fetch call.  Schemes 1-4.
+ *
+ * Stored blocks are the same records as those of the single-cache forms: a block offloaded through a set can be
+ * restored or fetched through _restore_paged / _fetch and the other way round.  An offload stores each chunk of
+ * ~128 MiB of payload as one contiguous pool extent, so a restore of the same ids in the same order (for a request:
+ * cache-major, all blocks of cache 0, then of cache 1, ...) moves each chunk with one or a few copies. */
+typedef struct speckv_cache_set speckv_cache_set_t;
+SPECKV_API speckv_status_t speckv_ext_cache_set_create(const void* const* h_bases, size_t n_caches, size_t block_elems,
+                                                       size_t block_stride_elems, speckv_dtype_t dtype,
+                                                       speckv_cache_set_t** out);
+SPECKV_API void speckv_ext_cache_set_destroy(speckv_cache_set_t* set);
+/* speckv_ext_compress_gather / _compress_ragged over a set (d_group_len optional: NULL stores whole blocks) */
+SPECKV_API speckv_status_t speckv_ext_compress_gather_set(const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                                          const uint32_t* d_block_table, const uint32_t* d_group_len,
+                                                          size_t n_groups, void* d_payload, size_t slot_bytes,
+                                                          float* d_scales, uint32_t* d_comp_bytes,
+                                                          speckv_comp_scheme_t scheme, void* cuda_stream);
+/* speckv_ext_decompress_scatter over a set */
+SPECKV_API speckv_status_t speckv_ext_decompress_scatter_set(const void* d_payload, size_t slot_bytes,
+                                                             const float* d_scales, const uint32_t* d_comp_bytes,
+                                                             const uint32_t* d_src_index, const speckv_cache_set_t* set,
+                                                             const uint32_t* d_cache_index, const uint32_t* d_block_table,
+                                                             size_t n_requests, uint32_t* d_out_elems,
+                                                             speckv_comp_scheme_t scheme, void* cuda_stream);
+/* speckv_ext_tier_offload_paged / _offload_ragged (d_group_len non-NULL) and _restore_paged over a set */
+SPECKV_API speckv_status_t speckv_ext_tier_offload_set(speckv_tier_t* tier, const speckv_cache_set_t* set,
+                                                       const uint32_t* d_cache_index, const uint32_t* d_block_table,
+                                                       const uint32_t* d_group_len, size_t n_blocks,
+                                                       const uint64_t* h_block_ids, void* cuda_stream);
+SPECKV_API speckv_status_t speckv_ext_tier_restore_set(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_blocks,
+                                                       const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                                       const uint32_t* d_block_table, void* cuda_stream);
+/* speckv_ext_tier_fetch over a set: the same workspace (speckv_ext_tier_fetch_workspace_bytes with the set's
+ * block_elems) and ordering rules.  A request whose d_cache_index[i] >= n_caches is also unserved (status 0,
+ * nothing written).  No host synchronisation; capturable into a CUDA graph. */
+SPECKV_API speckv_status_t speckv_ext_tier_fetch_set(speckv_tier_t* tier, const uint64_t* d_block_ids,
+                                                     const uint32_t* d_n_requests, size_t max_requests,
+                                                     const speckv_cache_set_t* set, const uint32_t* d_cache_index,
+                                                     const uint32_t* d_block_table, speckv_comp_scheme_t scheme,
+                                                     uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
+                                                     size_t workspace_bytes, void* cuda_stream);
+
 /* ---- descriptor-level interface (what the reference's ioctl client speaks) ------------------ */
 /* One transfer descriptor, identical to struct speckv_ioctl_dma_desc (driver/uapi/speckv_ioctl.h:
  * 10-15) / SpeckvDmaDesc (host/include/speckv_driver.hpp:8-13): fpga_addr names the first 4 KiB
