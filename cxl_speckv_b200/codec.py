@@ -38,6 +38,34 @@ class CompressedKV:
         return self.scales.numel()
 
 
+def _compressed(n_groups: int, group_elems: int, dtype: torch.dtype, scheme: int, device) -> CompressedKV:
+    """An empty container for n_groups groups (one slot of the scheme's worst case each)."""
+    return CompressedKV(torch.empty((n_groups, slot_bytes(group_elems, scheme)), dtype=torch.uint8, device=device),
+                        torch.empty(n_groups, dtype=torch.float32, device=device),
+                        torch.empty(n_groups, dtype=torch.int32, device=device), group_elems, dtype, scheme)
+
+
+def _i32(t: torch.Tensor, device) -> torch.Tensor:
+    """An index tensor as the C entry points take it: contiguous int32 on `device`."""
+    return t.to(device=device, dtype=torch.int32).contiguous()
+
+
+def _lengths(lengths: torch.Tensor, device, n=None, convert=False, check_negative=False) -> torch.Tensor:
+    """The lengths of a ragged call as contiguous int32 on `device`, n of them when n is given (ValueError otherwise).
+    `convert` converts any integer tensor; without it they must be an int32 tensor on `device` already (TypeError).
+    `check_negative` reads them on the host and refuses a negative one: as unsigned, it would store the whole block."""
+    if convert:
+        lengths = lengths.to(device=device, dtype=torch.int32)
+    elif not lengths.is_cuda or lengths.dtype != torch.int32 or lengths.device != device:
+        raise TypeError(f"lengths must be an int32 tensor on {device}")
+    lengths = lengths.contiguous()
+    if n is not None and lengths.numel() != n:
+        raise ValueError(f"lengths must hold one entry per group ({n})")
+    if check_negative and bool((lengths < 0).any()):
+        raise ValueError("negative length")
+    return lengths
+
+
 def compress(x: torch.Tensor, group_elems: int, scheme: int = COMP_INT8_DELTA_RLE,
              out: Optional[CompressedKV] = None) -> CompressedKV:
     """Compress x (flat view, contiguous) as consecutive groups of group_elems elements."""
@@ -50,12 +78,8 @@ def compress(x: torch.Tensor, group_elems: int, scheme: int = COMP_INT8_DELTA_RL
     if group_elems <= 0 or n % group_elems:
         raise ValueError("numel must be a multiple of group_elems")
     n_groups = n // group_elems
-    sb = slot_bytes(group_elems, scheme)
     if out is None:
-        out = CompressedKV(torch.empty((n_groups, sb), dtype=torch.uint8, device=x.device),
-                           torch.empty(n_groups, dtype=torch.float32, device=x.device),
-                           torch.empty(n_groups, dtype=torch.int32, device=x.device),
-                           group_elems, x.dtype, scheme)
+        out = _compressed(n_groups, group_elems, x.dtype, scheme, x.device)
     with torch.cuda.device(x.device):
         st = lib().speckv_ext_compress(x.data_ptr(), _DTYPES[x.dtype], group_elems, n_groups,
                                        out.payload.data_ptr(), out.payload.shape[1], out.scales.data_ptr(),
@@ -125,14 +149,10 @@ def compress_gather(cache: torch.Tensor, block_table: torch.Tensor, scheme: int 
     if not cache.is_cuda or cache.dtype not in _DTYPES or not cache.is_contiguous():
         raise ValueError("compress_gather() takes a contiguous CUDA fp16/bf16/fp32 cache tensor")
     group_elems = cache[0].numel()
-    block_table = block_table.to(device=cache.device, dtype=torch.int32).contiguous()
+    block_table = _i32(block_table, cache.device)
     n_groups = block_table.numel()
-    sb = slot_bytes(group_elems, scheme)
     if out is None:
-        out = CompressedKV(torch.empty((n_groups, sb), dtype=torch.uint8, device=cache.device),
-                           torch.empty(n_groups, dtype=torch.float32, device=cache.device),
-                           torch.empty(n_groups, dtype=torch.int32, device=cache.device),
-                           group_elems, cache.dtype, scheme)
+        out = _compressed(n_groups, group_elems, cache.dtype, scheme, cache.device)
     with torch.cuda.device(cache.device):
         st = lib().speckv_ext_compress_gather(cache.data_ptr(), block_table.data_ptr(), _DTYPES[cache.dtype],
                                               group_elems, n_groups, out.payload.data_ptr(), out.payload.shape[1],
@@ -155,22 +175,12 @@ def compress_ragged(x: torch.Tensor, group_elems: int, lengths: torch.Tensor,
         raise ValueError("compress_ragged() takes a contiguous CUDA fp16/bf16/fp32 tensor")
     if group_elems <= 0 or x.numel() % group_elems:
         raise ValueError("numel must be a multiple of group_elems")
-    if not lengths.is_cuda or lengths.dtype != torch.int32 or lengths.device != x.device:
-        raise TypeError("lengths must be an int32 tensor on the device of x")
-    lengths = lengths.contiguous()
+    n_groups = block_table.numel() if block_table is not None else x.numel() // group_elems
+    lengths = _lengths(lengths, x.device, n_groups)
     if block_table is not None:
-        block_table = block_table.to(device=x.device, dtype=torch.int32).contiguous()
-        if block_table.numel() != lengths.numel():
-            raise ValueError("block_table and lengths differ in length")
-    elif lengths.numel() != x.numel() // group_elems:
-        raise ValueError("lengths must hold one entry per block of x")
-    n_groups = lengths.numel()
-    sb = slot_bytes(group_elems, scheme)
+        block_table = _i32(block_table, x.device)
     if out is None:
-        out = CompressedKV(torch.empty((n_groups, sb), dtype=torch.uint8, device=x.device),
-                           torch.empty(n_groups, dtype=torch.float32, device=x.device),
-                           torch.empty(n_groups, dtype=torch.int32, device=x.device),
-                           group_elems, x.dtype, scheme)
+        out = _compressed(n_groups, group_elems, x.dtype, scheme, x.device)
     with torch.cuda.device(x.device):
         st = lib().speckv_ext_compress_ragged(x.data_ptr(), block_table.data_ptr() if block_table is not None else None,
                                               lengths.data_ptr(), _DTYPES[x.dtype], group_elems, n_groups,
@@ -189,10 +199,10 @@ def decompress_scatter(c: CompressedKV, cache: torch.Tensor, block_table: torch.
         raise ValueError("decompress_scatter() takes a contiguous CUDA fp16/bf16/fp32 cache tensor")
     if cache[0].numel() != c.group_elems:
         raise ValueError("cache block size differs from the stored group size")
-    block_table = block_table.to(device=cache.device, dtype=torch.int32).contiguous()
+    block_table = _i32(block_table, cache.device)
     n = block_table.numel()
     if src_index is not None:
-        src_index = src_index.to(device=cache.device, dtype=torch.int32).contiguous()
+        src_index = _i32(src_index, cache.device)
         if src_index.numel() != n:
             raise ValueError("src_index and block_table differ in length")
     elif n != c.n_groups:
@@ -284,9 +294,7 @@ def _set_groups(cset: KVCacheSet, cache_index: torch.Tensor, block_table: torch.
     """Checked (cache_index, block_table) of a set call: contiguous int32 on the set's device, equal lengths."""
     if not isinstance(cset, KVCacheSet):
         raise TypeError("expected a KVCacheSet")
-    dev = cset.device
-    cache_index = cache_index.to(device=dev, dtype=torch.int32).contiguous()
-    block_table = block_table.to(device=dev, dtype=torch.int32).contiguous()
+    cache_index, block_table = _i32(cache_index, cset.device), _i32(block_table, cset.device)
     if cache_index.numel() != block_table.numel():
         raise ValueError("cache_index and block_table differ in length")
     return cache_index, block_table
@@ -301,19 +309,10 @@ def compress_gather_set(cset: KVCacheSet, cache_index: torch.Tensor, block_table
     cache_index, block_table = _set_groups(cset, cache_index, block_table)
     n_groups = block_table.numel()
     if lengths is not None:
-        if not lengths.is_cuda or lengths.dtype != torch.int32 or lengths.device != cset.device:
-            raise TypeError("lengths must be an int32 tensor on the device of the set")
-        lengths = lengths.contiguous()
-        if lengths.numel() != n_groups:
-            raise ValueError("lengths must hold one entry per group")
-    dev = cset.device
-    sb = slot_bytes(cset.block_elems, scheme)
+        lengths = _lengths(lengths, cset.device, n_groups)
     if out is None:
-        out = CompressedKV(torch.empty((n_groups, sb), dtype=torch.uint8, device=dev),
-                           torch.empty(n_groups, dtype=torch.float32, device=dev),
-                           torch.empty(n_groups, dtype=torch.int32, device=dev),
-                           cset.block_elems, cset.dtype, scheme)
-    with torch.cuda.device(dev):
+        out = _compressed(n_groups, cset.block_elems, cset.dtype, scheme, cset.device)
+    with torch.cuda.device(cset.device):
         st = lib().speckv_ext_compress_gather_set(cset.handle(), cache_index.data_ptr(), block_table.data_ptr(),
                                                   lengths.data_ptr() if lengths is not None else None, n_groups,
                                                   out.payload.data_ptr(), out.payload.shape[1], out.scales.data_ptr(),
@@ -332,7 +331,7 @@ def decompress_scatter_set(c: CompressedKV, cset: KVCacheSet, cache_index: torch
     cache_index, block_table = _set_groups(cset, cache_index, block_table)
     n = block_table.numel()
     if src_index is not None:
-        src_index = src_index.to(device=cset.device, dtype=torch.int32).contiguous()
+        src_index = _i32(src_index, cset.device)
         if src_index.numel() != n:
             raise ValueError("src_index and block_table differ in length")
     elif n != c.n_groups:

@@ -422,18 +422,19 @@ size_t speckv_ext_slot_bytes(size_t group_elems, speckv_comp_scheme_t scheme) {
 
 namespace speckv {
 // validation shared by every codec call + the fields every call fills the same way
-static speckv_status_t codec_args(CodecArgs& a, int dtype, size_t group_elems, size_t n_groups, const void* d_payload,
-                                  size_t slot_bytes, const float* d_scales, const uint32_t* d_comp_bytes, int scheme,
-                                  const void* d_elems) {
+static speckv_status_t codec_args(CodecArgs& a, bool decompress, const KvBlocks& b, int dtype, size_t group_elems,
+                                  size_t n_groups, const void* d_payload, size_t slot_bytes, const float* d_scales,
+                                  const uint32_t* d_comp_bytes, int scheme) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
     if (!valid_common(dtype, group_elems, n_groups, slot_bytes, scheme)) return SPECKV_ERR_INVAL;
     if (n_groups == 0) return SPECKV_OK;
-    if (!d_payload || !d_scales || !d_comp_bytes || (!d_elems && group_elems)) return SPECKV_ERR_INVAL;
+    if (!d_payload || !d_scales || !d_comp_bytes || (!b.base && !b.set && group_elems)) return SPECKV_ERR_INVAL;
     if (reinterpret_cast<uintptr_t>(d_payload) & 15) return SPECKV_ERR_INVAL;
     a = CodecArgs(slot_bytes, group_elems, n_groups, dtype, scheme);
     a.payload = const_cast<void*>(d_payload);
     a.scales = const_cast<float*>(d_scales);
     a.comp_bytes = const_cast<uint32_t*>(d_comp_bytes);
+    b.bind(a, decompress, 0, elem_bytes(dtype));
     return SPECKV_OK;
 }
 static speckv_status_t codec_run(bool decompress, const CodecArgs& a, void* cuda_stream) {
@@ -447,6 +448,35 @@ static speckv_status_t codec_run(bool decompress, const CodecArgs& a, void* cuda
     }
     return status_of(e);
 }
+
+// every compress entry point: group i of the blocks b into slot i
+static speckv_status_t compress_blocks(const KvBlocks& b, int dtype, size_t group_elems, size_t n_groups,
+                                       void* d_payload, size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
+                                       int scheme, void* cuda_stream) {
+    CodecArgs a;
+    const speckv_status_t rc = codec_args(a, false, b, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales,
+                                          d_comp_bytes, scheme);
+    return rc != SPECKV_OK ? rc : codec_run(false, a, cuda_stream);
+}
+
+// every decompress entry point: request i decodes stored block d_src_index[i] (block i without it) into group i of
+// the blocks b; with d_n_requests (device), only the first *d_n_requests requests are served
+static speckv_status_t decompress_blocks(const void* d_payload, size_t slot_bytes, const float* d_scales,
+                                         const uint32_t* d_comp_bytes, const uint32_t* d_src_index,
+                                         const uint32_t* d_n_requests, size_t n_requests, const KvBlocks& b, int dtype,
+                                         size_t group_elems, uint32_t* d_out_elems, int scheme, void* cuda_stream) {
+    CodecArgs a;
+    const speckv_status_t rc = codec_args(a, true, b, dtype, group_elems, n_requests, d_payload, slot_bytes, d_scales,
+                                          d_comp_bytes, scheme);
+    if (rc != SPECKV_OK) return rc;
+    a.out_elems = d_out_elems;
+    a.src_index = d_src_index;
+    a.n_groups_dev = d_n_requests;
+    return codec_run(true, a, cuda_stream);
+}
+
+// a rejected argument of an entry point that reports a missing device first (SPECKV_ERR_DRIVER)
+static speckv_status_t invalid_argument() { return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL; }
 }  // namespace speckv
 
 extern "C" {
@@ -454,37 +484,25 @@ extern "C" {
 speckv_status_t speckv_ext_compress(const void* d_in, speckv_dtype_t dtype, size_t group_elems, size_t n_groups,
                                     void* d_payload, size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
                                     speckv_comp_scheme_t scheme, void* cuda_stream) {
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_in);
-    if (rc != SPECKV_OK) return rc;
-    a.in = d_in;
-    return codec_run(false, a, cuda_stream);
+    return compress_blocks(KvBlocks{d_in}, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes,
+                           scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_decompress(const void* d_payload, size_t slot_bytes, const float* d_scales,
                                       const uint32_t* d_comp_bytes, size_t group_elems, size_t n_groups,
                                       speckv_dtype_t dtype, void* d_out, uint32_t* d_out_elems,
                                       speckv_comp_scheme_t scheme, void* cuda_stream) {
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_out);
-    if (rc != SPECKV_OK) return rc;
-    a.out = d_out;
-    a.out_elems = d_out_elems;
-    return codec_run(true, a, cuda_stream);
+    return decompress_blocks(d_payload, slot_bytes, d_scales, d_comp_bytes, nullptr, nullptr, n_groups, KvBlocks{d_out},
+                             dtype, group_elems, d_out_elems, scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_decompress_indexed(const void* d_payload, size_t slot_bytes, const float* d_scales,
                                               const uint32_t* d_comp_bytes, const uint32_t* d_block_index,
                                               size_t n_requests, size_t group_elems, speckv_dtype_t dtype, void* d_out,
                                               uint32_t* d_out_elems, speckv_comp_scheme_t scheme, void* cuda_stream) {
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_requests, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_out);
-    if (rc != SPECKV_OK) return rc;
-    if (n_requests && !d_block_index) return SPECKV_ERR_INVAL;
-    a.out = d_out;
-    a.out_elems = d_out_elems;
-    a.src_index = d_block_index;
-    return codec_run(true, a, cuda_stream);
+    if (n_requests && !d_block_index) return invalid_argument();
+    return decompress_blocks(d_payload, slot_bytes, d_scales, d_comp_bytes, d_block_index, nullptr, n_requests,
+                             KvBlocks{d_out}, dtype, group_elems, d_out_elems, scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_decompress_routed(const void* d_payload, size_t slot_bytes, const float* d_scales,
@@ -492,44 +510,28 @@ speckv_status_t speckv_ext_decompress_routed(const void* d_payload, size_t slot_
                                              const uint32_t* d_n_requests, size_t max_requests, size_t group_elems,
                                              speckv_dtype_t dtype, void* d_out, uint32_t* d_out_elems,
                                              speckv_comp_scheme_t scheme, void* cuda_stream) {
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, max_requests, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_out);
-    if (rc != SPECKV_OK) return rc;
-    if (max_requests && (!d_block_index || !d_n_requests)) return SPECKV_ERR_INVAL;
-    a.out = d_out;
-    a.out_elems = d_out_elems;
-    a.src_index = d_block_index;
-    a.n_groups_dev = d_n_requests;
-    return codec_run(true, a, cuda_stream);
+    if (max_requests && (!d_block_index || !d_n_requests)) return invalid_argument();
+    return decompress_blocks(d_payload, slot_bytes, d_scales, d_comp_bytes, d_block_index, d_n_requests, max_requests,
+                             KvBlocks{d_out}, dtype, group_elems, d_out_elems, scheme, cuda_stream);
 }
 
+// the paged and ragged forms have no raw passthrough (scheme 0)
 speckv_status_t speckv_ext_compress_gather(const void* d_cache, const uint32_t* d_block_table, speckv_dtype_t dtype,
                                            size_t group_elems, size_t n_groups, void* d_payload, size_t slot_bytes,
                                            float* d_scales, uint32_t* d_comp_bytes, speckv_comp_scheme_t scheme,
                                            void* cuda_stream) {
-    if (scheme == SPECKV_COMP_FP16) return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL;
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_cache);
-    if (rc != SPECKV_OK) return rc;
-    if (n_groups && !d_block_table) return SPECKV_ERR_INVAL;
-    a.in = d_cache;
-    a.elem_index = d_block_table;
-    return codec_run(false, a, cuda_stream);
+    if (scheme == SPECKV_COMP_FP16 || (n_groups && !d_block_table)) return invalid_argument();
+    return compress_blocks(KvBlocks{d_cache, d_block_table}, dtype, group_elems, n_groups, d_payload, slot_bytes,
+                           d_scales, d_comp_bytes, scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_compress_ragged(const void* d_in, const uint32_t* d_block_table, const uint32_t* d_group_len,
                                            speckv_dtype_t dtype, size_t group_elems, size_t n_groups, void* d_payload,
                                            size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
                                            speckv_comp_scheme_t scheme, void* cuda_stream) {
-    if (scheme == SPECKV_COMP_FP16) return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL;
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_in);
-    if (rc != SPECKV_OK) return rc;
-    if (n_groups && !d_group_len) return SPECKV_ERR_INVAL;
-    a.in = d_in;
-    a.elem_index = d_block_table;
-    a.group_len = d_group_len;
-    return codec_run(false, a, cuda_stream);
+    if (scheme == SPECKV_COMP_FP16 || (n_groups && !d_group_len)) return invalid_argument();
+    return compress_blocks(KvBlocks{d_in, d_block_table, d_group_len}, dtype, group_elems, n_groups, d_payload,
+                           slot_bytes, d_scales, d_comp_bytes, scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_decompress_scatter(const void* d_payload, size_t slot_bytes, const float* d_scales,
@@ -537,16 +539,9 @@ speckv_status_t speckv_ext_decompress_scatter(const void* d_payload, size_t slot
                                               const uint32_t* d_block_table, size_t n_requests, size_t group_elems,
                                               speckv_dtype_t dtype, void* d_cache, uint32_t* d_out_elems,
                                               speckv_comp_scheme_t scheme, void* cuda_stream) {
-    if (scheme == SPECKV_COMP_FP16) return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL;
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, dtype, group_elems, n_requests, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, d_cache);
-    if (rc != SPECKV_OK) return rc;
-    if (n_requests && !d_block_table) return SPECKV_ERR_INVAL;
-    a.out = d_cache;
-    a.elem_index = d_block_table;
-    a.out_elems = d_out_elems;
-    a.src_index = d_src_index;
-    return codec_run(true, a, cuda_stream);
+    if (scheme == SPECKV_COMP_FP16 || (n_requests && !d_block_table)) return invalid_argument();
+    return decompress_blocks(d_payload, slot_bytes, d_scales, d_comp_bytes, d_src_index, nullptr, n_requests,
+                             KvBlocks{d_cache, d_block_table}, dtype, group_elems, d_out_elems, scheme, cuda_stream);
 }
 
 // ---- KV cache sets ---------------------------------------------------------------------------------------------
@@ -592,16 +587,11 @@ speckv_status_t speckv_ext_compress_gather_set(const speckv_cache_set_t* set, co
                                                const uint32_t* d_block_table, const uint32_t* d_group_len, size_t n_groups,
                                                void* d_payload, size_t slot_bytes, float* d_scales, uint32_t* d_comp_bytes,
                                                speckv_comp_scheme_t scheme, void* cuda_stream) {
-    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!set || scheme == SPECKV_COMP_FP16 || !cache_set_on_current_device(*set)) return SPECKV_ERR_INVAL;
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, set->dtype, set->block_elems, n_groups, d_payload, slot_bytes, d_scales,
-                                          d_comp_bytes, scheme, set->d_bases);
+    const speckv_status_t rc = check_set(set, d_cache_index, d_block_table, n_groups);
     if (rc != SPECKV_OK) return rc;
-    if (n_groups && (!d_cache_index || !d_block_table)) return SPECKV_ERR_INVAL;
-    use_cache_set(a, *set, d_cache_index, d_block_table);
-    a.group_len = d_group_len;
-    return codec_run(false, a, cuda_stream);
+    if (scheme == SPECKV_COMP_FP16) return SPECKV_ERR_INVAL;
+    return compress_blocks(KvBlocks{nullptr, d_block_table, d_group_len, set, d_cache_index}, set->dtype,
+                           set->block_elems, n_groups, d_payload, slot_bytes, d_scales, d_comp_bytes, scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_decompress_scatter_set(const void* d_payload, size_t slot_bytes, const float* d_scales,
@@ -609,17 +599,12 @@ speckv_status_t speckv_ext_decompress_scatter_set(const void* d_payload, size_t 
                                                   const speckv_cache_set_t* set, const uint32_t* d_cache_index,
                                                   const uint32_t* d_block_table, size_t n_requests, uint32_t* d_out_elems,
                                                   speckv_comp_scheme_t scheme, void* cuda_stream) {
-    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!set || scheme == SPECKV_COMP_FP16 || !cache_set_on_current_device(*set)) return SPECKV_ERR_INVAL;
-    CodecArgs a;
-    const speckv_status_t rc = codec_args(a, set->dtype, set->block_elems, n_requests, d_payload, slot_bytes, d_scales,
-                                          d_comp_bytes, scheme, set->d_bases);
+    const speckv_status_t rc = check_set(set, d_cache_index, d_block_table, n_requests);
     if (rc != SPECKV_OK) return rc;
-    if (n_requests && (!d_cache_index || !d_block_table)) return SPECKV_ERR_INVAL;
-    use_cache_set(a, *set, d_cache_index, d_block_table);
-    a.out_elems = d_out_elems;
-    a.src_index = d_src_index;
-    return codec_run(true, a, cuda_stream);
+    if (scheme == SPECKV_COMP_FP16) return SPECKV_ERR_INVAL;
+    return decompress_blocks(d_payload, slot_bytes, d_scales, d_comp_bytes, d_src_index, nullptr, n_requests,
+                             KvBlocks{nullptr, d_block_table, nullptr, set, d_cache_index}, set->dtype, set->block_elems,
+                             d_out_elems, scheme, cuda_stream);
 }
 
 speckv_status_t speckv_ext_compress_host(const void* h_in, speckv_dtype_t dtype, size_t group_elems, size_t n_groups,

@@ -435,21 +435,18 @@ void speckv_ext_tier_destroy(speckv_tier_t* tier) {
     delete tier;
 }
 
-// d_group_len (device, optional): group i is the first min(d_group_len[i], group_elems) elements of its block
-// set (optional): group i is block d_block_table[i] of cache d_cache_index[i] of the set (d_in unused)
-static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, const uint32_t* d_block_table,
-                                         const uint32_t* d_group_len, speckv_dtype_t dtype, size_t group_elems,
-                                         size_t n_groups, const uint64_t* h_block_ids, void* cuda_stream,
-                                         const speckv_cache_set* set = nullptr, const uint32_t* d_cache_index = nullptr) {
+static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const KvBlocks& blocks, speckv_dtype_t dtype,
+                                         size_t group_elems, size_t n_groups, const uint64_t* h_block_ids,
+                                         void* cuda_stream) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!tier || !h_block_ids || (!d_in && !set && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0 ||
+    if (!tier || !h_block_ids || (!blocks.base && !blocks.set && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0 ||
         group_elems >= (1ull << 31))
         return SPECKV_ERR_INVAL;
     if (n_groups == 0) return SPECKV_OK;
     Tier& t = tier->t;
     std::lock_guard<std::mutex> lk(t.mu);
     const int scheme = t.scheme;
-    if (scheme == SPECKV_COMP_FP16 && (d_block_table || d_group_len || dtype == SPECKV_DTYPE_F32))
+    if (scheme == SPECKV_COMP_FP16 && (blocks.block_table || blocks.group_len || dtype == SPECKV_DTYPE_F32))
         return SPECKV_ERR_INVAL;   // raw passthrough: no gather or ragged form
     const size_t slot = speckv_ext_slot_bytes(group_elems, (speckv_comp_scheme_t)scheme);
     const size_t esz = dtype == SPECKV_DTYPE_F32 ? 4 : 2;
@@ -483,7 +480,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
             r.comp_bytes = t.h_comp[b][i];
             r.scale = t.h_scales[b][i];
             r.group_elems = (uint32_t)group_elems;
-            r.dtype = (int)dtype | (scheme << 8) | (d_group_len ? BlockRec::kRagged : 0);
+            r.dtype = (int)dtype | (scheme << 8) | (blocks.group_len ? BlockRec::kRagged : 0);
             if (t.blocks.exchange(h_block_ids[g0 + i], r, &old)) {
                 t.stats.used_bytes -= ((uint64_t)old.comp_bytes + 15u) & ~15ull;
                 // an id listed twice in this chunk: its first copy is part of the transfer in flight, so its
@@ -505,11 +502,7 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
         // buffer b is free once the payload copy of chunk - 2 has completed
         cudaStreamWaitEvent(st, t.ev_copy[b], 0);
         CodecArgs a(slot, group_elems, ng, dtype, scheme);
-        // paged form: the chunk's groups are the cache blocks its slice of the block table names
-        a.in = d_block_table ? d_in : (const void*)((const char*)d_in + g0 * group_elems * esz);
-        a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
-        a.group_len = d_group_len ? d_group_len + g0 : nullptr;   // ragged: slots + scan + pack (no packed emission)
-        if (set) use_cache_set(a, *set, d_cache_index + g0, d_block_table + g0);
+        blocks.bind(a, false, g0, esz);   // ragged: slots + scan + pack (no packed emission)
         a.payload = t.d_slots[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
@@ -548,9 +541,9 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
     if ((e = t.sync_dir(st)) != cudaSuccess && rc == SPECKV_OK) rc = status_of(e);   // the records this call changed
     if ((e = cudaGetLastError()) != cudaSuccess && rc == SPECKV_OK) rc = status_of(e);
     uint64_t raw = (uint64_t)n_groups * group_elems * esz;
-    if (rc == SPECKV_OK && d_group_len) {   // ragged: count the valid bytes (the lengths live on the device)
+    if (rc == SPECKV_OK && blocks.group_len) {   // ragged: count the valid bytes (the lengths live on the device)
         std::vector<uint32_t> len(n_groups);
-        e = cudaMemcpyAsync(len.data(), d_group_len, n_groups * 4, cudaMemcpyDeviceToHost, st);
+        e = cudaMemcpyAsync(len.data(), blocks.group_len, n_groups * 4, cudaMemcpyDeviceToHost, st);
         if (e == cudaSuccess) e = cudaStreamSynchronize(st);
         if (e != cudaSuccess) rc = status_of(e);
         raw = 0;
@@ -569,29 +562,29 @@ static speckv_status_t tier_offload_impl(speckv_tier_t* tier, const void* d_in, 
 
 speckv_status_t speckv_ext_tier_offload(speckv_tier_t* tier, const void* d_in, speckv_dtype_t dtype, size_t group_elems,
                                         size_t n_groups, const uint64_t* h_block_ids, void* cuda_stream) {
-    return tier_offload_impl(tier, d_in, nullptr, nullptr, dtype, group_elems, n_groups, h_block_ids, cuda_stream);
+    return tier_offload_impl(tier, KvBlocks{d_in}, dtype, group_elems, n_groups, h_block_ids, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_offload_paged(speckv_tier_t* tier, const void* d_cache, const uint32_t* d_block_table,
                                               speckv_dtype_t dtype, size_t group_elems, size_t n_blocks,
                                               const uint64_t* h_block_ids, void* cuda_stream) {
     if (!d_block_table && n_blocks) return SPECKV_ERR_INVAL;
-    return tier_offload_impl(tier, d_cache, d_block_table, nullptr, dtype, group_elems, n_blocks, h_block_ids, cuda_stream);
+    return tier_offload_impl(tier, KvBlocks{d_cache, d_block_table}, dtype, group_elems, n_blocks, h_block_ids, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_offload_ragged(speckv_tier_t* tier, const void* d_in, const uint32_t* d_block_table,
                                                const uint32_t* d_group_len, speckv_dtype_t dtype, size_t group_elems,
                                                size_t n_blocks, const uint64_t* h_block_ids, void* cuda_stream) {
     if (!d_group_len && n_blocks) return device_count() <= 0 ? SPECKV_ERR_DRIVER : SPECKV_ERR_INVAL;
-    return tier_offload_impl(tier, d_in, d_block_table, d_group_len, dtype, group_elems, n_blocks, h_block_ids, cuda_stream);
+    return tier_offload_impl(tier, KvBlocks{d_in, d_block_table, d_group_len}, dtype, group_elems, n_blocks, h_block_ids,
+                             cuda_stream);
 }
 
 static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_groups,
-                                         size_t group_elems, speckv_dtype_t dtype, void* d_out,
-                                         const uint32_t* d_block_table, void* cuda_stream,
-                                         const speckv_cache_set* set = nullptr, const uint32_t* d_cache_index = nullptr) {
+                                         size_t group_elems, speckv_dtype_t dtype, const KvBlocks& blocks,
+                                         void* cuda_stream) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!tier || !h_block_ids || (!d_out && !set && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0)
+    if (!tier || !h_block_ids || (!blocks.base && !blocks.set && n_groups) || dtype < 0 || dtype > 2 || group_elems == 0)
         return SPECKV_ERR_INVAL;
     if (n_groups == 0) return SPECKV_OK;
     Tier& t = tier->t;
@@ -657,14 +650,12 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
         cudaEventRecord(t.ev_copy[b], t.copy_st[b]);
         cudaStreamWaitEvent(st, t.ev_copy[b], 0);
         CodecArgs a(slot, group_elems, ng, dtype, scheme);
-        a.out = d_block_table ? d_out : (void*)((char*)d_out + g0 * group_elems * esz);
-        a.elem_index = d_block_table ? d_block_table + g0 : nullptr;
-        if (set) use_cache_set(a, *set, d_cache_index + g0, d_block_table + g0);
+        blocks.bind(a, true, g0, esz);
         a.payload = t.d_packed[b];
         a.scales = t.d_scales[b];
         a.comp_bytes = t.d_comp[b];
         a.slot_offsets = t.d_offsets[b];
-        if (scheme == SPECKV_COMP_FP16 && (d_block_table || dtype == SPECKV_DTYPE_F32)) return SPECKV_ERR_INVAL;
+        if (scheme == SPECKV_COMP_FP16 && (blocks.block_table || dtype == SPECKV_DTYPE_F32)) return SPECKV_ERR_INVAL;
         // a chunk holding ragged blocks counts what was decoded; otherwise every block is a whole group
         if (any_ragged) a.out_elems = t.d_oel[b];
         if ((e = launch_decompress(a, st)) != cudaSuccess) return status_of(e);
@@ -690,41 +681,34 @@ static speckv_status_t tier_restore_impl(speckv_tier_t* tier, const uint64_t* h_
 
 speckv_status_t speckv_ext_tier_restore(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_groups,
                                         size_t group_elems, speckv_dtype_t dtype, void* d_out, void* cuda_stream) {
-    return tier_restore_impl(tier, h_block_ids, n_groups, group_elems, dtype, d_out, nullptr, cuda_stream);
+    return tier_restore_impl(tier, h_block_ids, n_groups, group_elems, dtype, KvBlocks{d_out}, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_restore_paged(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_blocks,
                                               size_t group_elems, speckv_dtype_t dtype, void* d_cache,
                                               const uint32_t* d_block_table, void* cuda_stream) {
     if (!d_block_table && n_blocks) return SPECKV_ERR_INVAL;
-    return tier_restore_impl(tier, h_block_ids, n_blocks, group_elems, dtype, d_cache, d_block_table, cuda_stream);
+    return tier_restore_impl(tier, h_block_ids, n_blocks, group_elems, dtype, KvBlocks{d_cache, d_block_table}, cuda_stream);
 }
 
 // the set forms: geometry and dtype from the set, the rest shared with the single-cache forms
-static speckv_status_t check_set_call(const speckv_cache_set* set, const uint32_t* d_cache_index,
-                                      const uint32_t* d_block_table, size_t n) {
-    if (device_count() <= 0) return SPECKV_ERR_DRIVER;
-    if (!set || !cache_set_on_current_device(*set) || (n && (!d_cache_index || !d_block_table))) return SPECKV_ERR_INVAL;
-    return SPECKV_OK;
-}
-
 speckv_status_t speckv_ext_tier_offload_set(speckv_tier_t* tier, const speckv_cache_set_t* set,
                                             const uint32_t* d_cache_index, const uint32_t* d_block_table,
                                             const uint32_t* d_group_len, size_t n_blocks, const uint64_t* h_block_ids,
                                             void* cuda_stream) {
-    const speckv_status_t rc = check_set_call(set, d_cache_index, d_block_table, n_blocks);
+    const speckv_status_t rc = check_set(set, d_cache_index, d_block_table, n_blocks);
     if (rc != SPECKV_OK) return rc;
-    return tier_offload_impl(tier, nullptr, d_block_table, d_group_len, (speckv_dtype_t)set->dtype, set->block_elems,
-                             n_blocks, h_block_ids, cuda_stream, set, d_cache_index);
+    return tier_offload_impl(tier, KvBlocks{nullptr, d_block_table, d_group_len, set, d_cache_index},
+                             (speckv_dtype_t)set->dtype, set->block_elems, n_blocks, h_block_ids, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_restore_set(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n_blocks,
                                             const speckv_cache_set_t* set, const uint32_t* d_cache_index,
                                             const uint32_t* d_block_table, void* cuda_stream) {
-    const speckv_status_t rc = check_set_call(set, d_cache_index, d_block_table, n_blocks);
+    const speckv_status_t rc = check_set(set, d_cache_index, d_block_table, n_blocks);
     if (rc != SPECKV_OK) return rc;
-    return tier_restore_impl(tier, h_block_ids, n_blocks, set->block_elems, (speckv_dtype_t)set->dtype, nullptr,
-                             d_block_table, cuda_stream, set, d_cache_index);
+    return tier_restore_impl(tier, h_block_ids, n_blocks, set->block_elems, (speckv_dtype_t)set->dtype,
+                             KvBlocks{nullptr, d_block_table, nullptr, set, d_cache_index}, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_drop(speckv_tier_t* tier, const uint64_t* h_block_ids, size_t n) {
@@ -862,10 +846,8 @@ size_t speckv_ext_tier_fetch_workspace_bytes(size_t max_requests, size_t group_e
 
 static speckv_status_t tier_fetch_impl(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
                                        size_t max_requests, size_t group_elems, speckv_dtype_t dtype,
-                                       speckv_comp_scheme_t scheme, void* d_out, const uint32_t* d_block_table,
-                                       uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
-                                       size_t workspace_bytes, void* cuda_stream, const speckv_cache_set* set = nullptr,
-                                       const uint32_t* d_cache_index = nullptr) {
+                                       speckv_comp_scheme_t scheme, const KvBlocks& blocks, uint32_t* d_out_elems,
+                                       uint8_t* d_status, void* d_workspace, size_t workspace_bytes, void* cuda_stream) {
     if (device_count() <= 0) return SPECKV_ERR_DRIVER;
     if (!tier || dtype < 0 || dtype > 2 || (int)scheme < 1 || (int)scheme > 4 || group_elems == 0 ||
         group_elems >= (1ull << 31) || max_requests >= (1ull << 31))
@@ -876,7 +858,7 @@ static speckv_status_t tier_fetch_impl(speckv_tier_t* tier, const uint64_t* d_bl
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess || dev != t.device) return SPECKV_ERR_INVAL;
     if (max_requests == 0) return SPECKV_OK;
-    if (!d_block_ids || (!d_out && !set) || !d_workspace || (reinterpret_cast<uintptr_t>(d_workspace) & 15) ||
+    if (!d_block_ids || (!blocks.base && !blocks.set) || !d_workspace || (reinterpret_cast<uintptr_t>(d_workspace) & 15) ||
         workspace_bytes < speckv_ext_tier_fetch_workspace_bytes(max_requests, group_elems))
         return SPECKV_ERR_INVAL;
     const size_t n = max_requests;
@@ -889,8 +871,8 @@ static speckv_status_t tier_fetch_impl(speckv_tier_t* tier, const uint64_t* d_bl
     float* scales = reinterpret_cast<float*>(comp + n);
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     cudaError_t e = launch_fetch_lookup(t.d_dir, d_block_ids, d_n_requests, (uint32_t)n, (uint32_t)group_elems, dtype,
-                                        (int)scheme, slot, src_off, comp, scales, d_status, st, d_cache_index,
-                                        set ? set->n_caches : 0u);
+                                        (int)scheme, slot, src_off, comp, scales, d_status, st, blocks.cache_index,
+                                        blocks.set ? blocks.set->n_caches : 0u);
     if (e != cudaSuccess) return status_of(e);
     pack_offsets_kernel<<<1, 1024, 0, st>>>(comp, (uint32_t)n, d_n_requests, offsets, total);
     count_launch();
@@ -899,9 +881,7 @@ static speckv_status_t tier_fetch_impl(speckv_tier_t* tier, const uint64_t* d_bl
     if (e != cudaSuccess) return status_of(e);
     // the staged payloads form a packed container: the codec's decoders take it as it is
     CodecArgs a(slot, group_elems, n, dtype, (int)scheme);
-    a.out = d_out;
-    a.elem_index = d_block_table;
-    if (set) use_cache_set(a, *set, d_cache_index, d_block_table);
+    blocks.bind(a, true, 0, dtype == SPECKV_DTYPE_F32 ? 4 : 2);
     a.payload = staging;
     a.slot_offsets = offsets;
     a.scales = scales;
@@ -916,8 +896,8 @@ speckv_status_t speckv_ext_tier_fetch(speckv_tier_t* tier, const uint64_t* d_blo
                                       speckv_comp_scheme_t scheme, void* d_out, const uint32_t* d_block_table,
                                       uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
                                       size_t workspace_bytes, void* cuda_stream) {
-    return tier_fetch_impl(tier, d_block_ids, d_n_requests, max_requests, group_elems, dtype, scheme, d_out, d_block_table,
-                           d_out_elems, d_status, d_workspace, workspace_bytes, cuda_stream);
+    return tier_fetch_impl(tier, d_block_ids, d_n_requests, max_requests, group_elems, dtype, scheme,
+                           KvBlocks{d_out, d_block_table}, d_out_elems, d_status, d_workspace, workspace_bytes, cuda_stream);
 }
 
 speckv_status_t speckv_ext_tier_fetch_set(speckv_tier_t* tier, const uint64_t* d_block_ids, const uint32_t* d_n_requests,
@@ -925,11 +905,11 @@ speckv_status_t speckv_ext_tier_fetch_set(speckv_tier_t* tier, const uint64_t* d
                                           const uint32_t* d_block_table, speckv_comp_scheme_t scheme,
                                           uint32_t* d_out_elems, uint8_t* d_status, void* d_workspace,
                                           size_t workspace_bytes, void* cuda_stream) {
-    const speckv_status_t rc = check_set_call(set, d_cache_index, d_block_table, max_requests);
+    const speckv_status_t rc = check_set(set, d_cache_index, d_block_table, max_requests);
     if (rc != SPECKV_OK) return rc;
     return tier_fetch_impl(tier, d_block_ids, d_n_requests, max_requests, set->block_elems, (speckv_dtype_t)set->dtype,
-                           scheme, nullptr, d_block_table, d_out_elems, d_status, d_workspace, workspace_bytes,
-                           cuda_stream, set, d_cache_index);
+                           scheme, KvBlocks{nullptr, d_block_table, nullptr, set, d_cache_index}, d_out_elems, d_status,
+                           d_workspace, workspace_bytes, cuda_stream);
 }
 
 }  // extern "C"

@@ -10,7 +10,7 @@ import torch
 
 from . import _lib
 from ._lib import COMP_INT8_DELTA_RLE, check, lib
-from .codec import _DTYPES, KVCacheSet, _set_groups, _stream
+from .codec import _DTYPES, KVCacheSet, _i32, _lengths, _set_groups, _stream
 
 
 class HostTier:
@@ -58,7 +58,7 @@ class HostTier:
         group) named by `block_table` (CUDA int32) into the pool under `block_ids`, reading them in place."""
         assert cache.is_cuda and cache.is_contiguous()
         ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
-        table = block_table.to(device=cache.device, dtype=torch.int32).contiguous()
+        table = _i32(block_table, cache.device)
         assert ids.size == table.numel()
         with torch.cuda.device(cache.device):
             check(lib().speckv_ext_tier_offload_paged(self._h, cache.data_ptr(), table.data_ptr(), _DTYPES[cache.dtype],
@@ -72,13 +72,11 @@ class HostTier:
         write those elements back and leave the rest of each destination block untouched."""
         assert x.is_cuda and x.is_contiguous() and x.numel() % group_elems == 0
         ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
-        lengths = lengths.to(device=x.device, dtype=torch.int32).contiguous()
         assert ids.size == lengths.numel()
-        if bool((lengths < 0).any()):   # the offload synchronises anyway; a negative length would store the whole block
-            raise ValueError("offload_ragged: negative length")
+        lengths = _lengths(lengths, x.device, convert=True, check_negative=True)   # the offload synchronises anyway
         table = None
         if block_table is not None:
-            table = block_table.to(device=x.device, dtype=torch.int32).contiguous()
+            table = _i32(block_table, x.device)
             assert ids.size == table.numel()
         else:
             assert ids.size == x.numel() // group_elems
@@ -91,7 +89,7 @@ class HostTier:
         """Paged form: decompress the stored blocks `block_ids` straight into cache blocks `block_table`."""
         assert cache.is_cuda and cache.is_contiguous()
         ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
-        table = block_table.to(device=cache.device, dtype=torch.int32).contiguous()
+        table = _i32(block_table, cache.device)
         assert ids.size == table.numel()
         with torch.cuda.device(cache.device):
             check(lib().speckv_ext_tier_restore_paged(self._h, ids.ctypes.data, ids.size, cache[0].numel(),
@@ -109,12 +107,8 @@ class HostTier:
         ids = np.ascontiguousarray(block_ids, dtype=np.uint64)
         if ids.size != block_table.numel():
             raise ValueError("block_ids must hold one id per block")
-        if lengths is not None:
-            lengths = lengths.to(device=cset.device, dtype=torch.int32).contiguous()
-            if lengths.numel() != ids.size:
-                raise ValueError("lengths must hold one entry per block")
-            if bool((lengths < 0).any()):   # the offload synchronises anyway; a negative length would store the whole block
-                raise ValueError("offload_set: negative length")
+        if lengths is not None:   # the offload synchronises anyway: the lengths are read on the host
+            lengths = _lengths(lengths, cset.device, ids.size, convert=True, check_negative=True)
         with torch.cuda.device(cset.device):
             check(lib().speckv_ext_tier_offload_set(self._h, cset.handle(), cache_index.data_ptr(), block_table.data_ptr(),
                                                     lengths.data_ptr() if lengths is not None else None, ids.size,
@@ -142,23 +136,11 @@ class HostTier:
         a request is unserved (status 0, its block untouched) as in fetch(), and also when cache_index[i] >= len(cset).
         No host synchronisation: a warm call can be captured into a CUDA graph (the workspace is shared with fetch()
         calls of the same shape)."""
-        if not block_ids.is_cuda or block_ids.dtype not in (torch.int64, torch.uint64) or not block_ids.is_contiguous():
-            raise TypeError("block_ids must be a contiguous CUDA int64 tensor")
-        dev = block_ids.device
-        if dev != cset.device:
-            raise ValueError("block_ids must be on the device of the set")
-        n = block_ids.numel()
+        dev, n = self._fetch_requests(block_ids, count, cset.device)
         for name, t in (("cache_index", cache_index), ("block_table", block_table)):
             if not t.is_cuda or t.dtype != torch.int32 or t.numel() < n or not t.is_contiguous() or t.device != dev:
                 raise TypeError(f"{name} must be a contiguous CUDA int32 tensor with one entry per request")
-        if count is not None and (not count.is_cuda or count.dtype != torch.int32 or count.device != dev):
-            raise TypeError("count must be a CUDA int32 tensor on the device of block_ids")
-        if out_elems is None:
-            out_elems = torch.zeros(n, dtype=torch.int32, device=dev)
-        if status is None:
-            status = torch.zeros(n, dtype=torch.uint8, device=dev)
-        assert out_elems.numel() >= n and status.numel() >= n and out_elems.is_cuda and status.is_cuda
-        ws = self._workspace(n, cset.block_elems, dev)
+        out_elems, status, ws = self._fetch_outputs(n, cset.block_elems, dev, out_elems, status)
         with torch.cuda.device(dev):
             check(lib().speckv_ext_tier_fetch_set(self._h, block_ids.data_ptr(),
                                                   count.data_ptr() if count is not None else None, n, cset.handle(),
@@ -189,14 +171,9 @@ class HostTier:
         other geometry, dtype or decoder, raw block) leaves its destination as it is and gets out_elems 0.  Entries
         at and behind the count are not written.  The workspace is cached per (len(block_ids), group_elems) and
         allocated on the first eager call of that shape: run one before capturing."""
-        if not block_ids.is_cuda or block_ids.dtype not in (torch.int64, torch.uint64) or not block_ids.is_contiguous():
-            raise TypeError("block_ids must be a contiguous CUDA int64 tensor")
         if dtype not in _DTYPES:
             raise TypeError(f"unsupported dtype {dtype}")
-        dev = block_ids.device
-        n = block_ids.numel()
-        if count is not None and (not count.is_cuda or count.dtype != torch.int32 or count.device != dev):
-            raise TypeError("count must be a CUDA int32 tensor on the device of block_ids")
+        dev, n = self._fetch_requests(block_ids, count)
         if block_table is not None:
             if out is None:
                 raise ValueError("a block table needs the cache to write into (out)")
@@ -208,12 +185,7 @@ class HostTier:
         if out.dtype != dtype or out.device != dev or not out.is_contiguous() or out.numel() % group_elems or \
                 (block_table is None and out.numel() < n * group_elems):
             raise ValueError("out must be a contiguous tensor of whole blocks of `dtype` on the device of block_ids")
-        if out_elems is None:
-            out_elems = torch.zeros(n, dtype=torch.int32, device=dev)
-        if status is None:
-            status = torch.zeros(n, dtype=torch.uint8, device=dev)
-        assert out_elems.numel() >= n and status.numel() >= n and out_elems.is_cuda and status.is_cuda
-        ws = self._workspace(n, group_elems, dev)
+        out_elems, status, ws = self._fetch_outputs(n, group_elems, dev, out_elems, status)
         with torch.cuda.device(dev):
             check(lib().speckv_ext_tier_fetch(self._h, block_ids.data_ptr(), count.data_ptr() if count is not None else None,
                                               n, group_elems, _DTYPES[dtype], int(scheme), out.data_ptr(),
@@ -222,7 +194,27 @@ class HostTier:
                                               _stream()), "speckv_ext_tier_fetch")
         return out, out_elems, status
 
-    def _workspace(self, n: int, group_elems: int, dev: torch.device) -> torch.Tensor:
+    @staticmethod
+    def _fetch_requests(block_ids: torch.Tensor, count: Optional[torch.Tensor], set_device=None):
+        """The checks of fetch() and fetch_set() on the request list (block_ids on the set's device, for fetch_set):
+        -> (device, number of requests)."""
+        if not block_ids.is_cuda or block_ids.dtype not in (torch.int64, torch.uint64) or not block_ids.is_contiguous():
+            raise TypeError("block_ids must be a contiguous CUDA int64 tensor")
+        dev = block_ids.device
+        if set_device is not None and dev != set_device:
+            raise ValueError("block_ids must be on the device of the set")
+        if count is not None and (not count.is_cuda or count.dtype != torch.int32 or count.device != dev):
+            raise TypeError("count must be a CUDA int32 tensor on the device of block_ids")
+        return dev, block_ids.numel()
+
+    def _fetch_outputs(self, n: int, group_elems: int, dev: torch.device, out_elems: Optional[torch.Tensor],
+                       status: Optional[torch.Tensor]):
+        """fetch()'s and fetch_set()'s per-request outputs (zeroed when not given) and the workspace of the call."""
+        if out_elems is None:
+            out_elems = torch.zeros(n, dtype=torch.int32, device=dev)
+        if status is None:
+            status = torch.zeros(n, dtype=torch.uint8, device=dev)
+        assert out_elems.numel() >= n and status.numel() >= n and out_elems.is_cuda and status.is_cuda
         key = (n, group_elems, dev)
         ws = self._fetch_ws.get(key)
         if ws is None:
@@ -231,7 +223,7 @@ class HostTier:
             ws = torch.empty(max(lib().speckv_ext_tier_fetch_workspace_bytes(n, group_elems), 1), dtype=torch.uint8,
                              device=dev)
             self._fetch_ws[key] = ws
-        return ws
+        return out_elems, status, ws
 
     def stats(self) -> dict:
         s = _lib.TierStats()

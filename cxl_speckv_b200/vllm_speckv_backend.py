@@ -130,11 +130,8 @@ class CxlSpeckvKVAllocator:
         if num_tokens is None:
             tier.offload_blocks(kv_cache, block_table, ids)
             return
-        import torch
-        token_elems = kv_cache[0, 0].numel()   # kv_heads x head_dim: one token of the block is a contiguous row
-        lengths = torch.as_tensor(num_tokens, device=kv_cache.device).to(torch.int64) * token_elems
-        lengths = lengths.clamp_(0, kv_cache[0].numel()).to(torch.int32)
-        tier.offload_ragged(kv_cache, kv_cache[0].numel(), lengths, ids, block_table=block_table)
+        tier.offload_ragged(kv_cache, kv_cache[0].numel(), _token_lengths(num_tokens, kv_cache), ids,
+                            block_table=block_table)
 
     @staticmethod
     def restore_kv_blocks(kv_cache, block_table, tier, block_ids=None):
@@ -178,28 +175,26 @@ class CxlSpeckvKVAllocator:
         cache out to the host tier in one call, cache-major.  block_ids: uint64 [n_caches, n_blocks] (default
         request_block_ids).  num_tokens (optional, one entry per block): the filled tokens of each block, as in
         offload_kv_blocks, applied to every cache."""
-        import torch
-        cset = self._registered()
-        table = torch.as_tensor(block_table).to(device=cset.device, dtype=torch.int32).reshape(-1)
-        ids = self._request_ids(cset, table, block_ids)
-        cache_index, blocks = cset.groups(table)
+        cset, table, ids = self._request(block_table, block_ids)
         lengths = None
         if num_tokens is not None:
-            token_elems = cset.caches[0][0, 0].numel()   # kv_heads x head_dim: one token of the block
-            lengths = torch.as_tensor(num_tokens, device=cset.device).to(torch.int64).reshape(-1) * token_elems
+            lengths = _token_lengths(num_tokens, cset.caches[0])
             if lengths.numel() != table.numel():
                 raise ValueError("num_tokens must hold one entry per block")
-            lengths = lengths.clamp_(0, cset.block_elems).to(torch.int32).repeat(len(cset))
-        tier.offload_set(cset, cache_index, blocks, ids, lengths=lengths)
+            lengths = lengths.repeat(len(cset))
+        tier.offload_set(cset, *cset.groups(table), ids, lengths=lengths)
 
     def restore_request(self, block_table, tier, block_ids=None):
         """Bring one request's blocks of every registered cache back from the host tier in one call."""
+        cset, table, ids = self._request(block_table, block_ids)
+        tier.restore_set(ids, cset, *cset.groups(table))
+
+    def _request(self, block_table, block_ids):
+        """-> (the registered set, the request's block numbers as int32 on its device, their ids cache-major)"""
         import torch
         cset = self._registered()
         table = torch.as_tensor(block_table).to(device=cset.device, dtype=torch.int32).reshape(-1)
-        ids = self._request_ids(cset, table, block_ids)
-        cache_index, blocks = cset.groups(table)
-        tier.restore_set(ids, cset, cache_index, blocks)
+        return cset, table, self._request_ids(cset, table, block_ids)
 
     def _registered(self):
         if self._kv_set is None:
@@ -243,6 +238,13 @@ class CxlSpeckvKVAllocator:
         # [req][layer][kind][pos][head] * entry_bytes  (reference :95-100)
         return ((((req_id * self._num_layers + layer) * 2 + kind) * self._num_tokens + pos)
                 * self._num_heads + head) * entry_bytes
+
+
+def _token_lengths(num_tokens, cache):
+    """Filled tokens per block of a paged KV cache [num_blocks, block_size, ...] -> int32 element lengths on its device"""
+    import torch
+    lengths = torch.as_tensor(num_tokens, device=cache.device).to(torch.int64).reshape(-1) * cache[0, 0].numel()
+    return lengths.clamp_(0, cache[0].numel()).to(torch.int32)
 
 
 def _runs(pages):

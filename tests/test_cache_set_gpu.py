@@ -399,6 +399,34 @@ def test_set_argument_checks():
     assert L.speckv_ext_decompress_scatter_set(c.payload.data_ptr(), c.payload.shape[1], c.scales.data_ptr(),
                                                c.comp_bytes.data_ptr(), None, h, ci.data_ptr(), None, 2, None, 2,
                                                None) == pkg.SPECKV_ERR_INVAL
+    # each rejected argument on its own; an empty call checks no index array, but the raw scheme is refused even then
+    buf = dict(h=h, ci=ci.data_ptr(), bt=bt.data_ptr(), n=2, p=c.payload.data_ptr(), sb=c.payload.shape[1],
+               s=c.scales.data_ptr(), cb=c.comp_bytes.data_ptr(), scheme=2)
+    codec_calls = {
+        "gather_set": lambda a: L.speckv_ext_compress_gather_set(a["h"], a["ci"], a["bt"], None, a["n"], a["p"], a["sb"],
+                                                                 a["s"], a["cb"], a["scheme"], None),
+        "scatter_set": lambda a: L.speckv_ext_decompress_scatter_set(a["p"], a["sb"], a["s"], a["cb"], None, a["h"],
+                                                                     a["ci"], a["bt"], a["n"], None, a["scheme"], None),
+    }
+    for name, call in codec_calls.items():
+        for bad_arg in [dict(h=None), dict(ci=None), dict(bt=None), dict(scheme=0), dict(scheme=5), dict(sb=16),
+                        dict(p=None), dict(s=None), dict(cb=None), dict(p=c.payload.data_ptr() + 8)]:
+            assert call({**buf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, (name, bad_arg)
+        assert call({**buf, "n": 0, "scheme": 0}) == pkg.SPECKV_ERR_INVAL, name
+        assert call({**buf, "n": 0, "ci": None, "bt": None, "p": None, "s": None, "cb": None}) == pkg.SPECKV_OK, name
+    lens = _i32([5, 7])
+    with pytest.raises(TypeError):
+        codec.compress_gather_set(cset, ci, bt, lengths=lens.long())
+    with pytest.raises(ValueError):
+        codec.compress_gather_set(cset, ci, bt, lengths=lens[:1])
+    with pytest.raises(ValueError):
+        codec.compress_gather_set(cset, ci[:1], bt)
+    with pytest.raises(TypeError):
+        codec.compress_gather_set(cs.caches, ci, bt)
+    with pytest.raises(ValueError):
+        codec.decompress_scatter_set(c, cset, ci, bt, src_index=_i32([0]))
+    with pytest.raises(ValueError):
+        codec.decompress_scatter_set(c, cset, ci[:1], bt[:1])
     tier = HostTier(pool_bytes=8 << 20)
     try:
         ids = np.array([1, 2], dtype=np.uint64)
@@ -406,6 +434,50 @@ def test_set_argument_checks():
                                              None) == pkg.SPECKV_ERR_INVAL
         assert L.speckv_ext_tier_restore_set(tier._h, ids.ctypes.data, 2, h, ci.data_ptr(), None,
                                              None) == pkg.SPECKV_ERR_INVAL
+        tbuf = dict(t=tier._h, h=h, ci=ci.data_ptr(), bt=bt.data_ptr(), n=2, ids=ids.ctypes.data)
+        tier_calls = {
+            "offload_set": lambda a: L.speckv_ext_tier_offload_set(a["t"], a["h"], a["ci"], a["bt"], None, a["n"],
+                                                                   a["ids"], None),
+            "restore_set": lambda a: L.speckv_ext_tier_restore_set(a["t"], a["ids"], a["n"], a["h"], a["ci"], a["bt"],
+                                                                   None),
+        }
+        for name, call in tier_calls.items():
+            for bad_arg in [dict(t=None), dict(h=None), dict(ci=None), dict(bt=None), dict(ids=None)]:
+                assert call({**tbuf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, (name, bad_arg)
+            assert call({**tbuf, "n": 0, "ci": None, "bt": None}) == pkg.SPECKV_OK, name
+        with pytest.raises(ValueError):
+            tier.offload_set(cset, ci, bt, ids[:1])
+        with pytest.raises(ValueError):
+            tier.offload_set(cset, ci, bt, ids, lengths=lens[:1])
+        with pytest.raises(ValueError):
+            tier.offload_set(cset, ci, bt, ids, lengths=_i32([5, -1]))        # would store the whole block
+        with pytest.raises(ValueError):
+            tier.restore_set(ids[:1], cset, ci, bt)
+        dids = torch.from_numpy(ids.astype(np.int64)).to(DEV)
+        need = L.speckv_ext_tier_fetch_workspace_bytes(2, 2048)
+        ws = torch.empty(need, dtype=torch.uint8, device=DEV)
+        fbuf = dict(t=tier._h, ids=dids.data_ptr(), n=2, h=h, ci=ci.data_ptr(), bt=bt.data_ptr(), scheme=2,
+                    ws=ws.data_ptr(), wsb=need)
+
+        def fetch_set(a):
+            return L.speckv_ext_tier_fetch_set(a["t"], a["ids"], None, a["n"], a["h"], a["ci"], a["bt"], a["scheme"],
+                                               None, None, a["ws"], a["wsb"], None)
+
+        assert fetch_set(fbuf) == pkg.SPECKV_ERR_INVAL                                # before enable_fetch
+        tier.enable_fetch()
+        for bad_arg in [dict(t=None), dict(h=None), dict(ci=None), dict(bt=None), dict(ids=None), dict(scheme=0),
+                        dict(scheme=5), dict(ws=None), dict(ws=ws.data_ptr() + 8), dict(wsb=need - 1),
+                        dict(n=1 << 31)]:
+            assert fetch_set({**fbuf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, bad_arg
+        assert fetch_set({**fbuf, "n": 0, "ids": None, "ci": None, "bt": None, "ws": None}) == pkg.SPECKV_OK
+        with pytest.raises(TypeError):
+            tier.fetch_set(dids.int(), cset, ci, bt)
+        with pytest.raises(TypeError):
+            tier.fetch_set(dids, cset, ci[:1], bt)
+        with pytest.raises(TypeError):
+            tier.fetch_set(dids, cset, ci, bt.long())
+        with pytest.raises(TypeError):
+            tier.fetch_set(dids, cset, ci, bt, count=torch.ones(1, dtype=torch.int64, device=DEV))
         tier.set_scheme(0)
         with pytest.raises(SpeckvError):
             tier.offload_set(cset, ci, bt, ids)                                 # raw passthrough: no gather form

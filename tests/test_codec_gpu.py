@@ -291,6 +291,35 @@ def test_bad_arguments_are_rejected():
     bad = codec.CompressedKV(c.payload[:, :4080].contiguous(), c.scales, c.comp_bytes, 2048, c.dtype, c.scheme)
     with pytest.raises(SpeckvError):
         codec.decompress(bad)                  # slot smaller than the worst case
+    # the C entry points: each rejected argument on its own, and an empty call, which checks no buffer
+    import cxl_speckv_b200 as pkg
+    L = pkg.lib()
+    sb, o = c.payload.shape[1], torch.empty_like(x)
+    idx = torch.zeros(2, dtype=torch.int32, device=DEV)
+    cnt = torch.full((1,), 2, dtype=torch.int32, device=DEV)
+    buf = dict(p=c.payload.data_ptr(), sb=sb, s=c.scales.data_ptr(), cb=c.comp_bytes.data_ptr(), dt=0, G=2048, n=2,
+               scheme=2, x=x.data_ptr(), o=o.data_ptr(), idx=idx.data_ptr(), cnt=cnt.data_ptr())
+    calls = {
+        "compress": lambda a: L.speckv_ext_compress(a["x"], a["dt"], a["G"], a["n"], a["p"], a["sb"], a["s"], a["cb"],
+                                                    a["scheme"], None),
+        "decompress": lambda a: L.speckv_ext_decompress(a["p"], a["sb"], a["s"], a["cb"], a["G"], a["n"], a["dt"], a["o"],
+                                                        None, a["scheme"], None),
+        "indexed": lambda a: L.speckv_ext_decompress_indexed(a["p"], a["sb"], a["s"], a["cb"], a["idx"], a["n"], a["G"],
+                                                             a["dt"], a["o"], None, a["scheme"], None),
+        "routed": lambda a: L.speckv_ext_decompress_routed(a["p"], a["sb"], a["s"], a["cb"], a["idx"], a["cnt"], a["n"],
+                                                           a["G"], a["dt"], a["o"], None, a["scheme"], None),
+    }
+    common = [dict(dt=3), dict(dt=-1), dict(scheme=5), dict(scheme=-1), dict(dt=2, scheme=0), dict(sb=sb - 8),
+              dict(sb=sb - 16), dict(sb=1 << 32), dict(G=1 << 31), dict(n=1 << 32), dict(p=None), dict(s=None),
+              dict(cb=None), dict(p=c.payload.data_ptr() + 8)]
+    own = {"compress": [dict(x=None)], "decompress": [dict(o=None)], "indexed": [dict(o=None), dict(idx=None)],
+           "routed": [dict(o=None), dict(idx=None), dict(cnt=None)]}
+    for name, call in calls.items():
+        for bad_arg in common + own[name]:
+            assert call({**buf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, (name, bad_arg)
+        assert call({**buf, "n": 0, "p": None, "s": None, "cb": None, "x": None, "o": None, "idx": None,
+                     "cnt": None}) == pkg.SPECKV_OK, name
+        assert call({**buf, "n": 0, "dt": 3}) == pkg.SPECKV_ERR_INVAL, name
 
 
 def test_full_size_properties_llama70b_layer():
@@ -499,6 +528,40 @@ def test_paged_gather_scatter_rejects_bad_arguments():
         codec.decompress_scatter(c, torch.zeros((4, 4096), dtype=torch.float16, device=DEV), table)
     with pytest.raises(ValueError):
         codec.decompress_scatter(c, cache, table[:2])
+    lens = torch.full((4,), 100, dtype=torch.int32, device=DEV)
+    with pytest.raises(TypeError):
+        codec.compress_ragged(cache, 2048, lens.long())
+    with pytest.raises(TypeError):
+        codec.compress_ragged(cache, 2048, lens.cpu())
+    with pytest.raises(ValueError):
+        codec.compress_ragged(cache, 2048, lens[:3])                     # one length per block of x
+    with pytest.raises(ValueError):
+        codec.compress_ragged(cache, 2048, lens, block_table=table[:3])  # one length per table entry
+    with pytest.raises(ValueError):
+        codec.compress_ragged(cache, 1000, lens)
+    with pytest.raises(ValueError):
+        codec.compress_gather(cache.t(), table)
+    # the C entry points: each rejected argument on its own; the raw scheme is refused even for an empty call
+    import cxl_speckv_b200 as pkg
+    L = pkg.lib()
+    buf = dict(p=c.payload.data_ptr(), sb=c.payload.shape[1], s=c.scales.data_ptr(), cb=c.comp_bytes.data_ptr(), dt=0,
+               G=2048, n=4, scheme=2, x=cache.data_ptr(), t=table.data_ptr(), len=lens.data_ptr())
+    calls = {
+        "gather": lambda a: L.speckv_ext_compress_gather(a["x"], a["t"], a["dt"], a["G"], a["n"], a["p"], a["sb"], a["s"],
+                                                         a["cb"], a["scheme"], None),
+        "ragged": lambda a: L.speckv_ext_compress_ragged(a["x"], a["t"], a["len"], a["dt"], a["G"], a["n"], a["p"],
+                                                         a["sb"], a["s"], a["cb"], a["scheme"], None),
+        "scatter": lambda a: L.speckv_ext_decompress_scatter(a["p"], a["sb"], a["s"], a["cb"], None, a["t"], a["n"],
+                                                             a["G"], a["dt"], a["x"], None, a["scheme"], None),
+    }
+    own = {"gather": [dict(t=None)], "ragged": [dict(len=None)], "scatter": [dict(t=None)]}
+    for name, call in calls.items():
+        for bad_arg in [dict(scheme=0), dict(scheme=5), dict(dt=3), dict(x=None), dict(p=None), dict(s=None),
+                        dict(cb=None), dict(sb=16), dict(p=c.payload.data_ptr() + 8)] + own[name]:
+            assert call({**buf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, (name, bad_arg)
+        assert call({**buf, "n": 0, "scheme": 0}) == pkg.SPECKV_ERR_INVAL, name
+        assert call({**buf, "n": 0, "p": None, "s": None, "cb": None, "x": None, "t": None,
+                     "len": None}) == pkg.SPECKV_OK, name
 
 
 @pytest.mark.parametrize("G", [2048, 8192, 32768, 131072])

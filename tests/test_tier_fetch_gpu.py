@@ -280,6 +280,70 @@ def test_argument_checks():
         assert call(n, need) == pkg.SPECKV_OK
         torch.cuda.synchronize()
         assert torch.equal(_bits(out), _bits(tier.restore(np.arange(n, dtype=np.uint64), G, torch.float16)))
+        # each rejected argument on its own; an empty call checks no buffer
+        fbuf = dict(t=tier._h, ids=ids.data_ptr(), n=n, G=G, dt=0, scheme=2, out=out.data_ptr(), ws=ws.data_ptr(),
+                    wsb=need)
+
+        def fetch(a):
+            return L.speckv_ext_tier_fetch(a["t"], a["ids"], None, a["n"], a["G"], a["dt"], a["scheme"], a["out"], None,
+                                           None, None, a["ws"], a["wsb"], stream)
+
+        for bad_arg in [dict(t=None), dict(dt=3), dict(scheme=5), dict(G=0), dict(G=1 << 31), dict(n=1 << 31),
+                        dict(ids=None), dict(out=None), dict(ws=None), dict(ws=ws.data_ptr() + 8)]:
+            assert fetch({**fbuf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, bad_arg
+        assert fetch({**fbuf, "n": 0, "ids": None, "out": None, "ws": None}) == pkg.SPECKV_OK
+        hids = np.arange(n, dtype=np.uint64)
+        table = torch.arange(n, dtype=torch.int32, device=DEV)
+        lens = torch.full((n,), 100, dtype=torch.int32, device=DEV)
+        x = torch.randn(n * G, device=DEV).half()
+        obuf = dict(t=tier._h, x=x.data_ptr(), tab=table.data_ptr(), len=lens.data_ptr(), dt=0, G=G, n=n,
+                    ids=hids.ctypes.data)
+        offloads = {
+            "offload": lambda a: L.speckv_ext_tier_offload(a["t"], a["x"], a["dt"], a["G"], a["n"], a["ids"], stream),
+            "paged": lambda a: L.speckv_ext_tier_offload_paged(a["t"], a["x"], a["tab"], a["dt"], a["G"], a["n"],
+                                                               a["ids"], stream),
+            "ragged": lambda a: L.speckv_ext_tier_offload_ragged(a["t"], a["x"], a["tab"], a["len"], a["dt"], a["G"],
+                                                                 a["n"], a["ids"], stream),
+        }
+        restores = {
+            "restore": lambda a: L.speckv_ext_tier_restore(a["t"], a["ids"], a["n"], a["G"], a["dt"], a["x"], stream),
+            "paged": lambda a: L.speckv_ext_tier_restore_paged(a["t"], a["ids"], a["n"], a["G"], a["dt"], a["x"],
+                                                               a["tab"], stream),
+        }
+        own = {"offload": [], "paged": [dict(tab=None)], "ragged": [dict(len=None)], "restore": []}
+        for name, tier_call in list(offloads.items()) + list(restores.items()):
+            for bad_arg in [dict(t=None), dict(ids=None), dict(x=None), dict(dt=3), dict(G=0)] + own[name]:
+                assert tier_call({**obuf, **bad_arg}) == pkg.SPECKV_ERR_INVAL, (name, bad_arg)
+            assert tier_call({**obuf, "n": 0, "x": None, "tab": None, "len": None}) == pkg.SPECKV_OK, name
+        for name, tier_call in offloads.items():
+            assert tier_call({**obuf, "G": 1 << 31}) == pkg.SPECKV_ERR_INVAL, name
+        tier.set_scheme(0)                                                   # raw passthrough: dense fp16 only
+        for name, tier_call in offloads.items():
+            assert tier_call({**obuf, "dt": 2, "G": G // 2}) == pkg.SPECKV_ERR_INVAL, name
+        for name in ("paged", "ragged"):
+            assert offloads[name](obuf) == pkg.SPECKV_ERR_INVAL, name
+        assert offloads["offload"](obuf) == pkg.SPECKV_OK
+        assert restores["paged"](obuf) == pkg.SPECKV_ERR_INVAL               # the stored blocks are raw
+        assert restores["restore"]({**obuf, "dt": 2, "G": G}) == pkg.SPECKV_ERR_INVAL
+        assert restores["restore"](obuf) == pkg.SPECKV_OK
+        torch.cuda.synchronize()
+        assert torch.equal(_bits(x.view(n, G)), _bits(tier.restore(hids, G, torch.float16)))
+        with pytest.raises(TypeError):
+            tier.fetch(ids.int(), G, torch.float16)
+        with pytest.raises(TypeError):
+            tier.fetch(ids, G, torch.int8)
+        with pytest.raises(TypeError):
+            tier.fetch(ids, G, torch.float16, count=torch.ones(1, dtype=torch.int64, device=DEV))
+        with pytest.raises(ValueError):
+            tier.fetch(ids, G, torch.float16, block_table=table)                # a table needs the cache (out)
+        with pytest.raises(TypeError):
+            tier.fetch(ids, G, torch.float16, out=out, block_table=table[:2])
+        with pytest.raises(ValueError):
+            tier.fetch(ids, G, torch.float16, out=out[:2])
+        with pytest.raises(ValueError):
+            tier.fetch(ids, G, torch.bfloat16, out=out)
+        with pytest.raises(ValueError):
+            tier.offload_ragged(x, G, -lens, hids)                              # would store the whole block
         if torch.cuda.device_count() < 2:
             pytest.skip("one GPU: the other-device check needs two")
         with torch.cuda.device(1):
