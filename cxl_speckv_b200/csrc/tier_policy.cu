@@ -364,7 +364,9 @@ speckv_status_t speckv_ext_policy_place(speckv_policy_t* p, const uint64_t* h_id
         c.id = id; c.tier = (uint8_t)t; c.lru = 1; c.reset_count = 1;
         ch.push_back(c);
     }
-    return status_of(p->apply(ch));
+    cudaError_t e = cudaDeviceSynchronize();      // touches issued on other streams have landed
+    if (e == cudaSuccess) e = p->apply(ch);
+    return status_of(e);
 }
 
 speckv_status_t speckv_ext_policy_release(speckv_policy_t* p, const uint64_t* h_ids, size_t n) {
@@ -381,7 +383,9 @@ speckv_status_t speckv_ext_policy_release(speckv_policy_t* p, const uint64_t* h_
         c.id = id; c.tier = 255; c.lru = 1; c.reset_count = 1;
         ch.push_back(c);
     }
-    return status_of(p->apply(ch));
+    cudaError_t e = cudaDeviceSynchronize();      // touches issued on other streams have landed
+    if (e == cudaSuccess) e = p->apply(ch);
+    return status_of(e);
 }
 
 speckv_status_t speckv_ext_policy_touch(speckv_policy_t* p, const uint64_t* ids, size_t n, int ids_on_device, void* cuda_stream) {
@@ -389,8 +393,18 @@ speckv_status_t speckv_ext_policy_touch(speckv_policy_t* p, const uint64_t* ids,
     if (n == 0) return SPECKV_OK;
     std::lock_guard<std::mutex> lk(p->mu);
     DeviceGuard g(p->device);
-    if (p->clock + n >= kStampMax) return SPECKV_ERR_GENERAL;
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    // The stamps come from the host clock, which a graph replay would not advance: refuse capture
+    // before anything is enqueued.  CaptureImplicit: the legacy stream while a blocking stream captures.
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    cudaError_t ce = cudaStreamIsCapturing(st, &cs);
+    if (ce == cudaErrorStreamCaptureImplicit) {
+        cudaGetLastError();
+        return SPECKV_ERR_INVAL;
+    }
+    if (ce != cudaSuccess) return status_of(ce);
+    if (cs != cudaStreamCaptureStatusNone) return SPECKV_ERR_INVAL;
+    if (p->clock + n >= kStampMax) return SPECKV_ERR_GENERAL;
     const uint64_t* d_ids = ids;
     if (!ids_on_device) {
         cudaError_t e = p->need(n * 8);

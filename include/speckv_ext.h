@@ -487,7 +487,11 @@ SPECKV_API speckv_status_t speckv_ext_fetch_pages(speckv_handle_t handle, uint64
  * reference's pop drops them) until an L1 page has been popped and demoted; if the list holds
  * no L1 page nothing is evicted and the promotion proceeds, as in the reference.  Capacities
  * count pages.  Pair promote/demote with
- * speckv_ext_fetch_pages / speckv_ext_offload_pages to move the data. */
+ * speckv_ext_fetch_pages / speckv_ext_offload_pages to move the data.
+ * Ordering: place, release, promote, demote, lru_order and get_stats first wait for all
+ * outstanding device work, so a touch issued before them on any stream counts as done.
+ * Touches on two streams commute: each batch's stamps come from a host clock advanced when the
+ * call is made, so the LRU order follows the order of the calls, not of the kernels. */
 typedef struct speckv_policy speckv_policy_t;
 typedef struct {
     uint64_t l1_hits, l1_misses, l2_hits, l2_misses, l3_accesses;
@@ -504,7 +508,9 @@ SPECKV_API void speckv_ext_policy_destroy(speckv_policy_t* p);
 SPECKV_API speckv_status_t speckv_ext_policy_place(speckv_policy_t* p, const uint64_t* h_ids, size_t n, int tier,
                                                    uint8_t* out_tiers);
 SPECKV_API speckv_status_t speckv_ext_policy_release(speckv_policy_t* p, const uint64_t* h_ids, size_t n);
-/* ids on the device (ids_on_device != 0, stream-ordered, no host synchronisation) or on the host */
+/* ids on the device (ids_on_device != 0, stream-ordered, no host synchronisation) or on the host.
+ * Not capturable: the stamps come from the host clock, which a graph replay would not advance.  On a
+ * capturing stream it returns SPECKV_ERR_INVAL in both forms before it enqueues or copies anything. */
 SPECKV_API speckv_status_t speckv_ext_policy_touch(speckv_policy_t* p, const uint64_t* ids, size_t n,
                                                    int ids_on_device, void* cuda_stream);
 /* d_ids / d_out on the device, stream-ordered */

@@ -64,7 +64,9 @@ class Port:
     @classmethod
     def lib(cls):
         if cls._lib is None:
-            if not os.path.exists(PORT_SO):
+            srcs = [os.path.join(HERE, f) for f in ("speckv_oracle.c", "speckv_oracle.h")]
+            # a library older than its sources lacks what was added since: rebuild it
+            if not os.path.exists(PORT_SO) or os.path.getmtime(PORT_SO) < max(map(os.path.getmtime, srcs)):
                 build(ref=False)
             L = C.CDLL(PORT_SO)
             L.oracle_scale.restype = C.c_float
@@ -129,6 +131,18 @@ class Port:
             L.oracle_policy_lru.restype = C.c_size_t
             L.oracle_policy_lru.argtypes = [C.c_void_p, _u64p, C.c_size_t]
             L.oracle_policy_stats.argtypes = [C.c_void_p, C.c_void_p]
+            for f in ("oracle_policy_touch_n", "oracle_policy_release_n"):
+                getattr(L, f).restype = None
+                getattr(L, f).argtypes = [C.c_void_p, _u64p, C.c_size_t]
+            L.oracle_policy_place_n.restype = None
+            L.oracle_policy_place_n.argtypes = [C.c_void_p, _u64p, C.c_size_t, C.c_int, C.POINTER(C.c_int32)]
+            for f in ("oracle_policy_demote_n", "oracle_policy_is_hot_n"):
+                getattr(L, f).restype = None
+                getattr(L, f).argtypes = [C.c_void_p, _u64p, C.c_size_t, _u8p]
+            L.oracle_policy_promote_n.restype = C.c_size_t
+            L.oracle_policy_promote_n.argtypes = [C.c_void_p, _u64p, C.c_size_t, _u8p, _u64p]
+            L.oracle_policy_tiers.restype = None
+            L.oracle_policy_tiers.argtypes = [C.c_void_p, _u8p]
             cls._lib = L
         return cls._lib
 
@@ -408,6 +422,76 @@ class PolicyStats(C.Structure):
                                           "migrations_l1_to_l3", "migrations_l3_to_l1")] + \
                [("l1_hit_rate", C.c_double), ("l2_hit_rate", C.c_double)] + \
                [(n, C.c_uint64) for n in ("l1_pages", "l2_pages", "l3_pages")]
+
+
+class PolicyOracle:
+    """oracle_policy_* of the C restatement driven a batch at a time (its *_n forms: the single-page calls in
+    order), for traces too long for one ctypes call per page.  Ids are taken as uint64, so a negative id is a
+    page past the end."""
+
+    def __init__(self, n_pages: int, caps=(1 << 40, 1 << 40, 1 << 40)):
+        self.L = Port.lib()
+        self.n_pages = n_pages
+        self.h = C.c_void_p(self.L.oracle_policy_new(n_pages, *caps))
+
+    def close(self):
+        if self.h:
+            self.L.oracle_policy_free(self.h)
+            self.h = C.c_void_p()
+
+    @staticmethod
+    def _ids(ids) -> np.ndarray:
+        return np.ascontiguousarray(np.asarray(ids).astype(np.uint64, copy=False).ravel())
+
+    def place(self, ids, tier: int) -> np.ndarray:
+        """-> the tier each page went to, -1 where it was rejected"""
+        ids = self._ids(ids)
+        out = np.zeros(ids.size, dtype=np.int32)
+        self.L.oracle_policy_place_n(self.h, _ptr(ids, _u64p), ids.size, tier, _ptr(out, C.POINTER(C.c_int32)))
+        return out
+
+    def touch(self, ids) -> None:
+        ids = self._ids(ids)
+        self.L.oracle_policy_touch_n(self.h, _ptr(ids, _u64p), ids.size)
+
+    def release(self, ids) -> None:
+        ids = self._ids(ids)
+        self.L.oracle_policy_release_n(self.h, _ptr(ids, _u64p), ids.size)
+
+    def demote(self, ids) -> np.ndarray:
+        ids = self._ids(ids)
+        ok = np.zeros(ids.size, dtype=np.uint8)
+        self.L.oracle_policy_demote_n(self.h, _ptr(ids, _u64p), ids.size, _ptr(ok, _u8p))
+        return ok
+
+    def is_hot(self, ids) -> np.ndarray:
+        ids = self._ids(ids)
+        hot = np.zeros(ids.size, dtype=np.uint8)
+        self.L.oracle_policy_is_hot_n(self.h, _ptr(ids, _u64p), ids.size, _ptr(hot, _u8p))
+        return hot
+
+    def promote(self, ids):
+        """-> (ok[n] uint8, evicted page ids in order)"""
+        ids = self._ids(ids)
+        ok = np.zeros(ids.size, dtype=np.uint8)
+        ev = np.zeros(max(ids.size, 1), dtype=np.uint64)
+        k = self.L.oracle_policy_promote_n(self.h, _ptr(ids, _u64p), ids.size, _ptr(ok, _u8p), _ptr(ev, _u64p))
+        return ok, ev[:k].copy()
+
+    def tiers(self) -> np.ndarray:
+        out = np.zeros(max(self.n_pages, 1), dtype=np.uint8)
+        self.L.oracle_policy_tiers(self.h, _ptr(out, _u8p))
+        return out[: self.n_pages]
+
+    def lru_order(self) -> np.ndarray:
+        out = np.zeros(max(self.n_pages, 1), dtype=np.uint64)
+        k = self.L.oracle_policy_lru(self.h, _ptr(out, _u64p), self.n_pages)
+        return out[:k].copy()
+
+    def stats(self) -> dict:
+        st = PolicyStats()
+        self.L.oracle_policy_stats(self.h, C.byref(st))
+        return {n: getattr(st, n) for n, _ in PolicyStats._fields_}
 
 
 def run_policy_trace(ops, n_pages: int, caps=(1 << 40, 1 << 40, 1 << 40), impl: str = "port"):

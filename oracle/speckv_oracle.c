@@ -674,6 +674,51 @@ size_t oracle_policy_lru(const oracle_policy_t* p, uint64_t* out, size_t cap) {
     return k;
 }
 
+/* batch forms: the single-page calls above, in order */
+void oracle_policy_touch_n(oracle_policy_t* p, const uint64_t* pages, size_t n) {
+    for (size_t i = 0; i < n; ++i) oracle_policy_touch(p, pages[i]);
+}
+
+void oracle_policy_place_n(oracle_policy_t* p, const uint64_t* pages, size_t n, int tier, int32_t* out) {
+    for (size_t i = 0; i < n; ++i) {
+        const int t = oracle_policy_place(p, pages[i], tier);
+        if (out) out[i] = t;
+    }
+}
+
+void oracle_policy_release_n(oracle_policy_t* p, const uint64_t* pages, size_t n) {
+    for (size_t i = 0; i < n; ++i) oracle_policy_release(p, pages[i]);
+}
+
+void oracle_policy_demote_n(oracle_policy_t* p, const uint64_t* pages, size_t n, uint8_t* ok) {
+    for (size_t i = 0; i < n; ++i) {
+        const int r = oracle_policy_demote(p, pages[i]);
+        if (ok) ok[i] = (uint8_t)r;
+    }
+}
+
+void oracle_policy_is_hot_n(oracle_policy_t* p, const uint64_t* pages, size_t n, uint8_t* hot) {
+    for (size_t i = 0; i < n; ++i) hot[i] = (uint8_t)oracle_policy_is_hot(p, pages[i]);
+}
+
+size_t oracle_policy_promote_n(oracle_policy_t* p, const uint64_t* pages, size_t n, uint8_t* ok, uint64_t* evicted) {
+    size_t k = 0;
+    for (size_t i = 0; i < n; ++i) {
+        uint64_t ev;
+        const int r = oracle_policy_promote(p, pages[i], &ev);
+        if (ok) ok[i] = (uint8_t)r;
+        if (ev != POL_NONE) {
+            if (evicted) evicted[k] = ev;
+            ++k;
+        }
+    }
+    return k;
+}
+
+void oracle_policy_tiers(const oracle_policy_t* p, uint8_t* out) {
+    for (uint64_t g = 0; g < p->n; ++g) out[g] = p->tier[g];
+}
+
 void oracle_policy_stats(const oracle_policy_t* p, oracle_policy_stats_t* out) {
     *out = p->st;
     const uint64_t t1 = out->l1_hits + out->l1_misses, t2 = out->l2_hits + out->l2_misses;
